@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # our arm (CUDA, through libcvs_b200.so)
     python bench.py --impl reference --gpus N --steps K ...   # the reference's CPU path on the host cores
+    python bench.py ... --dump-outputs DIR                    # also writes what the last timed step computed
 
 Headline workload (BASELINE.json configs[1]): 1080p BGR24 synthetic 300-frame sequences at change densities
 1 % / 10 % / 50 %, thresholded diff + negative feedback + ordered compaction.  One STEP = one pass over the
@@ -45,6 +46,10 @@ BASE_SEED = 0xC0DA5EED
 W4K, H4K = 3840, 2160
 N4K = 3 * W4K * H4K
 C5_STREAMS, C5_FRAMES, C5_DENSITY = 8, 48, 100000
+# --dump-outputs, per density: (xs, diff) entries sampled over the frames of the last step (float64 + float32, 12 bytes
+# an entry) and bytes of the final reference frame (float32): three densities x 16 MB, under 64 MB.
+DUMP_PAYLOAD_ENTRIES = 1 << 20
+DUMP_REFERENCE_BYTES = 1 << 20
 
 
 def workload_config(frames: int) -> dict:
@@ -246,6 +251,40 @@ def gaussian_k3():
     return (k / total).astype(np.float32)
 
 
+def dump_slots(pos: np.ndarray, per_frame: int) -> np.ndarray:
+    """[T, per_frame] payload slots sampled from each frame's count: the same seeded fractions of every count, so two
+    builds that agree on `pos` are compared at the same entries."""
+    u = np.sort(np.random.default_rng(BASE_SEED).random(per_frame))
+    return (u[None, :] * np.asarray(pos, dtype=np.int64)[:, None]).astype(np.int64)
+
+
+def dump_reference_index(n: int) -> np.ndarray:
+    """Sorted, seeded byte positions of a reference frame of n bytes (all of them when n <= DUMP_REFERENCE_BYTES)."""
+    if n <= DUMP_REFERENCE_BYTES:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(BASE_SEED + 1).choice(n, size=DUMP_REFERENCE_BYTES, replace=False))
+
+
+def dump_outputs(out_dir: str, seqs, T: int, torch) -> None:
+    """What the headline's last timed step returned to its caller, per density: DIR/d<ppm>_pos.npy (every frame's
+    count), d<ppm>_xs.npy and d<ppm>_diff.npy ([T, S] entries at dump_slots(pos, S); -1 where a frame has none) and
+    d<ppm>_reference.npy (the stream's reference frame after the step, at dump_reference_index(N))."""
+    os.makedirs(out_dir, exist_ok=True)
+    per_frame = max(1, DUMP_PAYLOAD_ENTRIES // T)
+    ref_idx = dump_reference_index(N)
+    for q in seqs:
+        pos = q["pos"].cpu().numpy()
+        slots = dump_slots(pos, per_frame) + np.arange(T, dtype=np.int64)[:, None] * q["cap"]
+        flat = torch.from_numpy(slots).to(q["xs"].device)
+        xs = q["xs"][flat].cpu().numpy().astype(np.float64)
+        diff = q["diff"][flat].cpu().numpy().astype(np.float32)
+        xs[pos == 0], diff[pos == 0] = -1, -1
+        arrays = {"pos": pos.astype(np.float64), "xs": xs, "diff": diff,
+                  "reference": q["stream"].reference()[ref_idx].astype(np.float32)}
+        for name, a in arrays.items():
+            np.save(os.path.join(out_dir, "d%d_%s.npy" % (q["d"], name)), a)
+
+
 def ours(args):
     import torch
     import torch.distributed as dist
@@ -328,6 +367,8 @@ def ours(args):
     for q in seqs:
         q["stream"].sequence_status()
     launches = sum(q["stream"].launch_count() for q in seqs) - launches0
+    if args.dump_outputs and rank == 0:  # before the side workloads reuse the payload buffers
+        dump_outputs(args.dump_outputs, seqs, T, torch)
     # per-launch durations of the stream kernel and the algorithmic bytes each launch moved
     per_density = []
     tot_alg = tot_hbm = 0
@@ -741,7 +782,13 @@ def main():
     ap.add_argument("--ref-seconds", type=float, default=20.0, help="--impl reference: CPU seconds over all steps")
     ap.add_argument("--width", type=int, default=W, help="frame width (default: the 1080p headline workload)")
     ap.add_argument("--height", type=int, default=H)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write rank 0's last-step payload of the headline (per density: counts, a "
+                         "seeded sample of (xs, diff) and of the reference frame) as DIR/*.npy, float32/float64, under "
+                         "64 MB, to compare two builds on identical inputs")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     if (args.width, args.height) != (W, H):
         # other frame sizes for the headline loop (experiments); the driver runs the 1080p default
         W, H = args.width, args.height

@@ -5,6 +5,7 @@
 * 1080p sequences with the noise filter + binarisation (config 3) and heat map / red map (config 4)
 * the reference's own camera frames f1.jpg / f2.jpg at full size against the digests recorded in the build
   container (tests/golden/k1_f1_f2.json, REPORT/report.tex:2594)
+* what `bench.py --dump-outputs` writes: the last timed step of the headline loop
 
 Every comparison is bit-exact against oracle/cvs_oracle.c on the same frames (generated on the device by the
 synthetic camera, whose numpy twin is checked in test_sequence_gpu.py::test_synth_device_twin).
@@ -128,6 +129,58 @@ def test_1080p_filter_sequences(cvs, oracle, name, mode, noise):
     assert np.array_equal(s.reference(), oc.reference())
     s.close()
     oc.close()
+
+
+def _same_payloads(a, b):
+    return all(x[0] == y[0] and np.array_equal(x[1], y[1]) and np.array_equal(x[2], y[2]) for x, y in zip(a, b))
+
+
+def test_bench_dump_outputs_are_the_last_timed_step(cvs, oracle, tmp_path):
+    # bench.py --dump-outputs at the headline frame size, no warmup: every stream runs exactly `steps` passes over the
+    # same frames (each pass starts from the reference the previous one left), and the dump is the last of them,
+    # against the oracle.  On these frames the pass before and the pass after give other payloads, so a dump of one
+    # pass too few or too many, or a --steps that ran another number of passes, does not match.
+    import subprocess
+    import sys
+    import torch
+    import bench
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    w, h, T, steps = 1920, 1080, 4, 2
+    out = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--frames", str(T), "--warmup", "0",
+                          "--steps", str(steps), "--no-cpu", "--no-side", "--e2e-frames", "4", "--e2e-ring", "4",
+                          "--sync-frames", "4", "--dump-outputs", str(tmp_path)],
+                         capture_output=True, text=True, timeout=600, cwd=root)
+    assert out.returncode == 0, out.stderr[-2000:]
+    lines = [l for l in out.stdout.splitlines() if l.startswith("{")]
+    assert len(lines) == 1 and json.loads(lines[0])["steps"] == steps
+    files = sorted(os.listdir(tmp_path))
+    assert files == sorted("d%d_%s.npy" % (d, k) for d in bench.DENSITIES_PPM for k in ("pos", "xs", "diff", "reference"))
+    assert sum(os.path.getsize(tmp_path / f) for f in files) <= 64 << 20
+    n = 3 * w * h
+    for d in bench.DENSITIES_PPM:
+        got = {k: np.load(tmp_path / ("d%d_%s.npy" % (d, k))) for k in ("pos", "xs", "diff", "reference")}
+        assert all(a.dtype in (np.float32, np.float64) for a in got.values())
+        fr, stride = _device_sequence(cvs, torch, w, h, T, d, BENCH_SEED, stride=n)
+        frames = fr[:(T + 1) * n].cpu().numpy().reshape(T + 1, n)
+        oc = oracle.OracleCore(w, h, frames[0])
+        passes, refs = [], []
+        for _ in range(steps + 1):
+            passes.append([oc.exec_core(f)[:3] for f in frames[1:]])
+            refs.append(oc.reference())
+        oc.close()
+        last = passes[steps - 1]
+        assert not _same_payloads(passes[steps - 2], last) and not _same_payloads(passes[steps], last), \
+            f"density {d}: neighbouring passes give the same payload, the check would not tell them apart"
+        pos = np.array([p for p, _, _ in last])
+        assert np.array_equal(got["pos"], pos), f"density {d}: counts"
+        slots = bench.dump_slots(pos, got["xs"].shape[1])
+        for t, (p, xs, diff) in enumerate(last):
+            if p == 0:  # no entries: the dump holds the -1 sentinel
+                assert (got["xs"][t] == -1).all() and (got["diff"][t] == -1).all(), f"density {d} frame {t}"
+                continue
+            assert np.array_equal(got["xs"][t], xs[slots[t]]) and np.array_equal(got["diff"][t], diff[slots[t]]), \
+                f"density {d} frame {t}"
+        assert np.array_equal(got["reference"], refs[steps - 1][bench.dump_reference_index(n)]), f"density {d}: reference"
 
 
 def _sha(a):

@@ -6,7 +6,6 @@ import os
 import numpy as np
 import pytest
 
-REF = "/root/reference"
 GOLDEN = os.path.join(os.path.dirname(__file__), "golden")
 
 
@@ -98,13 +97,12 @@ def test_heat_pixel_endpoints(oracle):
     assert oracle.heat_pixel(510)[0] == 255
 
 
-@pytest.mark.skipif(not os.path.exists(os.path.join(REF, "tests/noise_filter_benchmark/f1.jpg")),
-                    reason="reference fixtures only exist in the build container")
 def test_k1_fixture_changed_bytes(oracle):
-    # REPORT/report.tex:2594: 369,350 changed bytes (5.93 %) between f1.jpg and f2.jpg
+    # REPORT/report.tex:2594: 369,350 changed bytes (5.93 %) between f1.jpg and f2.jpg (committed byte for byte as
+    # tests/golden/k1_f1.jpg, k1_f2.jpg)
     cv2 = pytest.importorskip("cv2")
-    a = cv2.imread(os.path.join(REF, "tests/noise_filter_benchmark/f1.jpg"))
-    b = cv2.imread(os.path.join(REF, "tests/noise_filter_benchmark/f2.jpg"))
+    a = cv2.imread(os.path.join(GOLDEN, "k1_f1.jpg"))
+    b = cv2.imread(os.path.join(GOLDEN, "k1_f2.jpg"))
     assert a.shape == (1080, 1920, 3)
     assert oracle.count_difference(a, b, 20) == 369350
     pos, xs, diff, ref, _ = oracle.diff_compact(b, a, 20)
@@ -114,10 +112,14 @@ def test_k1_fixture_changed_bytes(oracle):
 
 
 def test_k1_committed_fixture_copies(oracle):
-    # the same pair as committed fixtures (tests/golden/k1_f1.jpg, k1_f2.jpg: byte copies of the reference's files),
-    # so the K1 pin also holds where /root/reference does not exist
+    # the same pair as committed fixtures (tests/golden/k1_f1.jpg, k1_f2.jpg: byte copies of the reference's
+    # tests/noise_filter_benchmark/f1.jpg and f2.jpg, whose SHA-256 digests are pinned below)
     cv2 = pytest.importorskip("cv2")
     import hashlib
+    for name, digest in (("k1_f1.jpg", "809f5ef0d3b6a54f663c2c61989b31232a2262180ceaa6fdf8cdde65e0c1df49"),
+                         ("k1_f2.jpg", "4a2b18dde169e7859cec82626416eee48a50de520674790e08c426e9c5f25dea")):
+        with open(os.path.join(GOLDEN, name), "rb") as x:
+            assert hashlib.sha256(x.read()).hexdigest() == digest, name
     with open(os.path.join(GOLDEN, "k1_f1_f2.json")) as f:
         g = json.load(f)
     a = cv2.imread(os.path.join(GOLDEN, "k1_f1.jpg"))
@@ -127,10 +129,6 @@ def test_k1_committed_fixture_copies(oracle):
     pos, xs, diff, ref, _ = oracle.diff_compact(b, a, 20)
     assert pos == 369350 == oracle.count_difference(a, b, 20)
     assert sha(xs) == g["sha256_xs"] and sha(diff) == g["sha256_diff"] and sha(ref) == g["sha256_new_reference"]
-    if os.path.exists(os.path.join(REF, "tests/noise_filter_benchmark/f1.jpg")):
-        for mine, theirs in (("k1_f1.jpg", "f1.jpg"), ("k1_f2.jpg", "f2.jpg")):
-            with open(os.path.join(GOLDEN, mine), "rb") as x, open(os.path.join(REF, "tests/noise_filter_benchmark", theirs), "rb") as y:
-                assert x.read() == y.read()
 
 
 def test_golden_k1_record():
