@@ -21,8 +21,10 @@ struct ConvWeights {
 
 __device__ __forceinline__ uint32_t trunc_u8(float acc)
 {
-    // (uint8_t)acc as x86-64 compiles it: cvttss2si to a 32-bit integer, low byte
-    return (uint32_t)__float2int_rz(acc) & 0xffu;
+    // (uint8_t)acc as x86-64 compiles it: cvttss2si to a 32-bit integer, low byte.  cvttss2si gives 0x80000000 (low
+    // byte 0) for NaN and for anything outside [-2^31, 2^31); F2I saturates 2^31 and above (+inf too) to 0x7fffffff,
+    // whose low byte would be 0xff.  Below -2^31 it also gives 0x80000000, and NaN converts to 0.
+    return acc < 2147483648.0f ? (uint32_t)__float2int_rz(acc) & 0xffu : 0u;
 }
 
 template <int K>

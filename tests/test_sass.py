@@ -47,11 +47,15 @@ def test_no_kernel_spills_in_the_hot_variants():
 
 
 def test_noise_filter_is_fma_in_fixed_order():
-    for wb in (1, 2):   # k_conv_strip<3, true, WB>: WB words (4*WB bytes) per thread
-        k = _function(r"k_conv_stripILi3ELb1ELi%dE" % wb)
+    # every k_conv_strip<K, NONNEG, WB> launch_conv can pick: WB words (4*WB bytes) per thread
+    for K, nonneg, wb in ((3, True, 2), (3, False, 2), (3, True, 1), (3, False, 1), (5, True, 1), (5, False, 1)):
+        name = r"k_conv_stripILi%dELb%dELi%dE" % (K, int(nonneg), wb)
+        k = _function(name)
         # packed fp32 (sm_100): one FFMA2 carries the same tap of two neighbouring output bytes, each half rounded like FFMA
-        assert len(re.findall(r"\bFFMA2\b", k)) == 8 * 18 * wb, "8 rows x 2*WB byte pairs x 9 taps, one FFMA2 each"
-        assert not re.search(r"\bFFMA\b", k), "no scalar FFMA left"
-        assert re.search(r"\bFADD2\b", k) and re.search(r"\bFADD2\.RZ\b", k), "byte -> float and truncation are packed too"
-        assert "F2I" not in k, "non-negative weights truncate with FADD.RZ, not F2I"
-        assert not re.search(r"\b(LDL|STL)\b", k), "the row window must stay in registers"
+        assert len(re.findall(r"\bFFMA2\b", k)) == 8 * 2 * wb * K * K, f"{name}: 8 rows x 2*WB byte pairs x K*K taps, one FFMA2 each"
+        assert not re.search(r"\bFFMA\b", k), f"{name}: no scalar FFMA left"
+        assert re.search(r"\bFADD2\b", k), f"{name}: byte -> float is packed too"
+        if nonneg:
+            assert re.search(r"\bFADD2\.RZ\b", k), f"{name}: truncation is packed too"
+            assert "F2I" not in k, f"{name}: non-negative weights truncate with FADD.RZ, not F2I"
+        assert not re.search(r"\b(LDL|STL)\b", k), f"{name}: the row window must stay in registers"
