@@ -1638,7 +1638,9 @@ size_t cvs_wire_size(const uint8_t *wire)
     uint32_t hd[4];
     memcpy(hd, wire, sizeof hd);
     if (hd[0] != cvs::kWireMagic || hd[3] != cvs::kWireTile) return 0;
-    return (size_t)cvs::kWireHeader + cvs::wire_pad16(hd[2]) + cvs::wire_pad16(hd[1]) + hd[1];
+    // in 64 bits: ntiles and pos come from the sender, and near 2^32 their padding would wrap in 32
+    const uint64_t ntiles = hd[2], pos = hd[1];
+    return (size_t)(cvs::kWireHeader + ((ntiles + 15) & ~15ull) + ((pos + 15) & ~15ull) + pos);
 }
 
 cvs_status cvs_wire_encode_device(const int *d_xs, const uint8_t *d_diff, const unsigned int *d_pos, size_t capacity,
@@ -1668,8 +1670,12 @@ cvs_status cvs_wire_decode_device(const uint8_t *d_wire, uint32_t *d_scratch, ui
     if (!d_wire || !d_scratch || width <= 0 || height <= 0) return fail(CVS_ERR_INVALID, "bad argument");
     if ((uintptr_t)d_wire & 15) return fail(CVS_ERR_ALIGN, "16-byte alignment required");
     const uint32_t n = 3u * (uint32_t)width * (uint32_t)height, ntiles = (n + cvs::kWireTile - 1) / cvs::kWireTile;
+    const uint32_t last_len = n - (ntiles - 1) * cvs::kWireTile;
     cudaStream_t s = (cudaStream_t)cuda_stream;
-    cvs::k_wire_scan<<<1, 1024, 0, s>>>(d_wire, ntiles, d_scratch);
+    // header, counts and sum; then the offsets of a frame that passed; then the frame, unless one of the two refused it
+    cvs::k_wire_scan<<<1, 1024, 0, s>>>(d_wire, ntiles, last_len, d_scratch);
+    CU_TRY(cudaGetLastError());
+    cvs::k_wire_check<<<4 * sms, 256, 0, s>>>(d_wire, ntiles, last_len, d_scratch);
     CU_TRY(cudaGetLastError());
     cvs::k_wire_apply<<<4 * sms, 256, 0, s>>>(d_wire, ntiles, d_scratch, d_frame, d_xs, d_diff, d_pos);
     CU_TRY(cudaGetLastError());
@@ -1683,7 +1689,8 @@ cvs_status cvs_wire_decode_status(const uint32_t *d_scratch, int width, int heig
     uint32_t flag = 0;
     CU_TRY(cudaMemcpyAsync(&flag, d_scratch + ntiles + 1, sizeof flag, cudaMemcpyDeviceToHost, (cudaStream_t)cuda_stream));
     CU_TRY(cudaStreamSynchronize((cudaStream_t)cuda_stream));
-    if (flag) return fail(CVS_ERR_INVALID, "encoded frame is inconsistent (magic, geometry or counts): nothing was applied");
+    if (flag) return fail(CVS_ERR_INVALID, "encoded frame is inconsistent (magic, tile or geometry, a tile count above its tile's length, counts that do not "
+                                       "add up to pos, or offsets out of range or not ascending): nothing was applied");
     return CVS_OK;
 }
 

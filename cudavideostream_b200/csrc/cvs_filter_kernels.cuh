@@ -552,7 +552,8 @@ __global__ void __launch_bounds__(256) k_payload_push(const int *__restrict__ xs
 //     u8  diff[pos]                                               the reference's value bytes, unchanged
 // = 16 + N/192 + 2 pos bytes instead of 4 + 5 pos.  Encoding is two small kernels over the payload the stream kernel
 // left in device memory; they store 16 bytes per thread straight into the caller's (mapped, pinned) buffer.
-// Decoding (client side): exclusive scan of the counts, then one warp per tile.
+// Decoding (client side): exclusive scan of the counts, then one warp per tile checks the offsets, then one warp per
+// tile applies them.
 // ------------------------------------------------------------------------------------------------
 constexpr uint32_t kWireTile = 192;
 constexpr uint32_t kWireMagic = 0x31575643u; // "CVW1"
@@ -624,9 +625,10 @@ __global__ void __launch_bounds__(256) k_wire_pack(const int *__restrict__ xs, c
 }
 
 // client: exclusive scan of the per-tile counts of one encoded frame -> starts[0..ntiles], one 1024-thread block.
-// starts[ntiles + 1] = 0 when header and counts are consistent with the frame geometry, else 1.
+// starts[ntiles + 1] = 0 when the header matches the frame geometry, no tile counts more entries than it has bytes
+// (192, the last tile last_len) and the counts add up to pos (so pos <= N); else 1.
 __global__ void __launch_bounds__(1024) k_wire_scan(const uint8_t *__restrict__ wire, uint32_t ntiles_expected,
-                                                    uint32_t *__restrict__ starts)
+                                                    uint32_t last_len, uint32_t *__restrict__ starts)
 {
     __shared__ uint32_t wsum[32];
     const uint4 hd = *reinterpret_cast<const uint4 *>(wire);
@@ -636,12 +638,17 @@ __global__ void __launch_bounds__(1024) k_wire_scan(const uint8_t *__restrict__ 
     const uint32_t per = (ntiles + 1023u) / 1024u;
     const uint32_t t0 = threadIdx.x * per;
     uint32_t mine = 0;
+    bool too_many = false;
     for (uint32_t j = 0; j < per; j++)
-        if (t0 + j < ntiles) mine += cnt[t0 + j];
+        if (t0 + j < ntiles) {
+            const uint32_t c = cnt[t0 + j];
+            too_many |= c > (t0 + j + 1 == ntiles ? last_len : kWireTile);
+            mine += c;
+        }
     const uint32_t lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const uint32_t incl = warp_incl_scan(mine, lane);
     if (lane == 31) wsum[warp] = incl;
-    __syncthreads();
+    too_many = __syncthreads_or(too_many);
     if (warp == 0) {
         const uint32_t v = wsum[lane];
         const uint32_t iv = warp_incl_scan(v, lane);
@@ -656,8 +663,30 @@ __global__ void __launch_bounds__(1024) k_wire_scan(const uint8_t *__restrict__ 
         }
     if (threadIdx.x == 1023) {
         starts[ntiles] = run;
-        starts[ntiles + 1] = (header_ok && run == hd.y) ? 0u : 1u;
+        starts[ntiles + 1] = (header_ok && !too_many && run == hd.y) ? 0u : 1u;
     }
+}
+
+// client: inside every tile the offsets are strictly ascending and below the tile's length (192, the last tile
+// last_len), one warp per tile; a violation sets bit 1 of starts[ntiles + 1].  Runs only on a frame k_wire_scan found
+// consistent, so it reads no further than the frame's cvs_wire_size.  Afterwards no two entries name the same byte.
+__global__ void __launch_bounds__(256) k_wire_check(const uint8_t *__restrict__ wire, uint32_t ntiles, uint32_t last_len,
+                                                    uint32_t *starts)
+{
+    if (starts[ntiles + 1]) return;
+    const uint8_t *cnt = wire + kWireHeader;
+    const uint8_t *off = cnt + wire_pad16(ntiles);
+    const uint32_t lane = threadIdx.x & 31;
+    const uint32_t w = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, nw = (gridDim.x * blockDim.x) >> 5;
+    bool bad = false;
+    for (uint32_t t = w; t < ntiles; t += nw) {
+        const uint32_t c = cnt[t], s0 = starts[t], len = t + 1 == ntiles ? last_len : kWireTile;
+        for (uint32_t j = lane; j < c; j += 32) {
+            const uint32_t o = off[s0 + j];
+            bad |= o >= len || (j > 0 && o <= off[s0 + j - 1]);
+        }
+    }
+    if (bad) atomicOr(starts + ntiles + 1, 2u);
 }
 
 // client: frame[x] += diff (client/opencv.cpp:64-66) and/or the reference-format payload back, one warp per tile
@@ -666,6 +695,7 @@ __global__ void __launch_bounds__(256) k_wire_apply(const uint8_t *__restrict__ 
                                                     uint8_t *diff_out, unsigned int *pos_out)
 {
     if (starts[ntiles + 1]) return; // inconsistent frame: nothing is applied, the host reports it
+    // (offsets checked by k_wire_check: x < N and distinct, so the plain read-modify-write of frame[x] does not race)
     const uint32_t n = starts[ntiles];
     const uint8_t *cnt = wire + kWireHeader;
     const uint8_t *off = cnt + wire_pad16(ntiles);

@@ -208,7 +208,9 @@ cvs_status cvs_client_apply_device(uint8_t *d_frame, const int *d_xs, const uint
 #define CVS_WIRE_MAGIC 0x31575643u
 /* largest encoded frame for this geometry: size wire_out buffers with it */
 size_t cvs_wire_bound(int width, int height);
-/* total bytes of an encoded frame, read from its header (host memory); 0 if the header is not CVW1 */
+/* total bytes of an encoded frame, read from its header (host memory); 0 if the header is not CVW1.  Computed in 64
+ * bits from the sender's ntiles and pos, so it can be far larger than any real frame: a client refuses a frame whose
+ * cvs_wire_size exceeds cvs_wire_bound(width, height) before it reads (or receives) the frame's body. */
 size_t cvs_wire_size(const uint8_t *wire);
 /* cvs_submit_io that delivers the frame's payload as one CVW1 frame in wire_out (capacity cvs_wire_bound; pinned
  * memory from cvs_alloc_host lets the device store it directly).  Complete it with cvs_wait(ticket); the count is
@@ -223,8 +225,15 @@ cvs_status cvs_wire_encode_device(const int *d_xs, const uint8_t *d_diff, const 
 /* client side: decodes one CVW1 frame that lies in device memory.  Any of the outputs may be NULL:
  *   d_frame : frame[x] += diff for every entry (client/opencv.cpp:64-66)
  *   d_xs, d_diff, d_pos : the reference-format payload back (ascending indices)
- * d_scratch as above.  An inconsistent frame (bad magic, other geometry, counts that do not add up to pos) is not
- * applied at all; cvs_wire_decode_status (synchronises the stream) reports it. */
+ * d_scratch as above.  d_wire holds at least cvs_wire_size bytes of the frame and at least 16 + ntiles rounded up to
+ * 16 (what a cvs_wire_bound-sized buffer holds).  An inconsistent frame is not applied at all: no output is written,
+ * and cvs_wire_decode_status (synchronises the stream) returns CVS_ERR_INVALID.  Inconsistent means any of
+ *   - a magic other than CVW1, a tile other than CVS_WIRE_TILE, or ntiles other than this geometry's;
+ *   - a tile count above the tile's length (192; the last tile holds N - 192 * (ntiles - 1) bytes);
+ *   - counts that do not add up to pos (so pos <= N);
+ *   - inside a tile, an offset at or past the tile's length, or offsets that are not strictly ascending.
+ * The offsets are read only after the header and counts have passed, so never past cvs_wire_size bytes.  Pad bytes
+ * after the counts and after the offsets are ignored. */
 cvs_status cvs_wire_decode_device(const uint8_t *d_wire, uint32_t *d_scratch, uint8_t *d_frame, int *d_xs,
                                   uint8_t *d_diff, unsigned int *d_pos, int width, int height,
                                   void *cuda_stream);
