@@ -178,7 +178,6 @@ struct JpegDecoder {
     uint8_t *d_hmap = nullptr;
     uint32_t *d_mid_state = nullptr, *d_mid_nblk = nullptr;
     int32_t *d_mid_dc = nullptr;
-    bool hypotheses = true; // CVS_JPEG_HYPOTHESES=0: plain synchronisation rounds (measurements)
     int32_t *d_dcs = nullptr, *d_tile_dc = nullptr;
     size_t sub_cap = 0;
     unsigned int *d_changed = nullptr;
@@ -208,7 +207,7 @@ struct Slot {
     bool busy = false;
     bool copied = false; // payload fetched with cudaMemcpyAsync in cvs_wait (ev_done is valid)
     bool pushed = false; // payload already written to the caller's pinned buffers by k_payload_push
-    uint32_t spec = 0;   // entries copied speculatively behind the count (cvs_submit_io, CVS_EGRESS=2); 0 = none
+    uint32_t spec = 0;   // entries copied speculatively behind the count (cvs_submit_io); 0 = none
     uint64_t ticket = 0;
     uint8_t *u_frame = nullptr;
     int *u_xs = nullptr;
@@ -282,7 +281,6 @@ StreamKernel pick_ws_kernel(int mode, bool hi, bool refreg)
 struct cvs_stream_s {
     int width = 0, height = 0, threshold = 20, mode = 0, noise_filter = 0, ksize = 3, device = 0;
     int max_sequence = 512;
-    bool fused_gray = false; // CVS_FUSED_GRAY=1: sequences in modes 5 / 7 keep gray + histogram inside the stream kernel (A/B timing)
     uint32_t N = 0, N16 = 0, nchunks = 0, npix = 0;
     size_t Npad = 0, P16 = 0;
     bool hi = false;
@@ -291,12 +289,6 @@ struct cvs_stream_s {
     int stages = 0;     // CVS_STAGES: ring depth override (0 = default)
     bool trace = false;
     cudaEvent_t ev_base = nullptr;
-    bool push_payload = true; // CVS_PAYLOAD_PUSH=0 falls back to count round trip + copy engine
-    bool speculate = true;    // CVS_EGRESS_SPECULATE=0: cvs_submit_io never copies a predicted payload size
-    int coop = -1;             // CVS_COOP: 1 = every stream-kernel launch cooperative, 0 = none; default (-1): sequences
-                               // cooperative, single frames (the submit / exec path) plain -- see run_frames
-    int push_blocks = 0;       // CVS_PUSH_BLOCKS: grid of the payload push kernel (0 = one block per SM)
-    bool speculate_all = false; // CVS_EGRESS_SPECULATE=2: ... and 2: also for payloads above N/4 entries (measurements)
     uint32_t pred = 0;        // predicted entries of the next frame (previous count + margin)
     cvs::ConvWeights weights;
     int sms = 0;
@@ -315,7 +307,7 @@ struct cvs_stream_s {
                                         // for cvs_submit_jpeg on two streams (consecutive frames decode side by side),
                                         // set 2 for cvs_decode_jpeg_device on the caller's stream
     cudaStream_t s_jpg[2] = {nullptr, nullptr};
-    int jpeg_decoder = 0;               // 0: own decoder, nvJPEG for streams it does not cover; 1: own only; 2: nvJPEG only
+    bool jpeg_own_only = false;         // own decoder only: refuse the forms it does not cover instead of using nvJPEG
     nvjpegHandle_t jpeg = nullptr;      // cvs_submit_jpeg / cvs_decode_jpeg_device: nvJPEG handle (on first use)
     bool jpeg_batched = false;          // the handle's backend wants the batched entry points (hardware engine / GPU Huffman)
     nvjpegJpegState_t jpeg_state = nullptr; // decoder state of cvs_decode_jpeg_device
@@ -479,7 +471,7 @@ cvs_status run_frames(cvs_handle h, const uint8_t *d_frames, size_t stride, int 
     const bool binarize = (mode == 5 || mode == 7) && d_show;
     // A sequence in a binarising mode computes the gray byte and the histograms in a kernel of its own in front of the
     // plain stream kernel (k_gray_hist_seq: why, and what it measured); a single frame keeps the fused kernel.
-    const bool split_gray = binarize && nframes >= 2 && !h->fused_gray;
+    const bool split_gray = binarize && nframes >= 2;
     const int kmode = d_show && !split_gray ? mode : 0; // without a display buffer only the payload is produced
     const int piece_max = h->max_sequence < nframes ? h->max_sequence : nframes;
     const bool need_work = h->noise_filter || (txt.n && !frames_private);
@@ -646,8 +638,7 @@ cvs_status run_frames(cvs_handle h, const uint8_t *d_frames, size_t stride, int 
             // several camera streams on a GPU, whose decode kernels (cvs_jpeg.cuh) and payload pushes would otherwise
             // run strictly one after the other: 3 JPEG streams 3.8 k -> 7.1 k frames/s, raw streams unchanged.
             // (frames walked in several segments wait for the totals of ALL blocks of the previous segment: cooperative)
-            const bool coop = h->coop < 0 ? (piece > 1 || nseg > 1) : h->coop != 0;
-            if (coop)
+            if (piece > 1 || nseg > 1)
                 CU_TRY(cudaLaunchCooperativeKernel((const void *)kern, dim3(G), dim3(block_threads), args, (size_t)smem_bytes, st));
             else
                 CU_TRY(cudaLaunchKernel((const void *)kern, dim3(G), dim3(block_threads), args, (size_t)smem_bytes, st));
@@ -764,25 +755,19 @@ cvs_status cvs_create(const cvs_config *cfg, cvs_handle *out)
     if (const char *dbg = getenv("CVS_DEBUG_FLAGS")) h->debug = (uint32_t)atoi(dbg);
     if (const char *sg = getenv("CVS_STAGES")) h->stages = atoi(sg);
 #endif
-    if (const char *kk = getenv("CVS_STREAM_KERNEL")) { // both kernels are bit-exact; the switch exists for A/B timing
+    // both stream kernels are bit-exact; the tests use this to run each kernel on geometries the default does not give it
+    if (const char *kk = getenv("CVS_STREAM_KERNEL")) {
         h->use_ws = strcmp(kk, "v1") != 0;
         h->force_ws = strcmp(kk, "ws") == 0;
     }
-    if (const char *pp = getenv("CVS_PAYLOAD_PUSH")) h->push_payload = atoi(pp) != 0;
-    if (const char *sp = getenv("CVS_EGRESS_SPECULATE")) {
-        h->speculate = atoi(sp) != 0;
-        h->speculate_all = atoi(sp) == 2;
-    }
-    if (const char *tr = getenv("CVS_TRACE")) h->trace = atoi(tr) != 0;
-    if (const char *co = getenv("CVS_COOP")) h->coop = atoi(co) != 0 ? 1 : 0;
-    if (const char *fg = getenv("CVS_FUSED_GRAY")) h->fused_gray = atoi(fg) != 0;
-    if (const char *jd = getenv("CVS_JPEG_DECODER")) h->jpeg_decoder = !strcmp(jd, "own") ? 1 : (!strcmp(jd, "nvjpeg") ? 2 : 0);
-    if (const char *hy = getenv("CVS_JPEG_HYPOTHESES")) h->jd[0].hypotheses = h->jd[1].hypotheses = h->jd[2].hypotheses = atoi(hy) != 0;
-    if (const char *sb = getenv("CVS_JPEG_SUB_BITS")) { // subsequence length of the parallel Huffman decode (measurements)
+    if (const char *tr = getenv("CVS_TRACE")) h->trace = atoi(tr) != 0; // instrumentation only: timelines on stderr
+    // own decoder only (refuse, do not fall back to nvJPEG): part of the documented interface
+    if (const char *jd = getenv("CVS_JPEG_DECODER")) h->jpeg_own_only = !strcmp(jd, "own");
+    // subsequence length of the parallel Huffman decode: tests reach 128-bit subsequences (whole-subsequence rounds) only here
+    if (const char *sb = getenv("CVS_JPEG_SUB_BITS")) {
         const int v = atoi(sb);
         if (v >= 64 && v <= 65536 && v % 32 == 0) h->jd[0].sub_bits = h->jd[1].sub_bits = h->jd[2].sub_bits = (uint32_t)v;
     }
-    if (const char *pb = getenv("CVS_PUSH_BLOCKS")) h->push_blocks = atoi(pb);
     memset(&h->weights, 0, sizeof h->weights);
     if (cfg->noise_filter) memcpy(h->weights.k, cfg->kweights, sizeof(float) * cfg->ksize * cfg->ksize);
     const cvs_status st = init_device_state(h, cfg);
@@ -932,21 +917,18 @@ static cvs_status jpeg_decode_nvjpeg(cvs_handle h, nvjpegJpegState_t *state, con
     if (!nj) return fail(CVS_ERR_NODEVICE, "libnvjpeg could not be loaded: %s", dlerror());
     if (!h->jpeg) {
         // Backend, in order of preference: the hardware JPEG engine, GPU-assisted Huffman decoding (both through the
-        // batched entry points, batch of one), the library's default single-image decode.  CVS_JPEG_BACKEND=hw|gpu|default
-        // pins one.  Chroma is upsampled WITH interpolation, as libjpeg-turbo (OpenCV, the reference's decoder) does by
-        // default: on the reference's fixture frames that brings the decoded pixels from max |d| 26 / 63 % of the bytes
-        // differing to max |d| 5 / 55 %, and the K1 count from 404,321 to 370,732 (OpenCV: 369,350).  CVS_JPEG_INTERP=0
-        // turns it off (measurements).
-        const char *want = getenv("CVS_JPEG_BACKEND");
-        const unsigned flags = (getenv("CVS_JPEG_INTERP") && !atoi(getenv("CVS_JPEG_INTERP"))) ? NVJPEG_FLAGS_DEFAULT
-                                                                                             : NVJPEG_FLAGS_UPSAMPLING_WITH_INTERPOLATION;
+        // batched entry points, batch of one), the library's default single-image decode.  Chroma is upsampled WITH
+        // interpolation, as libjpeg-turbo (OpenCV, the reference's decoder) does by default: on the reference's fixture
+        // frames that brings the decoded pixels from max |d| 26 / 63 % of the bytes differing to max |d| 5 / 55 %, and the
+        // K1 count from 404,321 to 370,732 (OpenCV: 369,350).
+        const unsigned flags = NVJPEG_FLAGS_UPSAMPLING_WITH_INTERPOLATION;
         nvjpegStatus_t e = NVJPEG_STATUS_NOT_INITIALIZED;
         const bool can_batch = nj->CreateEx && nj->BatchedInit && nj->Batched;
-        if (can_batch && (!want || !strcmp(want, "hw"))) {
+        if (can_batch) {
             e = nj->CreateEx(NVJPEG_BACKEND_HARDWARE, nullptr, nullptr, flags, &h->jpeg);
             h->jpeg_batched = e == NVJPEG_STATUS_SUCCESS;
         }
-        if (e != NVJPEG_STATUS_SUCCESS && can_batch && (!want || !strcmp(want, "gpu"))) {
+        if (e != NVJPEG_STATUS_SUCCESS && can_batch) {
             e = nj->CreateEx(NVJPEG_BACKEND_GPU_HYBRID, nullptr, nullptr, flags, &h->jpeg);
             h->jpeg_batched = e == NVJPEG_STATUS_SUCCESS;
         }
@@ -1107,7 +1089,6 @@ static cvs_status jpeg_decode_own(cvs_handle h, JpegDecoder &jd, const uint8_t *
         J::k_entropy_restart<<<(rp.nseg + 127) / 128, 128, 0, st>>>(rp);
     } else {
     // ---- one cooperative launch: scratch cleared, FF 00 -> FF, Huffman decode (hypotheses, rounds, prefix sums, write)
-    // (entry states start as zero = "a block of phase 0 starts here": the first guess when the hypotheses are switched off)
     if (!jd.coop_blocks_per_sm) {
         CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&jd.coop_blocks_per_sm, J::k_entropy, J::kEntropyThreads, 0));
         if (jd.coop_blocks_per_sm < 1) return fail(CVS_ERR_INTERNAL, "k_entropy does not fit an SM");
@@ -1146,13 +1127,11 @@ static cvs_status jpeg_decode_own(cvs_handle h, JpegDecoder &jd, const uint8_t *
     ep.hym = jd.d_hym;
     ep.hwm = jd.d_hwm;
     ep.hmap = jd.d_hmap;
-    ep.hypotheses = jd.hypotheses ? 1u : 0u;
     ep.changed = jd.d_changed;
     ep.coef = jd.d_coef;
     ep.status = d_status;
-    ep.debug = getenv("CVS_JPEG_TRACE") ? (uint32_t)atoi(getenv("CVS_JPEG_TRACE")) : 0u;
     // one thread per subsequence and phase hypothesis in the first phases, one per subsequence afterwards
-    const uint32_t ntiles = (g.nsub_max * (jd.hypotheses ? (uint32_t)g.bpm : 1u) + J::kEntropyThreads - 1) / J::kEntropyThreads;
+    const uint32_t ntiles = (g.nsub_max * (uint32_t)g.bpm + J::kEntropyThreads - 1) / J::kEntropyThreads;
     const uint32_t egrid = std::max(1u, std::min(ntiles, (uint32_t)(jd.coop_blocks_per_sm * h->sms)));
     void *eargs[] = {&ep};
     CU_TRY(cudaLaunchCooperativeKernel((const void *)J::k_entropy, dim3(egrid), dim3(J::kEntropyThreads), eargs, 0, st));
@@ -1183,12 +1162,10 @@ static cvs_status jpeg_decode_own(cvs_handle h, JpegDecoder &jd, const uint8_t *
 static cvs_status jpeg_decode(cvs_handle h, int set, nvjpegJpegState_t *state, const uint8_t *jpeg, size_t jpeg_bytes,
                               uint8_t *d_out, cudaStream_t st, unsigned int *d_status)
 {
-    if (h->jpeg_decoder != 2) {
-        bool unsupported = false;
-        const cvs_status e = jpeg_decode_own(h, h->jd[set], jpeg, jpeg_bytes, d_out, st, d_status, &unsupported);
-        if (e || !unsupported) return e;
-        if (h->jpeg_decoder == 1) return fail(CVS_ERR_INVALID, "JPEG form not covered by the built-in decoder (CVS_JPEG_DECODER=own)");
-    }
+    bool unsupported = false;
+    const cvs_status e = jpeg_decode_own(h, h->jd[set], jpeg, jpeg_bytes, d_out, st, d_status, &unsupported);
+    if (e || !unsupported) return e;
+    if (h->jpeg_own_only) return fail(CVS_ERR_INVALID, "JPEG form not covered by the built-in decoder (CVS_JPEG_DECODER=own)");
     return jpeg_decode_nvjpeg(h, state, jpeg, jpeg_bytes, d_out, st);
 }
 
@@ -1277,17 +1254,15 @@ static cvs_status submit_common(cvs_handle h, const uint8_t *frame, uint8_t *dif
     // only with a prediction from a previous frame, and never more entries than the caller's buffers hold (N)
     if (wire_out) {
         // nothing else to fetch: the encoded frame carries the count
-    } else if (h->speculate && diff_out != frame && h->pred != 0 && h->pred >= spec_lo &&
-               (h->pred <= h->N / 4u || h->speculate_all)) {
+    } else if (diff_out != frame && h->pred != 0 && h->pred >= spec_lo && h->pred <= h->N / 4u) {
         const size_t guess = round_up(h->pred, 4);
         s.spec = (uint32_t)(guess > h->N ? h->N : guess);
     } else {
-        s.pushed = h->push_payload && mapped_device_pointer(diff_out, &dev_diff) && mapped_device_pointer(xs, &dev_xs) &&
+        s.pushed = mapped_device_pointer(diff_out, &dev_diff) && mapped_device_pointer(xs, &dev_xs) &&
                    ((uintptr_t)dev_diff % 16 == 0) && ((uintptr_t)dev_xs % 16 == 0);
     }
     if (s.pushed && !wire_out) {
-        cvs::k_payload_push<<<h->push_blocks > 0 ? h->push_blocks : h->sms, 256, 0, h->s_d2h>>>(s.d_xs, s.d_diff, s.d_pos, (int *)dev_xs,
-                                                                                             (uint8_t *)dev_diff, cap);
+        cvs::k_payload_push<<<h->sms, 256, 0, h->s_d2h>>>(s.d_xs, s.d_diff, s.d_pos, (int *)dev_xs, (uint8_t *)dev_diff, cap);
         CU_TRY(cudaGetLastError());
         h->launches++;
     }

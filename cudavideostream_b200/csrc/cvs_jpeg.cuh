@@ -564,19 +564,10 @@ struct EntropyParams {
     uint32_t *hx, *hy, *hw;   // [nsub_max * bpm] exit states of the phase hypotheses: fresh / followed one / two subsequences further
     uint32_t *hym, *hwm;      // [nsub_max * bpm] state of the Y / W runs in the middle of their subsequence (hym[0]: the exact run of subsequence 0)
     uint8_t *hmap;            // [nsub_max][16] successor of candidate c of boundary i-1 among the candidates of boundary i
-    uint32_t hypotheses;      // 0: plain rounds from the guess "a block starts here" (A/B measurements)
     unsigned int *changed;    // [kRoundCounters] states changed in a round, three counters in rotation
     int16_t *coef;            // [nblocks][64], zeroed
     unsigned int *status;
-    uint32_t debug;           // CVS_JPEG_TRACE=1: block 0 prints the time of every phase (measurements)
 };
-
-__device__ __forceinline__ unsigned long long jpg_now_ns()
-{
-    unsigned long long t;
-    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-    return t;
-}
 
 __global__ void __launch_bounds__(kEntropyThreads) k_entropy(const EntropyParams p)
 {
@@ -597,8 +588,6 @@ __global__ void __launch_bounds__(kEntropyThreads) k_entropy(const EntropyParams
     __syncthreads();
     const TableRef tbr = table_ref(&tb);
     const Geometry g = p.g;
-    const bool trace = p.debug && blockIdx.x == 0 && tid == 0;
-    unsigned long long t_prev = trace ? jpg_now_ns() : 0ull;
 
     // ---- clear what must start as zero (round counters, entry states, coefficients, the unstuffed string's buffer) and
     //      count the bytes that stay; then compact them.  Two grid barriers instead of a memset and two launches.
@@ -620,10 +609,6 @@ __global__ void __launch_bounds__(kEntropyThreads) k_entropy(const EntropyParams
             unstuff_write_block(vb, nvb, p.raw, p.raw_len, p.block_kept, p.block_marks, p.unst, p.total_bits_out, p.seg_start, p.seg_cap,
                                 p.total_marks_out, wsum, s_tile_base);
         grid.sync();
-        if (trace) {
-            printf("clear + unstuff: %llu ns\n", jpg_now_ns() - t_prev);
-            t_prev = jpg_now_ns();
-        }
     }
     const uint32_t T = __ldcg(p.total_bits);
     const uint32_t nsub = (T + g.sub_bits - 1) / g.sub_bits; // <= nsub_max
@@ -634,10 +619,10 @@ __global__ void __launch_bounds__(kEntropyThreads) k_entropy(const EntropyParams
     // compare and a select per token.  Measured and not adopted: the state at EVERY 128-bit boundary, stored from a
     // branch -- confirming round 28 -> 8 us, but with 32 lanes crossing boundaries at different tokens the branch is
     // taken by some lane in nearly every iteration and the hypothesis phases go from 105 to 160 us.)
-    const bool half = p.hypotheses && g.sub_bits % 256u == 0 && p.mid.nsplit % 2u == 0;
+    const bool half = g.sub_bits % 256u == 0 && p.mid.nsplit % 2u == 0;
     const uint32_t hstep = half ? 2u : 1u;
     // ---- phase hypotheses (see the header): seed entry[] with the states the true token sequence passes through
-    if (p.hypotheses) {
+    {
         const uint32_t B = (uint32_t)g.bpm, nh = nsub * B, gstride = gridDim.x * kEntropyThreads;
         const uint32_t first = blockIdx.x * kEntropyThreads + tid;
         // X: a block of phase h starts at the subsequence boundary; Y, W: that sequence followed through the next and the
@@ -752,10 +737,6 @@ __global__ void __launch_bounds__(kEntropyThreads) k_entropy(const EntropyParams
         }
         __threadfence();
         grid.sync();
-        if (trace) {
-            printf("hypotheses: %llu ns\n", jpg_now_ns() - t_prev);
-            t_prev = jpg_now_ns();
-        }
     }
 
     Geometry gr = g;
@@ -797,14 +778,7 @@ __global__ void __launch_bounds__(kEntropyThreads) k_entropy(const EntropyParams
                 if (i + 1 < nsubr) atomicAdd(counter, 1u);
             }
         }
-        const unsigned long long t_run = trace ? jpg_now_ns() : 0ull;
         grid.sync();
-        if (trace) {
-            const unsigned long long t_now = jpg_now_ns();
-            printf("round %u: run %llu ns, barrier %llu ns, %u states changed\n", round, t_run - t_prev, t_now - t_run,
-                   __ldcg(counter));
-            t_prev = t_now;
-        }
         if (__ldcg(counter) == 0) {
             converged = true;
             break;
@@ -902,10 +876,6 @@ __global__ void __launch_bounds__(kEntropyThreads) k_entropy(const EntropyParams
         }
     }
     grid.sync();
-    if (trace) {
-        printf("prefix sums: %llu ns\n", jpg_now_ns() - t_prev);
-        t_prev = jpg_now_ns();
-    }
     // ---- write pass: one thread per G bits, from the states the counting runs left at the inner boundaries
     {
         Geometry gw = gr;
@@ -926,7 +896,6 @@ __global__ void __launch_bounds__(kEntropyThreads) k_entropy(const EntropyParams
             run_subsequence<true>(tbr, gw, p.words, T, j, e, s_nat, p.coef, blk0, d0, d1, d2);
         }
     }
-    if (trace) printf("write pass (block 0): %llu ns\n", jpg_now_ns() - t_prev);
     // the string must hold exactly the image's blocks (padding bits after the last block decode to no complete block
     // in a well-formed stream; more or fewer blocks means a damaged frame)
     if (total_blocks_seen && total_blocks_seen < gr.nblocks) atomicOr(p.status, kJpegBlockCount);

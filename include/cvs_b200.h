@@ -130,7 +130,7 @@ cvs_status cvs_wait(cvs_handle h, uint64_t ticket);
  * frame (which is then left untouched): for callers that keep captured frames in a pinned ring.
  * diff_out (capacity N bytes) and xs (capacity N ints) hold the payload in [0, *pos); what lies past *pos is
  * unspecified on this entry point: the copy engine fetches a predicted number of entries right behind the
- * count instead of waiting for the host to read it (CVS_EGRESS_SPECULATE=0 turns that off). */
+ * count instead of waiting for the host to read it. */
 cvs_status cvs_submit_io(cvs_handle h, const uint8_t *frame, uint8_t *diff_out, uint8_t *show,
                          const char *text, unsigned int *pos, int *xs, uint64_t *ticket);
 
@@ -255,7 +255,7 @@ cvs_status cvs_wire_decode_status(const uint32_t *d_scratch, int width, int heig
  *   intervals (one thread per interval then); frames without a DHT segment use the standard tables (MJPG).
  *   Other forms (progressive, arithmetic coding, other samplings) go to nvJPEG (loaded with dlopen on first use), whose pixels
  *   are close to but not identical with libjpeg-turbo's (<= 5 apart on the fixture frames); CVS_JPEG_DECODER=own
- *   refuses them instead, CVS_JPEG_DECODER=nvjpeg sends everything there (measurements).
+ *   refuses them instead.
  *   A damaged entropy-coded segment never writes outside the frame; when the decoder notices (the stream holds
  *   fewer blocks than the image) cvs_wait / cvs_sequence_status return CVS_ERR_INVALID for that frame.  Every
  *   well-formed stream decodes, however unfriendly its code: the parallel decode falls back to as many rounds as it

@@ -30,5 +30,5 @@ for d in (10000, 100000, 500000):
         return tot
     run(8)
     t0 = time.perf_counter(); tot = run(F); dt = time.perf_counter() - t0
-    print(f"push={os.environ.get('CVS_PAYLOAD_PUSH','1')} spec={os.environ.get('CVS_EGRESS_SPECULATE','1')} d={d} {F/dt:8.0f} fps  {dt/F*1e6:7.1f} us/frame  payload {5*tot/F/1e6:.2f} MB/frame  last {s.timing()}")
+    print(f"d={d} {F/dt:8.0f} fps  {dt/F*1e6:7.1f} us/frame  payload {5*tot/F/1e6:.2f} MB/frame  last {s.timing()}")
     s.close()

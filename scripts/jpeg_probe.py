@@ -1,11 +1,10 @@
 """Decode rate of cvs_decode_jpeg_device on the reference's fixture frames: the library's own decoder (cvs_jpeg.cuh) at
-several subsequence lengths, with 1, 2 and 4 streams decoding side by side, and nvJPEG's backends beside it (rate and
-distance from OpenCV's pixels).  Run on the GPU box: python scripts/jpeg_probe.py"""
+several subsequence lengths, with 1, 2 and 4 streams decoding side by side (rate and distance from OpenCV's pixels).
+Run on the GPU box: python scripts/jpeg_probe.py"""
 import os, subprocess, sys, time
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 if len(sys.argv) == 1:
     runs = [("own", dict(CVS_JPEG_DECODER="own", CVS_JPEG_SUB_BITS=str(sb))) for sb in (256, 512, 1024, 2048, 4096)]
-    runs += [("nvjpeg", dict(CVS_JPEG_DECODER="nvjpeg", CVS_JPEG_BACKEND=be, CVS_JPEG_INTERP="1")) for be in ("hw", "gpu", "default")]
     for name, extra in runs:
         env = dict(os.environ, **extra)
         r = subprocess.run([sys.executable, __file__, "run"], env=env, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, timeout=300)
