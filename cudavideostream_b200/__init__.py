@@ -9,8 +9,8 @@ call needs the built library and an sm_100 GPU and fails loudly otherwise.
 """
 from .api import (CVSError, CUDACore, Stream, alloc_host, device_count, library_path, load_library,  # noqa: F401
                   MODE_NONE, MODE_HEAT_MAP, MODE_RED_BLACK, MODE_RED_OVERLAP, MODE_GRAY_WEIGHTED,
-                  MODE_BINARIZE, MODE_GRAY_AVERAGE, MODE_BINARIZE_AVERAGE)
+                  MODE_BINARIZE, MODE_GRAY_AVERAGE, MODE_BINARIZE_AVERAGE, MAX_BATCH, run_batch_device, submit_io_batch)
 from . import filters, sharding, synth, wire  # noqa: F401
 
 __all__ = ["CVSError", "CUDACore", "Stream", "alloc_host", "device_count", "library_path", "load_library",
-           "filters", "sharding", "synth", "wire"]
+           "run_batch_device", "submit_io_batch", "filters", "sharding", "synth", "wire"]

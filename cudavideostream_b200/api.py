@@ -16,6 +16,7 @@ _LIB_PATH = os.environ.get("CVS_B200_LIB") or os.path.join(_HERE, "libcvs_b200.s
 
 MODE_NONE, MODE_HEAT_MAP, MODE_RED_BLACK, MODE_RED_OVERLAP = 0, 1, 2, 3
 MODE_GRAY_WEIGHTED, MODE_BINARIZE, MODE_GRAY_AVERAGE, MODE_BINARIZE_AVERAGE = 4, 5, 6, 7
+MAX_BATCH = 64  # CVS_MAX_BATCH
 
 CHARS_STR = "0123456789BFPSWbkps :/"  # server/include/common.h:13
 
@@ -62,6 +63,10 @@ SIGNATURES = {
     "cvs_run_sequence_device": (C.c_int, [_vp, _vp, _sz, C.c_int, _vp, _vp, _vp, _sz, _vp, _sz, C.c_char_p, _vp]),
     "cvs_sequence_status": (C.c_int, [_vp]),
     "cvs_launch_count": (C.c_uint64, [_vp]),
+    "cvs_run_batch_device": (C.c_int, [C.POINTER(_vp), C.c_int, C.POINTER(_vp), _vp, _vp, _vp, _sz, _vp, _sz,
+                                       C.POINTER(C.c_char_p), _vp]),
+    "cvs_submit_io_batch": (C.c_int, [C.POINTER(_vp), C.c_int, C.POINTER(_vp), C.POINTER(_vp), C.POINTER(_vp),
+                                      C.POINTER(C.c_char_p), C.POINTER(_vp), C.POINTER(_vp), C.POINTER(C.c_uint64)]),
     "cvs_heat_map_device": (C.c_int, [_vp, _vp, _vp, C.c_int, C.c_int, _vp]),
     "cvs_red_map_device": (C.c_int, [_vp, _vp, _vp, C.c_int, C.c_int, C.c_int, _vp]),
     "cvs_grayscale_device": (C.c_int, [_vp, _vp, C.c_int, C.c_int, C.c_int, C.c_int, _vp]),
@@ -271,6 +276,36 @@ class Stream:
             self.close()
         except Exception:
             pass
+
+
+def _ptrs(values):
+    """n addresses (None / 0 = NULL) as a C array of void*, or NULL for None."""
+    return None if values is None else (_vp * len(values))(*[v or None for v in values])
+
+
+def _texts(texts):
+    return None if texts is None else (C.c_char_p * len(texts))(*[None if t is None else t.encode() for t in texts])
+
+
+def run_batch_device(streams, d_frames, d_pos: int, d_xs: int, d_diff: int, capacity: int, d_show: int = 0,
+                     show_stride: int = 0, texts=None, cuda_stream: int = 0) -> None:
+    """cvs_run_batch_device: one device-resident frame of each stream (d_frames[i] for streams[i]) in one stream-kernel
+    launch; outputs laid out like a sequence indexed by camera.  texts: None or one entry (str or None) per stream."""
+    n = len(streams)
+    hs = (_vp * n)(*[s._h.value for s in streams])
+    _check(load_library().cvs_run_batch_device(hs, n, _ptrs(d_frames), d_pos, d_xs, d_diff, capacity, d_show or None,
+                                               show_stride, _texts(texts), cuda_stream or None))
+
+
+def submit_io_batch(streams, frames, diff_out, pos, xs, show=None, texts=None) -> list:
+    """cvs_submit_io_batch: one frame of each stream; returns the tickets (tickets[i] is completed by streams[i].wait).
+    frames, diff_out, pos, xs (and show, None entries allowed) are lists of host addresses, one per stream."""
+    n = len(streams)
+    hs = (_vp * n)(*[s._h.value for s in streams])
+    tk = (C.c_uint64 * n)()
+    _check(load_library().cvs_submit_io_batch(hs, n, _ptrs(frames), _ptrs(diff_out), _ptrs(show), _texts(texts),
+                                              _ptrs(pos), _ptrs(xs), tk))
+    return list(tk)
 
 
 class matsz:

@@ -150,9 +150,32 @@ __device__ __forceinline__ void flush_diff_shifted(uint32_t sv, uint8_t *df_out,
     if (lane < 8 && e1 < (lane < 4 ? head : n)) stg_stream_u8(dg + e1, lds_u8(sv + e1));
 }
 
-template <int MODE, bool HI, bool REFREG>
-__global__ void __launch_bounds__(kWsThreads, 1) k_stream_ws(const StreamParams p)
+// Batches: one frame of each of up to kMaxBatch camera streams in one launch (k_stream_ws_batch).  Step q is camera q
+// (every frame fits one pass, nseg == 1); the pointers of camera q come from this table, which travels in the kernel
+// parameters (kMaxBatch * 72 bytes): no upload, nothing to keep alive after the launch.
+constexpr int kMaxBatch = 64;
+struct BatchCam {
+    const uint8_t *frame;  // the camera's frame (16-byte aligned)
+    uint8_t *ref;          // its reference frame
+    unsigned int *pos;     // its count
+    int *xs;               // its payload (capacity StreamParams::cap)
+    uint8_t *diff;
+    uint8_t *show;         // its display frame (MODE 1,2,3,4,6)
+    uint8_t *gray1;        // MODE 5/7: its gray bytes and histogram
+    unsigned int *hist;
+    unsigned int *status;  // its StatusBits
+};
+struct BatchTable {
+    BatchCam cam[kMaxBatch];
+};
+
+// The body of k_stream_ws and of k_stream_ws_batch.  BATCH: step q is the single pass of camera q, every per-frame
+// pointer comes from cams[q], and the reference goes through L2 step by step (each step is another camera's reference:
+// the !REFREG reload / store, at the camera's address).
+template <int MODE, bool HI, bool REFREG, bool BATCH>
+__device__ __forceinline__ void ws_body(const StreamParams &p, const BatchCam *cams)
 {
+    static_assert(!(BATCH && REFREG), "a batch reloads the reference of every step");
     extern __shared__ __align__(128) unsigned char smem[];
     // role of a warp: the scheduler arbitrates highest-warp-id-first, so which group gets the upper half decides who
     // wins when both want an issue slot
@@ -193,14 +216,15 @@ __global__ void __launch_bounds__(kWsThreads, 1) k_stream_ws(const StreamParams 
     };
     // one thread: refill ring stage st with the slice of step q
     auto issue = [&](uint32_t q, uint32_t st) {
-        const uint32_t t = REFREG ? q : q / p.nseg, s = REFREG ? 0u : q - t * p.nseg;
+        const uint32_t t = (REFREG || BATCH) ? q : q / p.nseg, s = (REFREG || BATCH) ? 0u : q - t * p.nseg;
         uint32_t off, bytes;
         slice(s, off, bytes);
         if (bytes) {
             const uint64_t pol = l2_policy_evict_first();
             asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); // parked bytes were written through the generic proxy
             mbar_expect_tx(bar_full + 8 * st, bytes);
-            bulk_g2s(stage_addr + st * stage_bytes, p.frames + (size_t)t * p.frame_stride + off, bytes, bar_full + 8 * st, pol);
+            bulk_g2s(stage_addr + st * stage_bytes, (BATCH ? cams[t].frame : p.frames + (size_t)t * p.frame_stride) + off, bytes,
+                     bar_full + 8 * st, pol);
         } else {
             // a block whose slice lies past the end of the frame still hands the stage over: the front warps must not
             // run ahead of the back warps by more than the ring (fdone[st] would complete twice before it is waited for)
@@ -266,11 +290,12 @@ __global__ void __launch_bounds__(kWsThreads, 1) k_stream_ws(const StreamParams 
             coff = ok ? (uint32_t)(c * kChunkBytes) : 0u;
             nv = ok ? min(N - coff, (uint32_t)kChunkBytes) : 0u;
         };
-        auto load_ref = [&]() {
+        // rb: the reference frame of the step's camera (p.ref unless BATCH)
+        auto load_ref = [&](uint8_t *rb) {
             if (nv) {
 #pragma unroll
                 for (int v = 0; v < kChunkWords / 4; v++) {
-                    uint4 a = ldg_keep(p.ref + coff + voff(v), keep);
+                    uint4 a = ldg_keep(rb + coff + voff(v), keep);
                     r[4 * v] = a.x; r[4 * v + 1] = a.y; r[4 * v + 2] = a.z; r[4 * v + 3] = a.w;
                 }
             } else {
@@ -278,19 +303,23 @@ __global__ void __launch_bounds__(kWsThreads, 1) k_stream_ws(const StreamParams 
                 for (int k = 0; k < kChunkWords; k++) r[k] = 0;
             }
         };
-        auto store_ref = [&]() {
+        auto store_ref = [&](uint8_t *rb) {
 #pragma unroll
             for (int v = 0; v < kChunkWords / 4; v++)
-                stg_keep(p.ref + coff + voff(v), make_uint4(r[4 * v], r[4 * v + 1], r[4 * v + 2], r[4 * v + 3]), keep);
+                stg_keep(rb + coff + voff(v), make_uint4(r[4 * v], r[4 * v + 1], r[4 * v + 2], r[4 * v + 3]), keep);
         };
         geometry(0);
-        if (REFREG) load_ref();
+        if (REFREG) load_ref(p.ref);
 
         uint32_t phase = 0, st = 0, t = 0, s = 0;
         for (uint32_t q = 0; q < nsteps; q++) {
             if (!REFREG) {
-                geometry(s);
-                load_ref(); // L2 hit; issued before the wait on the frame slice
+                if (!BATCH) geometry(s);
+                // a batch has one geometry for all its steps; opaque here, so that what derives from it is recomputed per
+                // step instead of being held (spilled) across the loop
+                else asm volatile("" : "+r"(coff), "+r"(nv));
+                load_ref(BATCH ? cams[q].ref : p.ref); // L2 hit (a batch: the camera's reference, from HBM unless
+                                                       // recently used); issued before the wait on the frame slice
             }
             wait_bar(bar_full + 8 * st, (phase >> st) & 1u, CVS_WS_SLEEP_FULL); // completes at once for an empty slice (see issue())
             phase ^= 1u << st;
@@ -351,21 +380,21 @@ __global__ void __launch_bounds__(kWsThreads, 1) k_stream_ws(const StreamParams 
 #pragma unroll
                         for (int k = 0; k < kGroupWords; k++) ad[k] = absdiff4(cg[k], rg[k]);
                         group_heat(ad, slut, o);
-                        store_group(p.show + (size_t)t * p.show_stride + goff, o, gnv);
+                        store_group((BATCH ? cams[q].show : p.show + (size_t)t * p.show_stride) + goff, o, gnv);
                     } else if (MODE == kModeRedBlack || MODE == kModeRedOverlap) {
                         uint32_t mk[kGroupWords];
 #pragma unroll
                         for (int k = 0; k < kGroupWords; k++) mk[k] = changed80<HI>(absdiff4(cg[k], rg[k]), p.addc);
                         group_red<MODE == kModeRedOverlap>(mk, rg, o);
-                        store_group(p.show + (size_t)t * p.show_stride + goff, o, gnv);
+                        store_group((BATCH ? cams[q].show : p.show + (size_t)t * p.show_stride) + goff, o, gnv);
                     } else if (MODE == kModeGrayWeighted || MODE == kModeGrayAverage) {
                         group_gray3<kGrayW>(cg, o);
-                        store_group(p.show + (size_t)t * p.show_stride + goff, o, gnv);
+                        store_group((BATCH ? cams[q].show : p.show + (size_t)t * p.show_stride) + goff, o, gnv);
                     } else if (kBinarize) {
                         uint32_t g4[4];
                         group_gray1<kGrayW>(cg, g4);
                         const uint32_t npx = gnv / 3u;
-                        uint8_t *gdst = p.gray1 + (size_t)t * p.gray_stride + goff / 3u;
+                        uint8_t *gdst = (BATCH ? cams[q].gray1 : p.gray1 + (size_t)t * p.gray_stride) + goff / 3u;
                         if (npx == (uint32_t)kGroupPixels) stg_keep(gdst, make_uint4(g4[0], g4[1], g4[2], g4[3]), keep);
 #pragma unroll
                         for (int px = 0; px < kGroupPixels; px++) {
@@ -429,7 +458,7 @@ __global__ void __launch_bounds__(kWsThreads, 1) k_stream_ws(const StreamParams 
             }
             if (m[0] | m[1] | m[2]) {
                 if (REFREG) dirty = true;
-                else store_ref();
+                else store_ref(BATCH ? cams[q].ref : p.ref);
             }
             const uint32_t cnt = (uint32_t)__popc(m[0]) + (uint32_t)__popc(m[1]) + (uint32_t)__popc(m[2]);
             // hand the step to the back warps: (mask, count) per chunk, entries of this warp
@@ -455,7 +484,7 @@ __global__ void __launch_bounds__(kWsThreads, 1) k_stream_ws(const StreamParams 
                 }
 #endif
             }
-            if (kBinarize && s == p.nseg - 1) {
+            if (kBinarize && (BATCH || s == p.nseg - 1)) {
                 // histogram of the frame complete: flush and clear (front warps only: named barrier 1)
                 asm volatile("bar.sync 1, %0;" ::"n"(kWsFrontThreads) : "memory");
                 for (uint32_t i = tid; i < 256; i += kWsFrontThreads) {
@@ -465,17 +494,17 @@ __global__ void __launch_bounds__(kWsThreads, 1) k_stream_ws(const StreamParams 
                         hv += shist[i * kWsHistCopies + c];
                         shist[i * kWsHistCopies + c] = 0;
                     }
-                    if (hv) atomicAdd(p.hist + (size_t)t * 256 + i, hv);
+                    if (hv) atomicAdd((BATCH ? cams[q].hist : p.hist + (size_t)t * 256) + i, hv);
                 }
                 asm volatile("bar.sync 1, %0;" ::"n"(kWsFrontThreads) : "memory");
             }
             __syncwarp();
             if (lane == 0) mbar_arrive(bar_fdone + 8 * st); // release: the warp's shared stores above are visible to the waiters
-            if (REFREG) ++t;
+            if (REFREG || BATCH) ++t;
             else if (++s == p.nseg) { s = 0; ++t; }
             if (++st == nstages) st = 0;
         }
-        if (REFREG && dirty) store_ref();
+        if (REFREG && dirty) store_ref(p.ref);
     } else {
         // =====================================================================================================
         // BACK: block scan, cross-block look-back, emission of the (index, value) entries
@@ -503,6 +532,7 @@ __global__ void __launch_bounds__(kWsThreads, 1) k_stream_ws(const StreamParams 
 
         uint32_t ph_f = 0, ph_b = 0, st = 0, t = 0, s = 0;
         for (uint32_t q = 0; q < nsteps; q++) {
+            if (BATCH) asm volatile("" : "+l"(sxs), "+l"(sd)); // (as the front's geometry: recomputed, not spilled)
             // byte offset of lane 0's chunk in the frame (chunk S of the warp starts 96*S bytes later)
             const uint32_t wcoff = p.index_base + (uint32_t)((((uint64_t)s * G + b) * p.cps + c0) * kChunkBytes);
             // global-offset slot of the step: 2 x nstages slots, because a sparse warp lets its stage go before it waits
@@ -550,7 +580,7 @@ __global__ void __launch_bounds__(kWsThreads, 1) k_stream_ws(const StreamParams 
             if (p.debug & 2u) { // timing experiment: no emission at all (results wrong by construction)
                 release_stage();
                 ph_b ^= 1u << bslot;
-                if (REFREG) ++t;
+                if (REFREG || BATCH) ++t;
                 else if (++s == p.nseg) { s = 0; ++t; }
                 if (++st == nstages) st = 0;
                 continue;
@@ -601,18 +631,19 @@ __global__ void __launch_bounds__(kWsThreads, 1) k_stream_ws(const StreamParams 
                 if (lane == 0) {
                     sbase[bslot] = base;
                     if (b == G - 1) {
-                        if (!REFREG) desc_publish(row + G, ((unsigned long long)p.epoch << 32) | (base + total));
-                        if (REFREG || s == p.nseg - 1) p.pos[t] = base + total;
+                        if (!REFREG && !BATCH) desc_publish(row + G, ((unsigned long long)p.epoch << 32) | (base + total));
+                        if (BATCH) *cams[q].pos = base + total;
+                        else if (REFREG || s == p.nseg - 1) p.pos[t] = base + total;
                     }
-                    if ((size_t)base + total > p.cap) atomicOr(p.status, kStatusCapacity);
+                    if ((size_t)base + total > p.cap) atomicOr(BATCH ? cams[q].status : p.status, kStatusCapacity);
                     mbar_arrive(bar_base + 8 * bslot);
                 }
             }
             if (wtotal) {
                 wait_bar(bar_base + 8 * bslot, (ph_b >> bslot) & 1u, CVS_WS_SLEEP_BACK);
                 const uint32_t base = *reinterpret_cast<volatile uint32_t *>(sbase + bslot);
-                int *xs_out = p.xs + (size_t)t * p.cap;
-                uint8_t *df_out = p.diff + (size_t)t * p.cap;
+                int *xs_out = BATCH ? cams[q].xs : p.xs + (size_t)t * p.cap;
+                uint8_t *df_out = BATCH ? cams[q].diff : p.diff + (size_t)t * p.cap;
                 asm volatile("" : "+l"(xs_out), "+l"(df_out)); // keep the frame offset out of the emission loops
                 const size_t g0 = (size_t)base + wexc;
                 if (sparse) {
@@ -637,11 +668,28 @@ __global__ void __launch_bounds__(kWsThreads, 1) k_stream_ws(const StreamParams 
             }
             ph_b ^= 1u << bslot; // every step completes its bar_base slot exactly once, waited for or not
             if (!sparse) release_stage(); // a dense warp stores straight out of the stage
-            if (REFREG) ++t;
+            if (REFREG || BATCH) ++t;
             else if (++s == p.nseg) { s = 0; ++t; }
             if (++st == nstages) st = 0;
         }
     }
+    // (a batch's watchdog bits go to the first camera's word during the launch: the later steps of a thread that gave
+    // up are not run, so every camera is told)
+    if (BATCH && tripped)
+        for (uint32_t i = 0; i < nsteps; i++) atomicOr(cams[i].status, kStatusWatchdog);
+}
+
+template <int MODE, bool HI, bool REFREG>
+__global__ void __launch_bounds__(kWsThreads, 1) k_stream_ws(const StreamParams p)
+{
+    ws_body<MODE, HI, REFREG, false>(p, nullptr);
+}
+
+// one frame of each of p.nframes cameras (p.nseg == 1; p.frames, ref, pos, xs, diff, show, gray1, hist unused: see cams)
+template <int MODE, bool HI>
+__global__ void __launch_bounds__(kWsThreads, 1) k_stream_ws_batch(const StreamParams p, const __grid_constant__ BatchTable tbl)
+{
+    ws_body<MODE, HI, false, true>(p, tbl.cam);
 }
 
 } // namespace cvs

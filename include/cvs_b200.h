@@ -163,8 +163,43 @@ cvs_status cvs_run_sequence_device(cvs_handle h, const uint8_t *d_frames, size_t
                                    const char *text, void *cuda_stream);
 /* after the stream has been synchronised: status word the last sequence launch left behind */
 cvs_status cvs_sequence_status(cvs_handle h);
-/* how many kernels of this library the handle has launched so far (bench.py's gpu_launches) */
+/* how many kernels of this library the handle has launched so far (bench.py's gpu_launches).  A batch's stream-kernel
+ * launch counts once, on hs[0]; its per-camera pre- and post-passes count on their own handles. */
 uint64_t cvs_launch_count(cvs_handle h);
+
+/* ---------------------------------------------------------------------------------------------------------------
+ * Batches: one frame of each of n camera streams (n handles) in ONE stream-kernel launch.  A single frame costs a
+ * fixed launch-and-drain time on top of its pass (DESIGN.md section 9); a server with many cameras on one GPU pays it
+ * once per batch instead of once per camera.
+ *   - hs[0..n): 1 <= n <= CVS_MAX_BATCH distinct handles that share device, width, height, mode and threshold.  Noise
+ *     filter and weights, glyph atlas, overlay text and max_sequence may differ.
+ *   - Every output is bit for bit what n separate calls produce, in any order of the handles: payload, counts,
+ *     display frames, and each handle's reference afterwards.
+ *   - A refused batch (CVS_ERR_INVALID: n out of range, a NULL array or entry, a repeated handle, handles that differ
+ *     in device, size, mode or threshold; CVS_ERR_ALIGN as cvs_run_sequence_device) has enqueued nothing.
+ *   - Frames that do not fit one pass of the stream kernel (3840x2160 on a B200) run handle by handle through the
+ *     single-frame path: same results, n stream-kernel launches (cvs_launch_count shows them).  So does a batch of one,
+ *     which is faster there (the single-frame launch keeps the reference in registers).
+ *   - Noise filter, text overlay and the binarisation's second pass (modes 5, 7) stay per camera, in front of and
+ *     behind the one launch.
+ * --------------------------------------------------------------------------------------------------------------- */
+#define CVS_MAX_BATCH 64
+/* one frame of each of n streams, device-resident (d_frames[i]: 16-byte aligned, N bytes, readable up to N rounded up to
+ * 16), asynchronous on cuda_stream.  Outputs are laid out like a sequence indexed by camera: d_pos[i],
+ * d_xs + i*payload_capacity, d_diff + i*payload_capacity, d_show + i*show_stride (d_show may be NULL).  texts may be
+ * NULL or hold n entries (a NULL entry: no overlay).  Completion: cvs_sequence_status(hs[i]) after the stream has been
+ * synchronised; a capacity overflow of camera i is reported by hs[i] alone. */
+cvs_status cvs_run_batch_device(const cvs_handle *hs, int n, const uint8_t *const *d_frames,
+                                unsigned int *d_pos, int *d_xs, uint8_t *d_diff, size_t payload_capacity,
+                                uint8_t *d_show, size_t show_stride, const char *const *texts, void *cuda_stream);
+/* cvs_submit_io for one frame of each of n streams: tickets[i] belongs to hs[i] and is completed with
+ * cvs_wait(hs[i], tickets[i]); tickets of a handle still complete in submission order, batched or not.  show and texts
+ * may be NULL or hold n entries (NULL entries allowed).  Each frame is uploaded on its own handle's copy stream; the
+ * launch runs on hs[0]'s compute stream behind every handle's earlier tickets, and every handle's later tickets run
+ * behind it.  A handle with 4 outstanding tickets refuses the whole batch (nothing is enqueued for any camera). */
+cvs_status cvs_submit_io_batch(const cvs_handle *hs, int n, const uint8_t *const *frames, uint8_t *const *diff_out,
+                               uint8_t *const *show, const char *const *texts, unsigned int *const *pos,
+                               int *const *xs, uint64_t *tickets);
 
 /* Stand-alone filters on device buffers (config 4 of BASELINE.json and the micro-benchmarks of
  * tests/heat_map_benchmark, tests/heat_map_red_benchmark, tests/grayscale-*, tests/binarization,
