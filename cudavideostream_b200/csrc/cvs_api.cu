@@ -237,42 +237,40 @@ bool mapped_device_pointer(const void *host, void **dev)
 typedef void (*StreamKernel)(const cvs::StreamParams);
 
 template <int MODE>
-StreamKernel pick_hr(bool hi, bool refreg)
+StreamKernel pick_h(bool hi)
 {
-    if (hi) return refreg ? cvs::k_stream<MODE, true, true> : cvs::k_stream<MODE, true, false>;
-    return refreg ? cvs::k_stream<MODE, false, true> : cvs::k_stream<MODE, false, false>;
+    return hi ? cvs::k_stream<MODE, true> : cvs::k_stream<MODE, false>;
 }
-StreamKernel pick_kernel(int mode, bool hi, bool refreg)
+StreamKernel pick_kernel(int mode, bool hi)
 {
     switch (mode) {
-    case 1: return pick_hr<1>(hi, refreg);
-    case 2: return pick_hr<2>(hi, refreg);
-    case 3: return pick_hr<3>(hi, refreg);
-    case 4: return pick_hr<4>(hi, refreg);
-    case 5: return pick_hr<5>(hi, refreg);
-    case 6: return pick_hr<6>(hi, refreg);
-    case 7: return pick_hr<7>(hi, refreg);
-    default: return pick_hr<0>(hi, refreg);
+    case 1: return pick_h<1>(hi);
+    case 2: return pick_h<2>(hi);
+    case 3: return pick_h<3>(hi);
+    case 4: return pick_h<4>(hi);
+    case 5: return pick_h<5>(hi);
+    case 6: return pick_h<6>(hi);
+    case 7: return pick_h<7>(hi);
+    default: return pick_h<0>(hi);
     }
 }
 
 template <int MODE>
-StreamKernel pick_ws_hr(bool hi, bool refreg)
+StreamKernel pick_ws_h(bool hi)
 {
-    if (hi) return refreg ? cvs::k_stream_ws<MODE, true, true> : cvs::k_stream_ws<MODE, true, false>;
-    return refreg ? cvs::k_stream_ws<MODE, false, true> : cvs::k_stream_ws<MODE, false, false>;
+    return hi ? cvs::k_stream_ws<MODE, true> : cvs::k_stream_ws<MODE, false>;
 }
-StreamKernel pick_ws_kernel(int mode, bool hi, bool refreg)
+StreamKernel pick_ws_kernel(int mode, bool hi)
 {
     switch (mode) {
-    case 1: return pick_ws_hr<1>(hi, refreg);
-    case 2: return pick_ws_hr<2>(hi, refreg);
-    case 3: return pick_ws_hr<3>(hi, refreg);
-    case 4: return pick_ws_hr<4>(hi, refreg);
-    case 5: return pick_ws_hr<5>(hi, refreg);
-    case 6: return pick_ws_hr<6>(hi, refreg);
-    case 7: return pick_ws_hr<7>(hi, refreg);
-    default: return pick_ws_hr<0>(hi, refreg);
+    case 1: return pick_ws_h<1>(hi);
+    case 2: return pick_ws_h<2>(hi);
+    case 3: return pick_ws_h<3>(hi);
+    case 4: return pick_ws_h<4>(hi);
+    case 5: return pick_ws_h<5>(hi);
+    case 6: return pick_ws_h<6>(hi);
+    case 7: return pick_ws_h<7>(hi);
+    default: return pick_ws_h<0>(hi);
     }
 }
 
@@ -307,8 +305,6 @@ struct cvs_stream_s {
     size_t Npad = 0, P16 = 0;
     bool hi = false;
     uint32_t addc = 0;
-    uint32_t debug = 0; // CVS_DEBUG_FLAGS (profiling experiments only)
-    int stages = 0;     // CVS_STAGES: ring depth override (0 = default)
     bool trace = false;
     cudaEvent_t ev_base = nullptr;
     uint32_t pred = 0;        // predicted entries of the next frame (previous count + margin)
@@ -347,11 +343,9 @@ struct cvs_stream_s {
     cudaStream_t s_comp = nullptr, s_h2d = nullptr, s_d2h = nullptr, s_pay = nullptr;
     Slot slot[kSlots];
     int last_slot = -1; // slot of the most recently completed ticket (for cvs_get_timing)
-    int occ_cache[8][2][2] = {}; // co-resident blocks per SM of each k_stream variant (0 = not queried yet)
-    int occ_ws[8][2][2] = {};    // same for k_stream_ws
-    int occ_batch[8][2] = {};    // same for k_stream_ws_batch
-    bool use_ws = true;          // CVS_STREAM_KERNEL=v1 selects the one-group kernel (k_stream) for A/B measurements
-    bool force_ws = false;       // CVS_STREAM_KERNEL=ws: k_stream_ws also for multi-pass frames
+    int occ_cache[8][2] = {}; // co-resident blocks per SM of each k_stream variant (0 = not queried yet)
+    int occ_ws[8][2] = {};    // same for k_stream_ws
+    int occ_batch[8][2] = {}; // same for k_stream_ws_batch
     uint64_t next_ticket = 1;
     uint64_t launches = 0;
     float t_h2d = 0, t_kernel = 0, t_d2h = 0;
@@ -562,14 +556,14 @@ cvs_status run_frames(cvs_handle h, const uint8_t *d_frames, size_t stride, int 
     // before it (counts handed from launch to launch).  Same payload, 1.3-1.8x faster than walking the frame in
     // segments with the reference going through L2, which is what single frames (the drop-in call) still do, with
     // the one-group kernel k_stream (k_stream_ws measured 25 against 17 us per 4K frame there).
-    bool ws = h->use_ws;
+    bool ws = true;
     int nbands = 1;
     {
         const int g0 = h->sms < 32 * cvs::kWsLook ? h->sms : 32 * cvs::kWsLook;
-        if (ws && h->nchunks > (size_t)g0 * cvs::kThreads) {
-            if (piece_max >= 4 && !h->force_ws)
+        if (h->nchunks > (size_t)g0 * cvs::kThreads) {
+            if (piece_max >= 4)
                 nbands = (int)((h->nchunks + (size_t)g0 * cvs::kThreads - 1) / ((size_t)g0 * cvs::kThreads));
-            else if (!h->force_ws)
+            else
                 ws = false; // k_stream (segments, reference through L2)
         }
     }
@@ -581,23 +575,22 @@ cvs_status run_frames(cvs_handle h, const uint8_t *d_frames, size_t stride, int 
     if ((uint32_t)G > geo_chunks) G = (int)geo_chunks;
     uint32_t nseg = (uint32_t)((geo_chunks + (size_t)G * cvs::kThreads - 1) / ((size_t)G * cvs::kThreads));
     uint32_t cps = (uint32_t)((geo_chunks + (size_t)G * nseg - 1) / ((size_t)G * nseg));
-    const bool refreg = nseg == 1;
-    if (nbands > 1 && !refreg) return fail(CVS_ERR_INTERNAL, "band geometry does not fit one pass");
-    StreamKernel kern = ws ? pick_ws_kernel(kmode, h->hi, refreg) : pick_kernel(kmode, h->hi, refreg);
+    // k_stream_ws keeps the reference in registers, so it takes a frame (or a band) in one pass; k_stream walks the
+    // frame in segments
+    if ((nseg == 1) != ws)
+        return fail(CVS_ERR_INTERNAL, "%s launch geometry has %u passes per frame", ws ? "k_stream_ws" : "k_stream", nseg);
+    StreamKernel kern = ws ? pick_ws_kernel(kmode, h->hi) : pick_kernel(kmode, h->hi);
     const int block_threads = ws ? cvs::kWsThreads : cvs::kThreads;
-    // ring depth: all four stages when the reference lives in registers (measured +5 % at 1080p), three when it goes
-    // through L2 (a deeper prefetch measured 17 % slower at 3840x2160 with k_stream); fewer if shared memory is short
-    int nstages = refreg ? cvs::kStages : cvs::kStages - 1;
-#ifdef CVS_PROFILING
-    if (h->stages >= 2 && h->stages <= cvs::kStages) nstages = h->stages;
-#endif
+    // ring depth: all four stages for k_stream_ws (measured +5 % at 1080p), three for k_stream (a deeper prefetch
+    // measured 17 % slower at 3840x2160); fewer if shared memory is short
+    int nstages = ws ? cvs::kStages : cvs::kStages - 1;
     int smem_max = 0;
     CU_TRY(cudaDeviceGetAttribute(&smem_max, cudaDevAttrMaxSharedMemoryPerBlockOptin, h->device));
     auto smem_need = [&](int ns) { return ws ? (int)cvs::WsLayout::total(cps, (uint32_t)ns) : cvs::SmemLayout::total(ns); };
     while (nstages > 2 && smem_need(nstages) > smem_max) nstages--;
     const int smem_bytes = smem_need(nstages);
     if (smem_bytes > smem_max) return fail(CVS_ERR_INTERNAL, "stream kernel needs %d bytes of shared memory, device has %d", smem_bytes, smem_max);
-    int &occ = ws ? h->occ_ws[kmode][h->hi ? 1 : 0][refreg ? 1 : 0] : h->occ_cache[kmode][h->hi ? 1 : 0][refreg ? 1 : 0];
+    int &occ = ws ? h->occ_ws[kmode][h->hi ? 1 : 0] : h->occ_cache[kmode][h->hi ? 1 : 0];
     if (occ == 0) { // first launch of this variant on this handle
         CU_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max));
         CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, block_threads, smem_bytes));
@@ -607,7 +600,7 @@ cvs_status run_frames(cvs_handle h, const uint8_t *d_frames, size_t stride, int 
         G = occ * h->sms;
         nseg = (uint32_t)((geo_chunks + (size_t)G * cvs::kThreads - 1) / ((size_t)G * cvs::kThreads));
         cps = (uint32_t)((geo_chunks + (size_t)G * nseg - 1) / ((size_t)G * nseg));
-        if ((nseg == 1) != refreg) return fail(CVS_ERR_INTERNAL, "occupancy changed the segment count");
+        if ((nseg == 1) != ws) return fail(CVS_ERR_INTERNAL, "occupancy changed the segment count");
     }
     if (nbands > 1 && h->band_frames < (size_t)piece_max) {
         if (h->d_band_pos) {
@@ -679,7 +672,6 @@ cvs_status run_frames(cvs_handle h, const uint8_t *d_frames, size_t stride, int 
             p.desc = h->d_desc;
             p.epoch = h->epoch;
             p.addc = h->addc;
-            p.debug = h->debug;
             p.status = d_status;
             void *args[] = {&p};
             // The blocks only ever wait for blocks of LOWER index of the same step (look-back), never at a grid barrier, and
@@ -719,7 +711,7 @@ cvs_status run_batch(const cvs_handle *hs, int n, const uint8_t *const *frames, 
 {
     cvs_handle h0 = hs[0];
     const int G = std::min(std::min(h0->sms, 32 * cvs::kWsLook), (int)h0->nchunks);
-    if (n == 1 || !h0->use_ws || h0->nchunks > (size_t)G * cvs::kThreads) {
+    if (n == 1 || h0->nchunks > (size_t)G * cvs::kThreads) {
         for (int i = 0; i < n; i++) {
             cvs_status s = run_frames(hs[i], frames[i], hs[i]->Npad, 1, pos[i], xs[i], diff[i], cap, show ? show[i] : nullptr,
                                       hs[i]->Npad, texts ? texts[i] : nullptr, st, frames_private, status[i]);
@@ -785,7 +777,6 @@ cvs_status run_batch(const cvs_handle *hs, int n, const uint8_t *const *frames, 
     p.desc = h0->d_desc;
     p.epoch = h0->epoch;
     p.addc = h0->addc;
-    p.debug = h0->debug;
     p.status = status[0];
     void *args[] = {&p, &tbl};
     // plain launch, as for the single frames it replaces: blocks only wait for blocks of lower index (look-back)
@@ -889,17 +880,6 @@ cvs_status cvs_create(const cvs_config *cfg, cvs_handle *out)
     h->Npad = (size_t)h->nchunks * cvs::kChunkBytes;
     h->P16 = round_up(h->npix, 16);
     threshold_consts(cfg->threshold, h->hi, h->addc);
-#ifdef CVS_PROFILING
-    // timing experiments only (results are wrong by construction): compiled into profiling builds, never into the
-    // library a server links -- a stray environment variable must not be able to corrupt a stream
-    if (const char *dbg = getenv("CVS_DEBUG_FLAGS")) h->debug = (uint32_t)atoi(dbg);
-    if (const char *sg = getenv("CVS_STAGES")) h->stages = atoi(sg);
-#endif
-    // both stream kernels are bit-exact; the tests use this to run each kernel on geometries the default does not give it
-    if (const char *kk = getenv("CVS_STREAM_KERNEL")) {
-        h->use_ws = strcmp(kk, "v1") != 0;
-        h->force_ws = strcmp(kk, "ws") == 0;
-    }
     if (const char *tr = getenv("CVS_TRACE")) h->trace = atoi(tr) != 0; // instrumentation only: timelines on stderr
     // own decoder only (refuse, do not fall back to nvJPEG): part of the documented interface
     if (const char *jd = getenv("CVS_JPEG_DECODER")) h->jpeg_own_only = !strcmp(jd, "own");

@@ -83,10 +83,7 @@ __global__ void __launch_bounds__(256) k_conv_rows4(const uint8_t *__restrict__ 
 // 4 + 6*(K/2) bytes becomes a float once (PRMT into the mantissa of 2^23, one FADD) and stays in a K-row register
 // window, so an output costs K*K FFMA -- in the same row-major tap order as k_conv_rows4, hence the same bits.
 // NONNEG: all weights >= 0, so 0 <= acc < 2^23 and truncation is one FADD.RZ against 2^23 instead of F2I.
-#ifndef CVS_CONV_ROWS
-#define CVS_CONV_ROWS 8 // 12 / 16 / 24 rows per strip (fewer halo rows converted) measured the same: 6.67 / 6.66 / 6.73 vs 6.71 us per frame with the diff
-#endif
-constexpr int kConvRows = CVS_CONV_ROWS;
+constexpr int kConvRows = 8; // 12 / 16 / 24 rows per strip (fewer halo rows converted) measured the same: 6.67 / 6.66 / 6.73 vs 6.71 us per frame with the diff
 
 __device__ __forceinline__ float byte_to_float(uint32_t word, int b) // b: compile-time byte index
 {
@@ -457,14 +454,8 @@ __global__ void __launch_bounds__(256) k_filter(const uint8_t *__restrict__ prev
 //   hist: [nframes][256], zeroed by the caller; gray1: [nframes][gray_stride]
 // Lane L adds to histogram copy L mod kGrayHistCopies (copy-interleaved: the copies of a bin sit in different banks).
 // ------------------------------------------------------------------------------------------------
-#ifndef CVS_GRAY_HIST_COPIES
-#define CVS_GRAY_HIST_COPIES 1 // 4 / 8 / 16 copies measured 1-3 % slower (6.89 / 6.90 / 6.81 vs 6.72 us per frame, mode 5): not conflict-bound
-#endif
-constexpr int kGrayHistCopies = CVS_GRAY_HIST_COPIES;
-#ifndef CVS_GRAY_HIST_GROUPS
-#define CVS_GRAY_HIST_GROUPS 4
-#endif
-constexpr int kGrayHistGroupsPerThread = CVS_GRAY_HIST_GROUPS; // groups (16 pixels each) a thread walks: fewer histogram flushes per frame
+constexpr int kGrayHistCopies = 1; // 4 / 8 / 16 copies measured 1-3 % slower (6.89 / 6.90 / 6.81 vs 6.72 us per frame, mode 5): not conflict-bound
+constexpr int kGrayHistGroupsPerThread = 4; // groups (16 pixels each) a thread walks: fewer histogram flushes per frame
 
 template <bool WEIGHTED>
 __global__ void __launch_bounds__(256) k_gray_hist_seq(const uint8_t *__restrict__ frames, size_t frame_stride, uint32_t nbytes,

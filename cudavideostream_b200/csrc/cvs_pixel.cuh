@@ -26,18 +26,7 @@ enum Mode : int {
 // byte j (compile-time after unrolling) of a 12-word group
 __device__ __forceinline__ uint32_t gbyte(const uint32_t (&w)[kGroupWords], int j)
 {
-#ifdef CVS_GBYTE_SHIFT // (the shift-and-mask form: two instructions on the ALU pipe for bytes 1 and 2; A/B timing)
-    return (w[j >> 2] >> (8 * (j & 3))) & 0xffu;
-#else
-    return __byte_perm(w[j >> 2], 0u, 0x4440u + (uint32_t)(j & 3)); // one PRMT
-#endif
-}
-// OR the 24-bit value u (B | G<<8 | R<<16) into pixel p of a zero-initialised group
-__device__ __forceinline__ void put_pixel(uint32_t (&o)[kGroupWords], int p, uint32_t u)
-{
-    const int bit = 24 * p, w = bit >> 5, sh = bit & 31;
-    o[w] |= u << sh;
-    if (sh > 8) o[w + 1] |= u >> (32 - sh);
+    return __byte_perm(w[j >> 2], 0u, 0x4440u + (uint32_t)(j & 3)); // one PRMT (a shift and a mask are two)
 }
 
 // (B + G + R) / 3, integer division                                   server.cpp:96-101
@@ -135,15 +124,6 @@ __device__ __forceinline__ void group_gray3(const uint32_t (&c)[kGroupWords], ui
 __device__ __forceinline__ void group_heat(const uint32_t (&ad)[kGroupWords], const uint32_t *lut,
                                            uint32_t (&o)[kGroupWords])
 {
-#ifdef CVS_HEAT_PUT_PIXEL // (the shift-and-or assembly of the output words, ~12 instructions per 4 pixels; A/B timing)
-#pragma unroll
-    for (int k = 0; k < kGroupWords; k++) o[k] = 0;
-#pragma unroll
-    for (int p = 0; p < kGroupPixels; p++) {
-        uint32_t d = gbyte(ad, 3 * p) + gbyte(ad, 3 * p + 1) + gbyte(ad, 3 * p + 2);
-        put_pixel(o, p, lut[d]);
-    }
-#else
     // four pixels = three words: the 24-bit table entries l0..l3 are laid end to end with three PRMT (measured equal to the
     // shift-and-or form: 3.86 vs 3.87 us per frame -- after the one-PRMT gbyte the heat map no longer waits for this)
 #pragma unroll
@@ -158,7 +138,6 @@ __device__ __forceinline__ void group_heat(const uint32_t (&ad)[kGroupWords], co
         o[3 * i + 1] = __byte_perm(l[1], l[2], 0x5421); // G1 R1 B2 G2
         o[3 * i + 2] = __byte_perm(l[2], l[3], 0x6542); // R2 B3 G3 R3
     }
-#endif
 }
 
 // red map: pixel with any changed channel -> (0,0,255), else `base` (zero or the old reference)

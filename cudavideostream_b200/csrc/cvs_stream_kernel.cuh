@@ -18,17 +18,16 @@
 //     A frame is covered in nseg passes ("segments") of G*cps chunks; in segment s block b owns the cps
 //     consecutive chunks starting at (s*G + b)*cps and thread i of the block owns chunk i of that
 //     slice -- the SAME bytes in every frame.  One (frame, segment) pair is a "step";
-//   * ingest: a block streams its slice of the coming steps into a shared-memory ring (4 stages of 48 KB
-//     when the reference lives in registers, 3 otherwise) with 1-D bulk copies (TMA engine,
-//     cp.async.bulk + mbarrier, L2 evict-first): every byte of a frame crosses HBM -> SM exactly once,
+//   * ingest: a block streams its slice of the coming steps into a shared-memory ring (3 stages of 48 KB)
+//     with 1-D bulk copies (TMA engine, cp.async.bulk + mbarrier, L2 evict-first): every byte of a frame crosses HBM -> SM exactly once,
 //     as one contiguous request per slice (42 KB at 1080p), and each thread picks its 32 whole pixels
 //     out of shared memory with six conflict-free LDS.128 (half the lanes keep their two pixel groups
 //     in swapped order, see voff());
-//   * reference: when a frame fits one segment (1080p on 148 SMs) the thread's 96 reference bytes
-//     live in registers for the whole sequence (REFREG): HBM never sees the reference between the
-//     first frame and the last.  Otherwise each thread reloads / rewrites its own bytes with L2
-//     evict-last accesses (the reference frame stays L2 resident; same thread, same address, so no
-//     cross-thread hazard exists);
+//   * reference: the host runs this kernel only on frames that do not fit one pass of the grid
+//     (3840x2160 single frames and short sequences; k_stream_ws takes everything else), so nseg > 1
+//     and a thread's chunk changes from segment to segment.  In every step each thread reloads its
+//     96 reference bytes with L2 evict-last loads and, if any of them changed, stores them back (the
+//     reference frame stays L2 resident; same thread, same address, so no cross-thread hazard exists);
 //   * one pass over the 24 words of a chunk produces, per word: byte-SIMD |cur-ref| > T flags (the
 //     eight flags of two words are gathered into one byte of the 96-bit change mask by ONE multiply),
 //     the difference bytes cur-ref (parked in the thread's own 96 bytes of the ring stage) and the
@@ -55,10 +54,7 @@
 
 namespace cvs {
 
-#ifndef CVS_STREAM_THREADS
-#define CVS_STREAM_THREADS 512
-#endif
-constexpr int kThreads = CVS_STREAM_THREADS;           // threads per block
+constexpr int kThreads = 512;                         // threads per block
 constexpr int kWarps = kThreads / 32;
 constexpr int kWarpsPad = (kWarps + 3) / 4 * 4;       // stride of the per-warp total arrays
 constexpr int kBlocksPerSM = 512 / kThreads;          // 128 registers per thread fill the register file
@@ -106,7 +102,6 @@ struct StreamParams {
     // display offsets get index_base added -- and frame t's entries follow the pos_prior[t] entries of the bands before
     uint32_t index_base;
     const unsigned int *pos_prior;
-    uint32_t debug;             // profiling experiments only (CVS_DEBUG_FLAGS): 1 no look-back, 2 no emission, 4 no per-word pass
 };
 
 // dynamic shared memory layout (bytes).  The small tables come first and the ring last, so the launch decides
@@ -215,15 +210,10 @@ __device__ __forceinline__ uint8_t *at_u8(uint8_t *base, uint32_t i)
 // instead of shuffles and popcounts.  CHECK = false when the warp's whole run fits the payload capacity.
 // This loop is the bulk of a dense frame's instructions.
 // nchunk: chunks the warp holds (lanes >= nchunk have an empty mask); a multiple of the batch size.
-// STAGE_DIFF: the difference bytes are not stored to global memory one by one but compacted IN PLACE in the warp's part
-// of the ring stage (an entry's rank inside the warp is never larger than its byte position, and the chunks are
-// walked front to back, so a write never lands on a byte that is still to be read); the caller then flushes the
-// g_warp0-based run with whole words (flush_diff_shifted in cvs_stream_ws.cuh).  g_warp0 = global rank of the warp's
-// first entry.
-template <bool CHECK, bool STAGE_DIFF = false>
+template <bool CHECK>
 __device__ __forceinline__ void emit_coop(const uint32_t (&m)[kMaskWords], uint32_t coff0, uint32_t dvaddr0,
                                           int *xs_out, uint8_t *df_out, uint32_t g_lane, uint32_t cap32, uint32_t lane,
-                                          uint32_t scratch, uint32_t nchunk = 32, uint32_t g_warp0 = 0)
+                                          uint32_t scratch, uint32_t nchunk = 32)
 {
     {
         const uint32_t r1 = g_lane + (uint32_t)__popc(m[0]), r2 = r1 + (uint32_t)__popc(m[1]);
@@ -234,10 +224,7 @@ __device__ __forceinline__ void emit_coop(const uint32_t (&m)[kMaskWords], uint3
     __syncwarp();
     const uint32_t lanebit = 1u << lane;
     const uint32_t lt = lanebit - 1u;
-#ifndef CVS_COOP_BATCH
-#define CVS_COOP_BATCH 2
-#endif
-    constexpr int kBatch = CVS_COOP_BATCH; // chunks in flight: their shared loads are issued before any store
+    constexpr int kBatch = 2; // chunks in flight: their shared loads are issued before any store
 #pragma unroll 1
     for (uint32_t S0 = 0; S0 < nchunk; S0 += kBatch) {
         uint32_t sm[kBatch][kMaskWords], rk[kBatch][kMaskWords], v[kBatch][kMaskWords];
@@ -253,7 +240,6 @@ __device__ __forceinline__ void emit_coop(const uint32_t (&m)[kMaskWords], uint3
         for (int i = 0; i < kBatch; i++)
 #pragma unroll
             for (int w = 0; w < kMaskWords; w++) v[i][w] = lds_u8(dvaddr0 + (S0 + i) * kChunkBytes + lane + 32 * w);
-        if (STAGE_DIFF) __syncwarp(); // every lane has read the batch's bytes before anybody overwrites them
 #pragma unroll
         for (int i = 0; i < kBatch; i++) {
             const uint32_t cb = coff0 + (S0 + i) * kChunkBytes + lane;
@@ -263,19 +249,11 @@ __device__ __forceinline__ void emit_coop(const uint32_t (&m)[kMaskWords], uint3
                 // both stores under one predicate (no branch around two instructions)
                 uint32_t on = sm[i][w] & lanebit;
                 if (CHECK && g >= cap32) on = 0;
-                if (STAGE_DIFF) {
-                    asm volatile("{\n\t.reg .pred p;\n\tsetp.ne.u32 p, %0, 0;\n\t"
-                                 "@p st.global.cs.u32 [%1], %2;\n\t"
-                                 "@p st.shared.u8 [%3], %4;\n\t}" ::"r"(on), "l"(at_u32(xs_out, g)), "r"(cb + 32 * w),
-                                 "r"(dvaddr0 + (g - g_warp0)), "r"(v[i][w])
-                                 : "memory");
-                } else {
-                    asm volatile("{\n\t.reg .pred p;\n\tsetp.ne.u32 p, %0, 0;\n\t"
-                                 "@p st.global.cs.u32 [%1], %2;\n\t"
-                                 "@p st.global.cs.u8 [%3], %4;\n\t}" ::"r"(on), "l"(at_u32(xs_out, g)), "r"(cb + 32 * w),
-                                 "l"(at_u8(df_out, g)), "r"(v[i][w])
-                                 : "memory");
-                }
+                asm volatile("{\n\t.reg .pred p;\n\tsetp.ne.u32 p, %0, 0;\n\t"
+                             "@p st.global.cs.u32 [%1], %2;\n\t"
+                             "@p st.global.cs.u8 [%3], %4;\n\t}" ::"r"(on), "l"(at_u32(xs_out, g)), "r"(cb + 32 * w),
+                             "l"(at_u8(df_out, g)), "r"(v[i][w])
+                             : "memory");
             }
         }
     }
@@ -296,7 +274,7 @@ __device__ __forceinline__ uint32_t sum_warps(const uint32_t *p, uint32_t lane)
     return warp_add(lane < (uint32_t)kWarps ? p[lane] : 0u);
 }
 
-template <int MODE, bool HI, bool REFREG>
+template <int MODE, bool HI>
 __global__ void __launch_bounds__(kThreads, kBlocksPerSM) k_stream(const StreamParams p)
 {
     extern __shared__ __align__(128) unsigned char smem[];
@@ -312,8 +290,7 @@ __global__ void __launch_bounds__(kThreads, kBlocksPerSM) k_stream(const StreamP
     const uint32_t b = blockIdx.x, G = gridDim.x;
     const uint32_t N = p.nbytes;
     const uint32_t nsteps = (uint32_t)p.nframes * p.nseg;
-    // ring depth in use (chosen by the host, <= kStages): all four stages when the reference lives in registers
-    // (measured +5 % at 1080p); three when it goes through L2 (a deeper prefetch measured 17 % slower at 3840x2160)
+    // ring depth in use (chosen by the host, < kStages: a deeper prefetch measured 17 % slower at 3840x2160)
     const uint32_t nstages = p.nstages;
     constexpr bool kBinarize = (MODE == kModeBinarize || MODE == kModeBinarizeAvg);
     constexpr bool kGrayW = (MODE == kModeGrayWeighted || MODE == kModeBinarize);
@@ -337,8 +314,7 @@ __global__ void __launch_bounds__(kThreads, kBlocksPerSM) k_stream(const StreamP
     // one thread: refill ring stage st with the slice of step q (st == q mod nstages, tracked by the callers: the
     // ring depth is a launch parameter and a division per step would cost more than the rest of the bookkeeping)
     auto issue = [&](uint32_t q, uint32_t st) {
-        // REFREG <=> one segment per frame
-        const uint32_t t = REFREG ? q : q / p.nseg, s = REFREG ? 0u : q - t * p.nseg;
+        const uint32_t t = q / p.nseg, s = q - t * p.nseg;
         uint32_t off, bytes;
         slice(s, off, bytes);
         if (bytes) {
@@ -375,7 +351,6 @@ __global__ void __launch_bounds__(kThreads, kBlocksPerSM) k_stream(const StreamP
     auto voff = [&](int v) -> uint32_t { return v < 3 ? 16u * v + sw : 16u * v - sw; }; // chunk offset of slot vector v
     uint32_t r[kChunkWords];
     const uint64_t keep = l2_policy_evict_last();
-    bool dirty = false;
     uint32_t coff = 0, nv = 0; // byte offset of this thread's chunk in the frame, valid bytes (0..96)
     uint32_t sbytes = 0;       // bytes of the block's slice in the current segment
     auto geometry = [&](uint32_t s) {
@@ -404,8 +379,8 @@ __global__ void __launch_bounds__(kThreads, kBlocksPerSM) k_stream(const StreamP
             stg_keep(p.ref + coff + voff(v), make_uint4(r[4 * v], r[4 * v + 1], r[4 * v + 2], r[4 * v + 3]), keep);
     };
 
+    // (every step computes its own geometry below; without this first call the compiler schedules the loop differently)
     geometry(0);
-    if (REFREG) load_ref(); // nseg == 1: the geometry never changes and the reference stays in registers
 
     // The loop is software-pipelined by one step: iteration q runs the FRONT half of step q (ingest, flags,
     // change mask, feedback, counts, publish) and then the BACK half of step q-1 (look-back sum, staging,
@@ -425,23 +400,19 @@ __global__ void __launch_bounds__(kThreads, kBlocksPerSM) k_stream(const StreamP
         //      predecessors i, i+256, ...; thread b%256 also reads the running total of the earlier segments
         unsigned long long pv[kLook], pv2 = 0;
         const unsigned long long *prow = p.desc + (size_t)(q ? q - 1 : 0) * (G + 1);
-        const bool look = pending && !(p.debug & 1u);
-        // REFREG <=> one segment per frame: no running total of earlier segments, s stays 0 (compile-time)
-        const bool has2 = !REFREG && look && b_s > 0 && tid == (b % kThreads);
+        const bool has2 = pending && b_s > 0 && tid == (b % kThreads);
 #pragma unroll
         for (int i = 0; i < kLook; i++) {
             pv[i] = 0;
-            if (look && tid + i * kThreads < b) pv[i] = desc_peek(prow + tid + i * kThreads);
+            if (pending && tid + i * kThreads < b) pv[i] = desc_peek(prow + tid + i * kThreads);
         }
         if (has2) pv2 = desc_peek(prow - 1); // slot G of the previous step
 
         uint32_t m[kMaskWords] = {0, 0, 0};
         uint32_t cnt = 0, incl = 0, myaddr = 0;
         if (front) {
-            if (!REFREG) {
-                geometry(s);
-                load_ref(); // L2 hit; issued before the wait on the frame slice
-            }
+            geometry(s);
+            load_ref(); // L2 hit; issued before the wait on the frame slice
             if (kBinarize && s == 0) {
                 // the thread that zeroes bin i is the one that flushed it at the end of the previous frame;
                 // the barrier below orders the zeroing before this frame's atomics
@@ -462,7 +433,6 @@ __global__ void __launch_bounds__(kThreads, kBlocksPerSM) k_stream(const StreamP
             // The pixels are consumed straight from the ring, a few registers at a time: 16 bytes (one vector of
             // look-ahead) without a display filter, one 48-byte pixel group when a filter needs whole pixels.
             constexpr bool kStreamLoad = (MODE == kModeNone);
-            const bool pass_on = !(p.debug & 4u); // debug 4: skip the per-word pass (ingest-only experiment)
             // the chunk that holds the end of the frame: bytes past N never differ (slot word k of the chunk)
             auto clip_word = [&](int k, uint32_t cw) -> uint32_t {
                 const int vb = (int)nv - (int)(voff(k >> 2) + 4 * (k & 3)); // valid bytes from this slot word on
@@ -549,47 +519,40 @@ __global__ void __launch_bounds__(kThreads, kBlocksPerSM) k_stream(const StreamP
                         }
                     }
                     // the filter saw the reference as it was BEFORE this frame; now the pass over the same registers
-                    if (pass_on) {
 #pragma unroll
-                        for (int v = 0; v < kGroupWords / 4; v++) {
-                            const uint32_t cv[4] = {cg[4 * v], cg[4 * v + 1], cg[4 * v + 2], cg[4 * v + 3]};
-                            pass_vector(g * (kGroupWords / 4) + v, cv);
-                        }
+                    for (int v = 0; v < kGroupWords / 4; v++) {
+                        const uint32_t cv[4] = {cg[4 * v], cg[4 * v + 1], cg[4 * v + 2], cg[4 * v + 3]};
+                        pass_vector(g * (kGroupWords / 4) + v, cv);
                     }
                 }
             }
 
-            if (pass_on) {
-                if (kStreamLoad && nv) {
-                    uint4 nx = lds128(myaddr + voff(0));
+            if (kStreamLoad && nv) {
+                uint4 nx = lds128(myaddr + voff(0));
 #pragma unroll
-                    for (int v = 0; v < kChunkWords / 4; v++) {
-                        uint32_t cv[4] = {nx.x, nx.y, nx.z, nx.w};
-                        if (v + 1 < kChunkWords / 4) nx = lds128(myaddr + voff(v + 1));
-                        if (__builtin_expect(nv < (uint32_t)kChunkBytes, 0)) {
+                for (int v = 0; v < kChunkWords / 4; v++) {
+                    uint32_t cv[4] = {nx.x, nx.y, nx.z, nx.w};
+                    if (v + 1 < kChunkWords / 4) nx = lds128(myaddr + voff(v + 1));
+                    if (__builtin_expect(nv < (uint32_t)kChunkBytes, 0)) {
 #pragma unroll
-                            for (int h = 0; h < 4; h++) cv[h] = clip_word(4 * v + h, cv[h]);
-                        }
-                        pass_vector(v, cv);
+                        for (int h = 0; h < 4; h++) cv[h] = clip_word(4 * v + h, cv[h]);
                     }
-                }
-                if (sw) { // slot order -> byte order: rotate the 96-bit mask by 48
-                    const uint32_t n0 = __funnelshift_r(m[1], m[2], 16), n1 = __funnelshift_r(m[2], m[0], 16),
-                                   n2 = __funnelshift_r(m[0], m[1], 16);
-                    m[0] = n0; m[1] = n1; m[2] = n2;
-                }
-                if (__builtin_expect(nv < (uint32_t)kChunkBytes, 0)) { // bytes past the end of the frame are never entries (matters for T < 0)
-#pragma unroll
-                    for (int w = 0; w < kMaskWords; w++) {
-                        const int vb = (int)nv - 32 * w;
-                        m[w] &= vb >= 32 ? 0xffffffffu : (vb <= 0 ? 0u : ((1u << vb) - 1u));
-                    }
-                }
-                if (m[0] | m[1] | m[2]) {
-                    if (REFREG) dirty = true;
-                    else store_ref();
+                    pass_vector(v, cv);
                 }
             }
+            if (sw) { // slot order -> byte order: rotate the 96-bit mask by 48
+                const uint32_t n0 = __funnelshift_r(m[1], m[2], 16), n1 = __funnelshift_r(m[2], m[0], 16),
+                               n2 = __funnelshift_r(m[0], m[1], 16);
+                m[0] = n0; m[1] = n1; m[2] = n2;
+            }
+            if (__builtin_expect(nv < (uint32_t)kChunkBytes, 0)) { // bytes past the end of the frame are never entries (matters for T < 0)
+#pragma unroll
+                for (int w = 0; w < kMaskWords; w++) {
+                    const int vb = (int)nv - 32 * w;
+                    m[w] &= vb >= 32 ? 0xffffffffu : (vb <= 0 ? 0u : ((1u << vb) - 1u));
+                }
+            }
+            if (m[0] | m[1] | m[2]) store_ref();
             cnt = (uint32_t)__popc(m[0]) + (uint32_t)__popc(m[1]) + (uint32_t)__popc(m[2]);
             // only the warp total has to cross the barrier; the per-lane ranks are scanned after it
             const uint32_t wsum = warp_add(cnt);
@@ -614,7 +577,7 @@ __global__ void __launch_bounds__(kThreads, kBlocksPerSM) k_stream(const StreamP
             uint32_t part = 0;
 #pragma unroll
             for (int i = 0; i < kLook; i++)
-                if (look && tid + i * kThreads < b) part += settle(pv[i], prow + tid + i * kThreads);
+                if (tid + i * kThreads < b) part += settle(pv[i], prow + tid + i * kThreads);
             if (has2) part += settle(pv2, prow - 1);
             // G <= kLook * kThreads is enforced by the host, so kLook reads per thread cover every predecessor
             part = warp_add(part);
@@ -635,9 +598,8 @@ __global__ void __launch_bounds__(kThreads, kBlocksPerSM) k_stream(const StreamP
             const uint32_t base = sum_warps(red + (q & 1u) * kWarpsPad, lane);
             if (tid == 0) {
                 if (b == G - 1) {
-                    if (!REFREG)
-                        desc_publish(p.desc + (size_t)(q - 1) * (G + 1) + G, ((unsigned long long)p.epoch << 32) | (base + b_total));
-                    if (REFREG || b_s == p.nseg - 1) p.pos[b_t] = base + b_total;
+                    desc_publish(p.desc + (size_t)(q - 1) * (G + 1) + G, ((unsigned long long)p.epoch << 32) | (base + b_total));
+                    if (b_s == p.nseg - 1) p.pos[b_t] = base + b_total;
                 }
                 if ((size_t)base + b_total > p.cap) atomicOr(p.status, kStatusCapacity);
             }
@@ -651,7 +613,7 @@ __global__ void __launch_bounds__(kThreads, kBlocksPerSM) k_stream(const StreamP
             // and recomputes it there in 64-bit arithmetic (nine instructions per store pair instead of two)
             asm volatile("" : "+l"(xs_out), "+l"(df_out));
             const size_t g0 = (size_t)base + b_wexc; // global rank of this warp's first entry
-            if (b_wtotal && !(p.debug & 2u)) {
+            if (b_wtotal) {
                 if (b_wtotal <= (uint32_t)kWarpEntries) {
                     uint32_t o = b_wrank + (uint32_t)(g0 & 3);
 #pragma unroll
@@ -694,16 +656,13 @@ __global__ void __launch_bounds__(kThreads, kBlocksPerSM) k_stream(const StreamP
             b_wrank = incl - cnt; b_wexc = wexc; b_wtotal = wtotal; b_total = total;
             b_coff = coff; b_myaddr = myaddr; b_t = t; b_s = s;
             pending = true;
-            if (REFREG) ++t;
-            else if (++s == p.nseg) { s = 0; ++t; }
+            if (++s == p.nseg) { s = 0; ++t; }
             b_st = st;
             if (++st == nstages) st = 0;
         } else {
             pending = false;
         }
     }
-
-    if (REFREG && dirty) store_ref();
 }
 
 } // namespace cvs

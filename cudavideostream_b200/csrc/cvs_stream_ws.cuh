@@ -5,10 +5,10 @@
 // server/src/kernels.cu:289-334, and its CPU twin tests/cuda_streaming/test.cu:560-576), but a block is split into
 // two groups of warps that only meet through mbarriers:
 //
-//   FRONT warps (0..15)   own the reference bytes (in registers when a frame fits one pass of the grid) and run
-//                         the per-word pass of step q: pixels out of the TMA ring, flags, 96-bit change mask,
-//                         difference bytes parked in the thread's own 96 bytes of the ring stage, negative feedback,
-//                         display filter.  They leave (mask, count) per chunk and the warp totals in shared memory,
+//   FRONT warps (0..15)   own the reference bytes (in registers for the whole launch: a frame, or a band of a larger
+//                         frame, is one pass of the grid) and run the per-word pass of step q: pixels out of the TMA
+//                         ring, flags, 96-bit change mask, difference bytes parked in the thread's own 96 bytes of
+//                         the ring stage, negative feedback, display filter.  They leave (mask, count) per chunk and the warp totals in shared memory,
 //                         arrive on fdone[stage] and go straight on to step q+1 -- no block barrier, no look-back.
 //   BACK warps (16..31)   back warp w emits the entries of front warp w's 32 chunks: it waits for fdone[stage],
 //                         scans the counts, waits for the block's global offset and stages + flushes (sparse) or
@@ -32,28 +32,18 @@ constexpr int kWsBackWarps = 16;
 constexpr int kWsThreads = 32 * (kWsFrontWarps + kWsBackWarps); // 1024
 constexpr int kWsFrontThreads = 32 * kWsFrontWarps;             // chunks per block per step (= kThreads)
 constexpr int kWsLook = 5;                                      // descriptors a lane of the look-back warp reads: G <= 160
-#ifndef CVS_WS_FRONT_REGS
-#define CVS_WS_FRONT_REGS 80
-#endif
-#ifndef CVS_WS_BACK_REGS
-#define CVS_WS_BACK_REGS 48
-#endif
+// registers per thread after setmaxnreg (88 / 40 and 72 / 56 measured no faster, profiles/README.md)
+constexpr int kWsFrontRegs = 80;
+constexpr int kWsBackRegs = 48;
 // pause between two probes of an mbarrier (ns): front warps waiting for their slice / back warps waiting for the front
 // or for the block's global offset
-#ifndef CVS_WS_SLEEP_FULL
-#define CVS_WS_SLEEP_FULL 100
-#endif
-#ifndef CVS_WS_SLEEP_BACK
-#define CVS_WS_SLEEP_BACK 200
-#endif
+constexpr int kWsSleepFull = 100;
+constexpr int kWsSleepBack = 200;
 // binarisation histogram (modes 5, 7): copies in shared memory, lane L adds to copy L mod kWsHistCopies, which cuts the
 // same-address serialisation of the shared atomics inside a warp (neighbouring pixels have similar gray values)
-#ifndef CVS_WS_HIST_COPIES
-#define CVS_WS_HIST_COPIES 1   // 4 copies measured 2 % SLOWER (7.29 vs 7.16 us per frame, mode 5): the atomics are not conflict-bound
-#endif
-constexpr int kWsHistCopies = CVS_WS_HIST_COPIES;
+constexpr int kWsHistCopies = 1; // 4 copies measured 2 % SLOWER (7.29 vs 7.16 us per frame, mode 5): the atomics are not conflict-bound
 static_assert(kWsFrontThreads == kThreads, "front threads own one chunk each, like k_stream's threads");
-static_assert(512 * CVS_WS_FRONT_REGS + 512 * CVS_WS_BACK_REGS <= 65536, "register file");
+static_assert(512 * kWsFrontRegs + 512 * kWsBackRegs <= 65536, "register file");
 
 // dynamic shared memory of k_stream_ws (bytes).  Stage size and mask stride follow the chunks per block of the
 // launch (cps), so four stages fit next to the mask queue at 1080p / 3840x2160 (cps = 438).
@@ -129,27 +119,6 @@ __device__ __forceinline__ void flush_warp_shifted(const uint16_t *sxs, const ui
     }
 }
 
-// n difference bytes that lie compacted in shared memory at `sv` (16-byte aligned) go to df_out + g0 as whole words:
-// aligned 4-byte stores, the source cut out of two shared words with a funnel shift; the (at most three + three) bytes in
-// front of the first and behind the last whole word one by one.  The caller has checked g0 + n <= capacity.
-__device__ __forceinline__ void flush_diff_shifted(uint32_t sv, uint8_t *df_out, size_t g0, uint32_t n, uint32_t lane)
-{
-    const uint32_t a = (4u - (uint32_t)(g0 & 3)) & 3u; // bytes in front of the first rank that is a multiple of 4
-    const uint32_t head = min(a, n);
-    const uint32_t nq = (n - head) >> 2;
-    uint8_t *dg = df_out + g0;
-    const uint32_t sh8 = 8u * a;
-#pragma unroll 2
-    for (uint32_t k = lane; k < nq; k += 32) {
-        uint32_t d0, d1 = 0;
-        asm volatile("ld.shared.u32 %0, [%1];" : "=r"(d0) : "r"(sv + 4 * k) : "memory");
-        if (a) asm volatile("ld.shared.u32 %0, [%1];" : "=r"(d1) : "r"(sv + 4 * k + 4) : "memory"); // (a == 0: word k alone)
-        stg_stream_u32(dg + head + 4 * k, __funnelshift_r(d0, d1, sh8));
-    }
-    const uint32_t e1 = lane < 4 ? lane : head + 4 * nq + (lane - 4);
-    if (lane < 8 && e1 < (lane < 4 ? head : n)) stg_stream_u8(dg + e1, lds_u8(sv + e1));
-}
-
 // Batches: one frame of each of up to kMaxBatch camera streams in one launch (k_stream_ws_batch).  Step q is camera q
 // (every frame fits one pass, nseg == 1); the pointers of camera q come from this table, which travels in the kernel
 // parameters (kMaxBatch * 72 bytes): no upload, nothing to keep alive after the launch.
@@ -169,21 +138,15 @@ struct BatchTable {
     BatchCam cam[kMaxBatch];
 };
 
-// The body of k_stream_ws and of k_stream_ws_batch.  BATCH: step q is the single pass of camera q, every per-frame
-// pointer comes from cams[q], and the reference goes through L2 step by step (each step is another camera's reference:
-// the !REFREG reload / store, at the camera's address).
-template <int MODE, bool HI, bool REFREG, bool BATCH>
+// The body of k_stream_ws and of k_stream_ws_batch.  Every frame is one pass of the grid (p.nseg == 1, checked by the
+// host), so step q is frame q and every thread owns the same chunk in every step.  The reference stays in the front
+// warps' registers for the whole launch, except in a BATCH: there step q is camera q, every per-frame pointer comes from
+// cams[q], and the reference goes through L2 step by step (reloaded and stored at the camera's address).
+template <int MODE, bool HI, bool BATCH>
 __device__ __forceinline__ void ws_body(const StreamParams &p, const BatchCam *cams)
 {
-    static_assert(!(BATCH && REFREG), "a batch reloads the reference of every step");
     extern __shared__ __align__(128) unsigned char smem[];
-    // role of a warp: the scheduler arbitrates highest-warp-id-first, so which group gets the upper half decides who
-    // wins when both want an issue slot
-#ifdef CVS_WS_FRONT_HIGH
-    const uint32_t tid = threadIdx.x ^ (uint32_t)kWsFrontThreads; // front = hardware warps 16..31
-#else
     const uint32_t tid = threadIdx.x;
-#endif
     const uint32_t lane = tid & 31, warp = tid >> 5;
     const uint32_t b = blockIdx.x, G = gridDim.x;
     const uint32_t N = p.nbytes;
@@ -204,26 +167,21 @@ __device__ __forceinline__ void ws_body(const StreamParams &p, const BatchCam *c
     constexpr bool kBinarize = (MODE == kModeBinarize || MODE == kModeBinarizeAvg);
     constexpr bool kGrayW = (MODE == kModeGrayWeighted || MODE == kModeBinarize);
 
-    // slice of this block in segment s: byte offset and byte count of the bulk copy
-    auto slice = [&](uint32_t s, uint32_t &off, uint32_t &bytes) {
-        uint64_t c0 = ((uint64_t)s * G + b) * p.cps;
-        uint64_t o = c0 * kChunkBytes;
-        if (o >= p.nbytes16) { off = 0; bytes = 0; return; }
-        uint64_t e = o + (uint64_t)p.cps * kChunkBytes;
-        if (e > p.nbytes16) e = p.nbytes16;
-        off = (uint32_t)o;
-        bytes = (uint32_t)(e - o);
-    };
-    // one thread: refill ring stage st with the slice of step q
+    // one thread: refill ring stage st with this block's slice of frame q
     auto issue = [&](uint32_t q, uint32_t st) {
-        const uint32_t t = (REFREG || BATCH) ? q : q / p.nseg, s = (REFREG || BATCH) ? 0u : q - t * p.nseg;
-        uint32_t off, bytes;
-        slice(s, off, bytes);
+        uint32_t off = 0, bytes = 0;
+        const uint64_t o = (uint64_t)b * p.cps * kChunkBytes;
+        if (o < p.nbytes16) {
+            uint64_t e = o + (uint64_t)p.cps * kChunkBytes;
+            if (e > p.nbytes16) e = p.nbytes16;
+            off = (uint32_t)o;
+            bytes = (uint32_t)(e - o);
+        }
         if (bytes) {
             const uint64_t pol = l2_policy_evict_first();
             asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); // parked bytes were written through the generic proxy
             mbar_expect_tx(bar_full + 8 * st, bytes);
-            bulk_g2s(stage_addr + st * stage_bytes, (BATCH ? cams[t].frame : p.frames + (size_t)t * p.frame_stride) + off, bytes,
+            bulk_g2s(stage_addr + st * stage_bytes, (BATCH ? cams[q].frame : p.frames + (size_t)q * p.frame_stride) + off, bytes,
                      bar_full + 8 * st, pol);
         } else {
             // a block whose slice lies past the end of the frame still hands the stage over: the front warps must not
@@ -271,7 +229,7 @@ __device__ __forceinline__ void ws_body(const StreamParams &p, const BatchCam *c
         // =====================================================================================================
         // FRONT: the per-word pass
         // =====================================================================================================
-        asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;" ::"n"(CVS_WS_FRONT_REGS));
+        asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;" ::"n"(kWsFrontRegs));
         uint32_t *slut = reinterpret_cast<uint32_t *>(smem + WsLayout::lut);
         uint32_t *shist = reinterpret_cast<uint32_t *>(smem + WsLayout::hist);
         // bank-conflict-free 16-byte shared accesses: lanes with bit 2 set keep their two 48-byte pixel groups in
@@ -281,15 +239,13 @@ __device__ __forceinline__ void ws_body(const StreamParams &p, const BatchCam *c
         uint32_t r[kChunkWords];
         const uint64_t keep = l2_policy_evict_last();
         bool dirty = false;
-        uint32_t coff = 0, nv = 0, sbytes = 0;
-        auto geometry = [&](uint32_t s) {
-            uint32_t soff;
-            slice(s, soff, sbytes);
-            uint64_t c = ((uint64_t)s * G + b) * p.cps + tid;
-            bool ok = tid < p.cps && c < p.nchunks;
+        uint32_t coff, nv; // this thread's chunk: byte offset in the frame, valid bytes (0..96)
+        {
+            const uint64_t c = (uint64_t)b * p.cps + tid;
+            const bool ok = tid < p.cps && c < p.nchunks;
             coff = ok ? (uint32_t)(c * kChunkBytes) : 0u;
             nv = ok ? min(N - coff, (uint32_t)kChunkBytes) : 0u;
-        };
+        }
         // rb: the reference frame of the step's camera (p.ref unless BATCH)
         auto load_ref = [&](uint8_t *rb) {
             if (nv) {
@@ -308,20 +264,18 @@ __device__ __forceinline__ void ws_body(const StreamParams &p, const BatchCam *c
             for (int v = 0; v < kChunkWords / 4; v++)
                 stg_keep(rb + coff + voff(v), make_uint4(r[4 * v], r[4 * v + 1], r[4 * v + 2], r[4 * v + 3]), keep);
         };
-        geometry(0);
-        if (REFREG) load_ref(p.ref);
+        if (!BATCH) load_ref(p.ref);
 
-        uint32_t phase = 0, st = 0, t = 0, s = 0;
+        uint32_t phase = 0, st = 0;
         for (uint32_t q = 0; q < nsteps; q++) {
-            if (!REFREG) {
-                if (!BATCH) geometry(s);
-                // a batch has one geometry for all its steps; opaque here, so that what derives from it is recomputed per
+            if (BATCH) {
+                // the geometry is the same for all steps; opaque here, so that what derives from it is recomputed per
                 // step instead of being held (spilled) across the loop
-                else asm volatile("" : "+r"(coff), "+r"(nv));
-                load_ref(BATCH ? cams[q].ref : p.ref); // L2 hit (a batch: the camera's reference, from HBM unless
-                                                       // recently used); issued before the wait on the frame slice
+                asm volatile("" : "+r"(coff), "+r"(nv));
+                load_ref(cams[q].ref); // the camera's reference, from HBM unless recently used; issued before the wait
+                                       // on the frame slice
             }
-            wait_bar(bar_full + 8 * st, (phase >> st) & 1u, CVS_WS_SLEEP_FULL); // completes at once for an empty slice (see issue())
+            wait_bar(bar_full + 8 * st, (phase >> st) & 1u, kWsSleepFull); // completes at once for an empty slice (see issue())
             phase ^= 1u << st;
             const uint32_t myaddr = stage_addr + st * stage_bytes + tid * kChunkBytes;
             uint32_t m[kMaskWords] = {0, 0, 0};
@@ -380,31 +334,30 @@ __device__ __forceinline__ void ws_body(const StreamParams &p, const BatchCam *c
 #pragma unroll
                         for (int k = 0; k < kGroupWords; k++) ad[k] = absdiff4(cg[k], rg[k]);
                         group_heat(ad, slut, o);
-                        store_group((BATCH ? cams[q].show : p.show + (size_t)t * p.show_stride) + goff, o, gnv);
+                        store_group((BATCH ? cams[q].show : p.show + (size_t)q * p.show_stride) + goff, o, gnv);
                     } else if (MODE == kModeRedBlack || MODE == kModeRedOverlap) {
                         uint32_t mk[kGroupWords];
 #pragma unroll
                         for (int k = 0; k < kGroupWords; k++) mk[k] = changed80<HI>(absdiff4(cg[k], rg[k]), p.addc);
                         group_red<MODE == kModeRedOverlap>(mk, rg, o);
-                        store_group((BATCH ? cams[q].show : p.show + (size_t)t * p.show_stride) + goff, o, gnv);
+                        store_group((BATCH ? cams[q].show : p.show + (size_t)q * p.show_stride) + goff, o, gnv);
                     } else if (MODE == kModeGrayWeighted || MODE == kModeGrayAverage) {
                         group_gray3<kGrayW>(cg, o);
-                        store_group((BATCH ? cams[q].show : p.show + (size_t)t * p.show_stride) + goff, o, gnv);
+                        store_group((BATCH ? cams[q].show : p.show + (size_t)q * p.show_stride) + goff, o, gnv);
                     } else if (kBinarize) {
                         uint32_t g4[4];
                         group_gray1<kGrayW>(cg, g4);
                         const uint32_t npx = gnv / 3u;
-                        uint8_t *gdst = (BATCH ? cams[q].gray1 : p.gray1 + (size_t)t * p.gray_stride) + goff / 3u;
+                        uint8_t *gdst = (BATCH ? cams[q].gray1 : p.gray1 + (size_t)q * p.gray_stride) + goff / 3u;
                         if (npx == (uint32_t)kGroupPixels) stg_keep(gdst, make_uint4(g4[0], g4[1], g4[2], g4[3]), keep);
 #pragma unroll
                         for (int px = 0; px < kGroupPixels; px++) {
                             if ((uint32_t)px < npx) {
                                 uint32_t gv = byte_of(g4[px >> 2], px & 3);
                                 if (npx != (uint32_t)kGroupPixels) gdst[px] = (uint8_t)gv;
-#ifndef CVS_EXP_NO_HIST // (timing experiment: the atomics are 0.68 of mode 5's 7.87 us per frame; the weighted gray of
-                        //  32 pixels per thread, ~15 instructions each, is what mode 5 costs over mode 0)
+                                // (these atomics measured 0.68 of mode 5's 7.87 us per frame; the weighted gray of 32
+                                //  pixels per thread, ~15 instructions each, is what mode 5 costs over mode 0)
                                 atomicAdd(&shist[gv * kWsHistCopies + (lane & (kWsHistCopies - 1))], 1u); // server.cpp:103-106
-#endif
                             }
                         }
                     }
@@ -415,9 +368,6 @@ __device__ __forceinline__ void ws_body(const StreamParams &p, const BatchCam *c
                     }
                 }
             }
-#ifdef CVS_PROFILING
-            if (p.debug & 4u) nv = 0; // timing experiment: ingest only (results wrong by construction)
-#endif
             if (kStreamLoad && nv == (uint32_t)kChunkBytes) {
                 // the common case as ONE basic block (no per-vector test for the end of the frame), two vectors of look-ahead:
                 // the scheduler can interleave the six independent vector passes, which is what hides the ALU latency with
@@ -457,8 +407,8 @@ __device__ __forceinline__ void ws_body(const StreamParams &p, const BatchCam *c
                 }
             }
             if (m[0] | m[1] | m[2]) {
-                if (REFREG) dirty = true;
-                else store_ref(BATCH ? cams[q].ref : p.ref);
+                if (BATCH) store_ref(cams[q].ref);
+                else dirty = true;
             }
             const uint32_t cnt = (uint32_t)__popc(m[0]) + (uint32_t)__popc(m[1]) + (uint32_t)__popc(m[2]);
             // hand the step to the back warps: (mask, count) per chunk, entries of this warp
@@ -469,11 +419,10 @@ __device__ __forceinline__ void ws_body(const StreamParams &p, const BatchCam *c
             const uint32_t wsum = warp_add(cnt);
             if (lane == 0) {
                 wtot[st * 16 + warp] = wsum;
-#ifndef CVS_WS_SCAN_PUBLISH
                 // the block total of the step goes out to the other blocks as early as possible: the last front warp to
                 // get here publishes it (the back warps' look-back then rarely has to wait for a predecessor).  Publishing
-                // from the look-back warp instead (CVS_WS_SCAN_PUBLISH) makes the pass alone 4 % faster (1.58 vs 1.65 us per
-                // frame) and the whole kernel 4 % slower at 1 % density (2.28 vs 2.19): the look-backs start later.
+                // from the look-back warp instead makes the pass alone 4 % faster (1.58 vs 1.65 us per frame) and the
+                // whole kernel 4 % slower at 1 % density (2.28 vs 2.19): the look-backs start later.
                 atomicAdd(&ftot[st], wsum);
                 __threadfence_block();
                 if (atomicAdd(&fcnt[st], 1u) == (uint32_t)kWsFrontWarps - 1u) {
@@ -482,9 +431,8 @@ __device__ __forceinline__ void ws_body(const StreamParams &p, const BatchCam *c
                     fcnt[st] = 0;
                     desc_publish(p.desc + (size_t)q * (G + 1) + b, ((unsigned long long)p.epoch << 32) | total);
                 }
-#endif
             }
-            if (kBinarize && (BATCH || s == p.nseg - 1)) {
+            if (kBinarize) {
                 // histogram of the frame complete: flush and clear (front warps only: named barrier 1)
                 asm volatile("bar.sync 1, %0;" ::"n"(kWsFrontThreads) : "memory");
                 for (uint32_t i = tid; i < 256; i += kWsFrontThreads) {
@@ -494,22 +442,20 @@ __device__ __forceinline__ void ws_body(const StreamParams &p, const BatchCam *c
                         hv += shist[i * kWsHistCopies + c];
                         shist[i * kWsHistCopies + c] = 0;
                     }
-                    if (hv) atomicAdd((BATCH ? cams[q].hist : p.hist + (size_t)t * 256) + i, hv);
+                    if (hv) atomicAdd((BATCH ? cams[q].hist : p.hist + (size_t)q * 256) + i, hv);
                 }
                 asm volatile("bar.sync 1, %0;" ::"n"(kWsFrontThreads) : "memory");
             }
             __syncwarp();
             if (lane == 0) mbar_arrive(bar_fdone + 8 * st); // release: the warp's shared stores above are visible to the waiters
-            if (REFREG || BATCH) ++t;
-            else if (++s == p.nseg) { s = 0; ++t; }
             if (++st == nstages) st = 0;
         }
-        if (REFREG && dirty) store_ref(p.ref);
+        if (!BATCH && dirty) store_ref(p.ref);
     } else {
         // =====================================================================================================
         // BACK: block scan, cross-block look-back, emission of the (index, value) entries
         // =====================================================================================================
-        asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;" ::"n"(CVS_WS_BACK_REGS));
+        asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;" ::"n"(kWsBackRegs));
         // back warp w emits the chunks front warp w holds.  Measured and rejected (round 2, us per 1080p frame at
         // 1 / 10 / 50 % against 2.18 / 2.97 / 5.72): dealing the block's chunks out evenly to all sixteen back warps (28
         // each instead of 32 for 13.7 warps) 2.31 / 3.25 / 5.67 -- the look-back warp then has entries of its own and
@@ -530,16 +476,18 @@ __device__ __forceinline__ void ws_body(const StreamParams &p, const BatchCam *c
         uint8_t *sd = smem + WsLayout::sd + bw * SmemLayout::kSdBytes;
         const uint32_t cap32 = p.cap > 0xffffffffull ? 0xffffffffu : (uint32_t)p.cap;
 
-        uint32_t ph_f = 0, ph_b = 0, st = 0, t = 0, s = 0;
+        // t: the frame of step q, i.e. q (a counter of its own: derived from q, the frame offsets make the compiler
+        // schedule this loop differently)
+        uint32_t ph_f = 0, ph_b = 0, st = 0, t = 0;
         for (uint32_t q = 0; q < nsteps; q++) {
             if (BATCH) asm volatile("" : "+l"(sxs), "+l"(sd)); // (as the front's geometry: recomputed, not spilled)
             // byte offset of lane 0's chunk in the frame (chunk S of the warp starts 96*S bytes later)
-            const uint32_t wcoff = p.index_base + (uint32_t)((((uint64_t)s * G + b) * p.cps + c0) * kChunkBytes);
+            const uint32_t wcoff = p.index_base + (uint32_t)(((uint64_t)b * p.cps + c0) * kChunkBytes);
             // global-offset slot of the step: 2 x nstages slots, because a sparse warp lets its stage go before it waits
             // for the offset, so the look-back warp may be up to nstages steps ahead of it (not more: the bulk copy of
             // step q + nstages + 1 needs this warp's release of step q + 1)
             const uint32_t bslot = q & (2u * kStages - 1u);
-            wait_bar(bar_fdone + 8 * st, (ph_f >> st) & 1u, CVS_WS_SLEEP_BACK);
+            wait_bar(bar_fdone + 8 * st, (ph_f >> st) & 1u, kWsSleepBack);
             ph_f ^= 1u << st;
             uint32_t m[kMaskWords] = {0, 0, 0}, cnt = 0;
             if (has_chunk)
@@ -553,10 +501,6 @@ __device__ __forceinline__ void ws_body(const StreamParams &p, const BatchCam *c
                 total = warp_add(v);
                 wexc = warp_add(lane < bw ? v : 0u);
             }
-#ifdef CVS_WS_SCAN_PUBLISH
-            if (scan_warp && lane == 0)
-                desc_publish(p.desc + (size_t)q * (G + 1) + b, ((unsigned long long)p.epoch << 32) | total);
-#endif
             const uint32_t incl = warp_incl_scan(cnt, lane);
             const uint32_t wtotal = __shfl_sync(0xffffffffu, incl, 31);
             const uint32_t wrank = incl - cnt;
@@ -576,16 +520,6 @@ __device__ __forceinline__ void ws_body(const StreamParams &p, const BatchCam *c
             // go before it waits for the block's global offset: the look-back latency is then outside the stage's
             // lifetime (bulk copy -> pass -> this copy), which is what bounds the step rate with four stages.
             const bool sparse = wtotal <= (uint32_t)kWarpEntries;
-#ifdef CVS_PROFILING
-            if (p.debug & 2u) { // timing experiment: no emission at all (results wrong by construction)
-                release_stage();
-                ph_b ^= 1u << bslot;
-                if (REFREG || BATCH) ++t;
-                else if (++s == p.nseg) { s = 0; ++t; }
-                if (++st == nstages) st = 0;
-                continue;
-            }
-#endif
             if (sparse) {
                 if (wtotal) {
                     uint32_t o = wrank;
@@ -600,15 +534,13 @@ __device__ __forceinline__ void ws_body(const StreamParams &p, const BatchCam *c
                 // ---- cross-block exchange of the step: sum the predecessors' totals (each lane reads up to kWsLook
                 //      descriptors, all in flight together: one L2 round trip)
                 unsigned long long *row = p.desc + (size_t)q * (G + 1); // (the block's own total was published by the front)
-                unsigned long long pv[kWsLook], pv2 = 0;
-                const bool has2 = !REFREG && s > 0 && lane == 31;
+                unsigned long long pv[kWsLook];
 #pragma unroll
                 for (int i = 0; i < kWsLook; i++) {
                     pv[i] = 0;
                     if (lane + 32 * i < b) pv[i] = desc_peek(row + lane + 32 * i);
                 }
-                if (has2) pv2 = desc_peek(row - 1); // running total of the earlier segments: slot G of the previous step
-                uint32_t prior = 0;                 // entries of the frame that earlier bands (launches) produced
+                uint32_t prior = 0; // entries of the frame that earlier bands (launches) produced
                 if (p.pos_prior && lane == 0) prior = p.pos_prior[t];
                 auto settle = [&](unsigned long long v, const unsigned long long *d) -> uint32_t {
                     uint32_t polls = 0;
@@ -626,21 +558,19 @@ __device__ __forceinline__ void ws_body(const StreamParams &p, const BatchCam *c
 #pragma unroll
                 for (int i = 0; i < kWsLook; i++)
                     if (lane + 32 * i < b) part += settle(pv[i], row + lane + 32 * i);
-                if (has2) part += settle(pv2, row - 1);
                 const uint32_t base = warp_add(part);
                 if (lane == 0) {
                     sbase[bslot] = base;
                     if (b == G - 1) {
-                        if (!REFREG && !BATCH) desc_publish(row + G, ((unsigned long long)p.epoch << 32) | (base + total));
                         if (BATCH) *cams[q].pos = base + total;
-                        else if (REFREG || s == p.nseg - 1) p.pos[t] = base + total;
+                        else p.pos[t] = base + total;
                     }
                     if ((size_t)base + total > p.cap) atomicOr(BATCH ? cams[q].status : p.status, kStatusCapacity);
                     mbar_arrive(bar_base + 8 * bslot);
                 }
             }
             if (wtotal) {
-                wait_bar(bar_base + 8 * bslot, (ph_b >> bslot) & 1u, CVS_WS_SLEEP_BACK);
+                wait_bar(bar_base + 8 * bslot, (ph_b >> bslot) & 1u, kWsSleepBack);
                 const uint32_t base = *reinterpret_cast<volatile uint32_t *>(sbase + bslot);
                 int *xs_out = BATCH ? cams[q].xs : p.xs + (size_t)t * p.cap;
                 uint8_t *df_out = BATCH ? cams[q].diff : p.diff + (size_t)t * p.cap;
@@ -650,26 +580,14 @@ __device__ __forceinline__ void ws_body(const StreamParams &p, const BatchCam *c
                     flush_warp_shifted(sxs, sd, wcoff, xs_out, df_out, g0, wtotal, p.cap, lane);
                     __syncwarp(); // the window is refilled by the next step
                 } else if (g0 + wtotal <= (size_t)cap32) {
-#ifdef CVS_WS_DENSE_STAGED
-                    // Measured and rejected (round 2, bit-exact): indices straight to global memory, difference bytes
-                    // compacted in place in the stage and flushed as whole words instead of one st.global.u8 per entry --
-                    // 6.38 instead of 5.75 us per frame at 50 % (3.21 / 2.96 at 10 % from the larger kernel): the dense
-                    // emission is bound by the instructions it issues, not by its byte stores.
-                    emit_coop<false, true>(m, wcoff, dv0, xs_out, df_out, (uint32_t)g0 + wrank, cap32, lane, smem_u32(sxs), per,
-                                           (uint32_t)g0);
-                    __syncwarp();
-                    flush_diff_shifted(dv0, df_out, g0, wtotal, lane);
-#else
                     emit_coop<false>(m, wcoff, dv0, xs_out, df_out, (uint32_t)g0 + wrank, cap32, lane, smem_u32(sxs), per);
-#endif
                 } else {
                     emit_coop<true>(m, wcoff, dv0, xs_out, df_out, (uint32_t)g0 + wrank, cap32, lane, smem_u32(sxs), per);
                 }
             }
             ph_b ^= 1u << bslot; // every step completes its bar_base slot exactly once, waited for or not
             if (!sparse) release_stage(); // a dense warp stores straight out of the stage
-            if (REFREG || BATCH) ++t;
-            else if (++s == p.nseg) { s = 0; ++t; }
+            ++t;
             if (++st == nstages) st = 0;
         }
     }
@@ -679,17 +597,17 @@ __device__ __forceinline__ void ws_body(const StreamParams &p, const BatchCam *c
         for (uint32_t i = 0; i < nsteps; i++) atomicOr(cams[i].status, kStatusWatchdog);
 }
 
-template <int MODE, bool HI, bool REFREG>
+template <int MODE, bool HI>
 __global__ void __launch_bounds__(kWsThreads, 1) k_stream_ws(const StreamParams p)
 {
-    ws_body<MODE, HI, REFREG, false>(p, nullptr);
+    ws_body<MODE, HI, false>(p, nullptr);
 }
 
 // one frame of each of p.nframes cameras (p.nseg == 1; p.frames, ref, pos, xs, diff, show, gray1, hist unused: see cams)
 template <int MODE, bool HI>
 __global__ void __launch_bounds__(kWsThreads, 1) k_stream_ws_batch(const StreamParams p, const __grid_constant__ BatchTable tbl)
 {
-    ws_body<MODE, HI, false, true>(p, tbl.cam);
+    ws_body<MODE, HI, true>(p, tbl.cam);
 }
 
 } // namespace cvs

@@ -52,5 +52,5 @@ except Exception as e:
     print("status:", e)
 sp = int(pos.to(torch.int64).sum())
 m = min(ms)
-print(f"flags={os.environ.get('CVS_DEBUG_FLAGS','0')} {W}x{H} T={T} d={a.density} mode={a.mode} noiseK={a.noise} c={sp/(T*N):.4f} "
+print(f"{W}x{H} T={T} d={a.density} mode={a.mode} noiseK={a.noise} c={sp/(T*N):.4f} "
       f"best {m:.3f} ms  {m*1000/T:.2f} us/frame  hbm_model {(T*(N+4)+5*sp)/m/1e6:.0f} GB/s  alg {(T*(2*N+4)+6*sp)/m/1e6:.0f} GB/s")

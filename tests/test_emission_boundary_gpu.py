@@ -13,12 +13,13 @@ warp's total without knowing the launch geometry --
 plus 0..15 extra changes in the frame's first chunk, which moves the global offset of every later warp through all
 residues mod 16.  Changed bytes move by threshold + 1 or jump across the range (0 <-> 255), every other byte drifts by at
 most the threshold.  Every path of the library runs the same frames: k_stream_ws with the reference in registers
-(1080p sequences), in bands (3840x2160 sequences) and through L2 (CVS_STREAM_KERNEL=ws, a 3840x2160 single frame),
-and k_stream (3840x2160 single frames, CVS_STREAM_KERNEL=v1 sequences)."""
+(1080p sequences) and in bands (3840x2160 sequences), and k_stream in segments with the reference through L2 (single
+frames larger than one pass: 64 at 2560x1440, every pattern with every extra count, and four at 3840x2160)."""
 import functools
 
 import numpy as np
 import pytest
+from util import launched
 
 pytestmark = pytest.mark.gpu
 
@@ -132,48 +133,47 @@ def _run_sequence(cvs, oracle, w, h, nframes, seed):
 
 
 def _run_single_frames(cvs, oracle, w, h, nframes, seed):
+    """Frame by frame through cvs_exec, which takes frames larger than one pass to k_stream."""
     base, frames, counts = scenario(w, h, nframes, seed)
     s = cvs.Stream(w, h, base)
     oc = oracle.OracleCore(w, h, base)
-    for t in range(nframes):
-        pos, xs, diff, _ = s.exec(frames[t])
-        _check_frame(t, oc, frames[t], counts[t], pos, xs, diff)
+
+    def run():
+        for t in range(nframes):
+            pos, xs, diff, _ = s.exec(frames[t])
+            _check_frame(t, oc, frames[t], counts[t], pos, xs, diff)
+
+    _, names = launched(run)
+    assert names == {"k_stream<0,0>"}, names
     assert np.array_equal(s.reference(), oc.reference())
     s.close()
     oc.close()
 
 
-@pytest.mark.parametrize("kernel", ["default", "v1"])
-def test_1080p_sequence(cvs, oracle, monkeypatch, kernel):
-    # default: k_stream_ws, reference in registers; v1: k_stream.  64 frames: every pattern with every extra count
-    if kernel == "default":
-        monkeypatch.delenv("CVS_STREAM_KERNEL", raising=False)
-    else:
-        monkeypatch.setenv("CVS_STREAM_KERNEL", kernel)
+def test_1080p_sequence(cvs, oracle):
+    # k_stream_ws, reference in registers.  64 frames: every pattern with every extra count
     _run_sequence(cvs, oracle, 1920, 1080, 64, 11)
 
 
-def test_4k_sequence_in_bands(cvs, oracle, monkeypatch):
-    monkeypatch.delenv("CVS_STREAM_KERNEL", raising=False)
+def test_4k_sequence_in_bands(cvs, oracle):
     _run_sequence(cvs, oracle, 3840, 2160, 16, 12)
 
 
-@pytest.mark.parametrize("kernel", ["default", "ws"])
-def test_4k_single_frames(cvs, oracle, monkeypatch, kernel):
-    # default: k_stream in segments; ws: k_stream_ws with the reference through L2 (REFREG = false)
-    if kernel == "default":
-        monkeypatch.delenv("CVS_STREAM_KERNEL", raising=False)
-    else:
-        monkeypatch.setenv("CVS_STREAM_KERNEL", kernel)
+def test_1440p_single_frames(cvs, oracle):
+    # k_stream in two segments (115,200 chunks).  64 frames: every pattern with every extra count
+    _run_single_frames(cvs, oracle, 2560, 1440, 64, 15)
+
+
+def test_4k_single_frames(cvs, oracle):
+    # k_stream in four segments
     _run_single_frames(cvs, oracle, 3840, 2160, 4, 13)
 
 
-def test_capacity_at_the_dense_boundary(cvs, oracle, monkeypatch):
+def test_capacity_at_the_dense_boundary(cvs, oracle):
     """The 513 pattern (every full warp dense) with the last 128 chunks full (96 each).  A capacity equal to the count
     is no overflow; the next smaller capacity (capacities are multiples of 4), or a cut in the middle of the full
     chunks, reports CVS_ERR_CAPACITY and delivers exactly the first `cap` entries without writing past them."""
     import torch
-    monkeypatch.delenv("CVS_STREAM_KERNEL", raising=False)
     w, h, Gd = 1920, 1080, 4096
     n = 3 * w * h
     nchunks = n // CHUNK

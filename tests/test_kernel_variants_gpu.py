@@ -1,14 +1,13 @@
 """Every stream-kernel variant against the CPU oracle, on frames that sit on the edges of the byte compare.
 
-The hot path is one kernel body compiled into 80 functions: k_stream<MODE, HI, REFREG>, k_stream_ws<MODE, HI, REFREG>
-and k_stream_ws_batch<MODE, HI>.  MODE 0..7 is the display filter, HI the form of the carry-free byte compare
-(thresholds of 128 and above), REFREG whether the reference stays in registers (one pass over the frame) or goes
-through L2 (several segments).  The host picks one from the call, the frame size, the number of frames and
-CVS_STREAM_KERNEL.  Each GPU test below takes one route through that choice for every mode at low and high thresholds
-and compares the count, xs, diff, every display byte, the reference afterwards and the guard bytes behind the display
-buffer with OracleCore.  It also records with torch.profiler which kernels it launched and asserts that its route
-reached the whole family it is meant to reach, so a routing change that sends a case to another function fails here
-instead of passing on the wrong one.  The CPU test at the end pins the library's inventory of those functions.
+The hot path is compiled into 48 functions: k_stream<MODE, HI> (frames walked in several segments, the reference
+through L2), k_stream_ws<MODE, HI> (a frame or a band of it in one pass, the reference in registers) and
+k_stream_ws_batch<MODE, HI>.  MODE 0..7 is the display filter, HI the form of the carry-free byte compare (thresholds
+of 128 and above).  The host picks one from the call, the frame size and the number of frames.  Each GPU test below
+takes one route through that choice for every mode at low and high thresholds and compares the count, xs, diff, every
+display byte, the reference afterwards and the guard bytes behind the display buffer with OracleCore.  It also records
+with torch.profiler which kernels it launched and asserts that its route reached the whole family it is meant to
+reach, so a routing change that sends a case to another function fails here instead of passing on the wrong one.  The CPU test at the end pins the library's inventory of those functions.
 
 The frames (checked on the CPU by the tests without a gpu mark):
   pairs         every (reference, current) byte pair in each of the four byte lanes of a 32-bit word, laid out by seeded
@@ -25,10 +24,10 @@ import functools
 import re
 import shutil
 import subprocess
-import time
 
 import numpy as np
 import pytest
+from util import kernel_id, launched
 
 LO = (-1, 0, 20, 127)
 HI = (128, 200, 254, 255)
@@ -263,41 +262,8 @@ def test_binarisation_threshold_needs_the_first_and_last_rows(oracle, mode):
 # ---------------------------------------------------------------------------------------------------------------------
 # which kernels ran
 # ---------------------------------------------------------------------------------------------------------------------
-_KERNEL = re.compile(r"(k_stream_ws_batch|k_stream_ws|k_stream|k_filter)(?:<([^<>]*)>|I((?:L[ib]\d+E)+)E)")
-
-
-def kernel_id(name):
-    """'k_stream_ws<1,1,0>' for 'void cvs::k_stream_ws<1, true, false>(cvs::StreamParams)' or its mangled name, None
-    for any other kernel."""
-    m = _KERNEL.search(name)
-    if not m:
-        return None
-    if m.group(2) is not None:
-        args = [re.sub(r"^\(\w+\)", "", a.strip()) for a in m.group(2).split(",")]
-        vals = [1 if a == "true" else 0 if a == "false" else int(a) for a in args]
-    else:
-        vals = [int(v) for v in re.findall(r"L[ib](\d+)E", m.group(3))]
-    return f"{m.group(1)}<{','.join(map(str, vals))}>"
-
-
-def family(kernel, modes=range(8), refreg=None):
-    tail = "" if refreg is None else f",{refreg}"
-    return {f"{kernel}<{m},{hi}{tail}>" for m in modes for hi in (0, 1)}
-
-
-def launched(fn):
-    """Runs fn() under torch.profiler with CUDA activities (nothing is timed).  Returns fn's result and the set of
-    stream / filter kernels that ran, as kernel_id names.  The session is kept open a little before and after the
-    work, so that even a single kernel of a few microseconds lies well inside it."""
-    import torch
-    from torch.profiler import ProfilerActivity, profile
-    torch.cuda.synchronize()
-    with profile(activities=[ProfilerActivity.CUDA]) as prof:
-        time.sleep(0.02)
-        out = fn()
-        torch.cuda.synchronize()
-        time.sleep(0.02)
-    return out, {k for k in (kernel_id(e.name) for e in prof.events()) if k}
+def family(kernel, modes=range(8)):
+    return {f"{kernel}<{m},{hi}>" for m in modes for hi in (0, 1)}
 
 
 # ---------------------------------------------------------------------------------------------------------------------
@@ -448,35 +414,32 @@ def test_standalone_red_and_heat_maps(cvs, oracle):
 
 
 @pytest.mark.gpu
-def test_dropin_small(cvs, oracle, monkeypatch):
-    """cvs_exec at 514x173: one pass, reference in registers -- k_stream_ws<m, hi, true>."""
-    monkeypatch.delenv("CVS_STREAM_KERNEL", raising=False)
+def test_dropin_small(cvs, oracle):
+    """cvs_exec at 514x173: one pass, reference in registers -- k_stream_ws<m, hi>."""
     errors, seen = [], set()
     w, h = SMALL
     for mode in range(8):
         for thr in THRESHOLDS:
-            _run_case(cvs, oracle, errors, seen, _exec_frames, w, h, thr, mode, 2, f"k_stream_ws<{mode},{_hi(thr)},1>")
-    _report(errors, seen, family("k_stream_ws", refreg=1))
+            _run_case(cvs, oracle, errors, seen, _exec_frames, w, h, thr, mode, 2, f"k_stream_ws<{mode},{_hi(thr)}>")
+    _report(errors, seen, family("k_stream_ws"))
 
 
 @pytest.mark.gpu
-def test_sequence_small(cvs, oracle, monkeypatch):
-    """Three frames in one cvs_run_sequence_device -- k_stream_ws<kmode, hi, true>, kmode 0 for modes 5 / 7."""
-    monkeypatch.delenv("CVS_STREAM_KERNEL", raising=False)
+def test_sequence_small(cvs, oracle):
+    """Three frames in one cvs_run_sequence_device -- k_stream_ws<kmode, hi>, kmode 0 for modes 5 / 7."""
     errors, seen = [], set()
     w, h = SMALL
     for mode in range(8):
         for thr in THRESHOLDS:
             _run_case(cvs, oracle, errors, seen, _sequence, w, h, thr, mode, 3,
-                      f"k_stream_ws<{_seq_kmode(mode)},{_hi(thr)},1>")
-    _report(errors, seen, family("k_stream_ws", modes=(0, 1, 2, 3, 4, 6), refreg=1))
+                      f"k_stream_ws<{_seq_kmode(mode)},{_hi(thr)}>")
+    _report(errors, seen, family("k_stream_ws", modes=(0, 1, 2, 3, 4, 6)))
 
 
 @pytest.mark.gpu
-def test_batch_small(cvs, oracle, monkeypatch):
+def test_batch_small(cvs, oracle):
     """Three cameras per cvs_run_batch_device, two batches in a row -- k_stream_ws_batch<m, hi>."""
     import torch
-    monkeypatch.delenv("CVS_STREAM_KERNEL", raising=False)
     errors, seen = [], set()
     w, h = SMALL
     n = 3 * w * h
@@ -524,72 +487,45 @@ def test_batch_small(cvs, oracle, monkeypatch):
 
 
 @pytest.mark.gpu
-def test_dropin_uhd(cvs, oracle, monkeypatch):
-    """cvs_exec at 3840x2160: several segments, reference through L2 -- k_stream<m, hi, false>.  In modes 5 / 7 the
+def test_dropin_uhd(cvs, oracle):
+    """cvs_exec at 3840x2160: several segments, reference through L2 -- k_stream<m, hi>.  In modes 5 / 7 the
     block histograms gather all segments of the frame."""
-    monkeypatch.delenv("CVS_STREAM_KERNEL", raising=False)
     errors, seen = [], set()
     w, h = UHD
     for mode, thr in _uhd_cases():
-        _run_case(cvs, oracle, errors, seen, _exec_frames, w, h, thr, mode, 2, f"k_stream<{mode},{_hi(thr)},0>",
+        _run_case(cvs, oracle, errors, seen, _exec_frames, w, h, thr, mode, 2, f"k_stream<{mode},{_hi(thr)}>",
                   binarise=mode in (5, 7))
-    _report(errors, seen, family("k_stream", refreg=0))
+    _report(errors, seen, family("k_stream"))
 
 
 @pytest.mark.gpu
-def test_short_sequence_uhd(cvs, oracle, monkeypatch):
-    """Two 3840x2160 frames in one sequence (too few for bands): k_stream<kmode, hi, false>, several frames x several
+def test_short_sequence_uhd(cvs, oracle):
+    """Two 3840x2160 frames in one sequence (too few for bands): k_stream<kmode, hi>, several frames x several
     segments, the look-back carrying totals across both."""
-    monkeypatch.delenv("CVS_STREAM_KERNEL", raising=False)
     errors, seen = [], set()
     w, h = UHD
     for mode, thr in _uhd_cases():
-        _run_case(cvs, oracle, errors, seen, _sequence, w, h, thr, mode, 2, f"k_stream<{_seq_kmode(mode)},{_hi(thr)},0>",
+        _run_case(cvs, oracle, errors, seen, _sequence, w, h, thr, mode, 2, f"k_stream<{_seq_kmode(mode)},{_hi(thr)}>",
                   binarise=mode in (5, 7))
-    _report(errors, seen, family("k_stream", modes=(0, 1, 2, 3, 4, 6), refreg=0))
+    _report(errors, seen, family("k_stream", modes=(0, 1, 2, 3, 4, 6)))
 
 
 @pytest.mark.gpu
-def test_banded_sequence_uhd(cvs, oracle, monkeypatch):
-    """Five 3840x2160 frames: walked band by band, k_stream_ws<m, hi, true> per band."""
-    monkeypatch.delenv("CVS_STREAM_KERNEL", raising=False)
+def test_banded_sequence_uhd(cvs, oracle):
+    """Five 3840x2160 frames: walked band by band, k_stream_ws<m, hi> per band."""
     errors, seen = [], set()
     w, h = UHD
     modes = (1, 2, 3, 4, 6)
     for mode, thr in _uhd_cases(modes):
-        _run_case(cvs, oracle, errors, seen, _sequence, w, h, thr, mode, 5, f"k_stream_ws<{mode},{_hi(thr)},1>")
-    _report(errors, seen, family("k_stream_ws", modes=modes, refreg=1))
-
-
-@pytest.mark.gpu
-def test_v1_small(cvs, oracle, monkeypatch):
-    """CVS_STREAM_KERNEL=v1, cvs_exec at 514x173 -- k_stream<m, hi, true>."""
-    monkeypatch.setenv("CVS_STREAM_KERNEL", "v1")
-    errors, seen = [], set()
-    w, h = SMALL
-    for mode in range(8):
-        for thr in (LO[mode % 4], HI[mode % 4], LO[(mode + 2) % 4], HI[(mode + 2) % 4]):
-            _run_case(cvs, oracle, errors, seen, _exec_frames, w, h, thr, mode, 2, f"k_stream<{mode},{_hi(thr)},1>")
-    _report(errors, seen, family("k_stream", refreg=1))
-
-
-@pytest.mark.gpu
-def test_ws_uhd_single_frames(cvs, oracle, monkeypatch):
-    """CVS_STREAM_KERNEL=ws, cvs_exec at 3840x2160 -- k_stream_ws<m, hi, false>, segments through L2."""
-    monkeypatch.setenv("CVS_STREAM_KERNEL", "ws")
-    errors, seen = [], set()
-    w, h = UHD
-    for mode, thr in _uhd_cases():
-        _run_case(cvs, oracle, errors, seen, _exec_frames, w, h, thr, mode, 2, f"k_stream_ws<{mode},{_hi(thr)},0>",
-                  binarise=mode in (5, 7))
-    _report(errors, seen, family("k_stream_ws", refreg=0))
+        _run_case(cvs, oracle, errors, seen, _sequence, w, h, thr, mode, 5, f"k_stream_ws<{mode},{_hi(thr)}>")
+    _report(errors, seen, family("k_stream_ws", modes=modes))
 
 
 # ---------------------------------------------------------------------------------------------------------------------
 # CPU: the library holds exactly the functions the matrix above runs
 # ---------------------------------------------------------------------------------------------------------------------
 def test_library_inventory_matches_the_matrix():
-    """All 80 stream-kernel functions, and the 7 k_filter ones (ops 2..5 are run by test_standalone_filters).  A new
+    """All 48 stream-kernel functions, and the 7 k_filter ones (ops 2..5 are run by test_standalone_filters).  A new
     template parameter or mode fails here until the GPU tests above reach it."""
     import cudavideostream_b200 as cvs
     try:
@@ -599,8 +535,7 @@ def test_library_inventory_matches_the_matrix():
         pytest.skip(f"cuobjdump unavailable: {e}")
     names = [kernel_id(f) for f in re.findall(r"Function (\S+):", res)]
     stream = sorted(k for k in names if k and k.startswith("k_stream"))
-    assert len(stream) == len(set(stream)) == 80, len(stream)
-    assert set(stream) == (family("k_stream", refreg=0) | family("k_stream", refreg=1) | family("k_stream_ws", refreg=0)
-                           | family("k_stream_ws", refreg=1) | family("k_stream_ws_batch"))
+    assert len(stream) == len(set(stream)) == 48, len(stream)
+    assert set(stream) == family("k_stream") | family("k_stream_ws") | family("k_stream_ws_batch")
     filt = sorted(k for k in names if k and k.startswith("k_filter"))
     assert filt == sorted({"k_filter<0,0>", "k_filter<1,0>", "k_filter<1,1>"} | {f"k_filter<{op},0>" for op in range(2, 6)})

@@ -31,7 +31,7 @@ def test_library_is_sm_100a_only():
 
 
 def test_stream_kernel_uses_tma_bulk_copies_and_byte_simd():
-    k = _function(r"k_streamILi0ELb0ELb1E")          # k_stream<0, false, true>
+    k = _function(r"k_streamILi0ELb0EE")             # k_stream<0, false>
     assert "UBLKCP" in k, "the frame ingest must be a TMA bulk copy (cp.async.bulk)"
     assert "SYNCS" in k, "mbarrier (SYNCS.*) expected next to the bulk copy"
     assert k.count("VABSDIFF4") >= 24, "one byte-SIMD absolute difference per word of the 96-byte chunk"
@@ -41,7 +41,7 @@ def test_stream_kernel_uses_tma_bulk_copies_and_byte_simd():
 
 def test_no_kernel_spills_in_the_hot_variants():
     # local-memory traffic (LDL/STL) in the default-mode stream kernels would mean register spills
-    for name in (r"k_streamILi0ELb0ELb1E", r"k_streamILi0ELb0ELb0E"):
+    for name in (r"k_streamILi0ELb0EE", r"k_stream_wsILi0ELb0EE"):
         k = _function(name)
         assert not re.search(r"\b(LDL|STL)\b", k), f"{name} spills to local memory"
 

@@ -1,4 +1,7 @@
 """Shared helpers for the parity tests."""
+import re
+import time
+
 import numpy as np
 
 CHARS_STR = "0123456789BFPSWbkps :/"  # server/include/common.h:13
@@ -143,3 +146,36 @@ def transcode_huffman(jpg: bytes, coef: np.ndarray, hs: int, vs: int, ncomp: int
     if nacc:
         put((1 << (8 - nacc)) - 1, 8 - nacc)
     return bytes(out) + bytes(data) + b"\xff\xd9"
+
+
+# which stream / filter kernels a piece of work launched
+_KERNEL = re.compile(r"(k_stream_ws_batch|k_stream_ws|k_stream|k_filter)(?:<([^<>]*)>|I((?:L[ib]\d+E)+)E)")
+
+
+def kernel_id(name):
+    """'k_stream_ws<1,0>' for 'void cvs::k_stream_ws<1, false>(cvs::StreamParams)' or its mangled name, None
+    for any other kernel."""
+    m = _KERNEL.search(name)
+    if not m:
+        return None
+    if m.group(2) is not None:
+        args = [re.sub(r"^\(\w+\)", "", a.strip()) for a in m.group(2).split(",")]
+        vals = [1 if a == "true" else 0 if a == "false" else int(a) for a in args]
+    else:
+        vals = [int(v) for v in re.findall(r"L[ib](\d+)E", m.group(3))]
+    return f"{m.group(1)}<{','.join(map(str, vals))}>"
+
+
+def launched(fn):
+    """Runs fn() under torch.profiler with CUDA activities (nothing is timed).  Returns fn's result and the set of
+    stream / filter kernels that ran, as kernel_id names.  The session is kept open a little before and after the
+    work, so that even a single kernel of a few microseconds lies well inside it."""
+    import torch
+    from torch.profiler import ProfilerActivity, profile
+    torch.cuda.synchronize()
+    with profile(activities=[ProfilerActivity.CUDA]) as prof:
+        time.sleep(0.02)
+        out = fn()
+        torch.cuda.synchronize()
+        time.sleep(0.02)
+    return out, {k for k in (kernel_id(e.name) for e in prof.events()) if k}
