@@ -24,7 +24,8 @@
 //       write    one thread per 128 bits decodes once more from its exact state and stores the coefficients
 //   k_unstuff_count / k_unstuff_write / k_entropy_restart   scans WITH restart intervals: the markers are dropped with the
 //               stuffing, every interval starts in a known state and is decoded by one thread, no synchronisation
-//   k_idct      dequantisation + jidctint.c's accurate integer IDCT per 8x8 block -> Y / Cb / Cr planes
+//   k_idct      dequantisation + the accurate integer IDCT (jpeg_idct_islow in libjpeg-turbo's x86-64 SIMD form) per
+//               8x8 block -> Y / Cb / Cr planes
 //   k_colour    jdsample.c's h2v1 / h2v2 "fancy" upsampling (context rows replicated at the border) + jdcolor.c's
 //               fixed-point conversion, stored B, G, R
 //
@@ -901,7 +902,7 @@ __global__ void __launch_bounds__(kEntropyThreads) k_entropy(const EntropyParams
     if (total_blocks_seen && total_blocks_seen < gr.nblocks) atomicOr(p.status, kJpegBlockCount);
 }
 
-// ---- IDCT: jidctint.c jpeg_idct_islow, one thread per 8x8 block ---------------------------------------------------------
+// ---- IDCT: jpeg_idct_islow, one thread per 8x8 block ---------------------------------------------------------------------
 struct PlaneParams {
     Geometry g;
     const Tables *tables;
@@ -909,69 +910,36 @@ struct PlaneParams {
     uint8_t *y, *cb, *cr; // planes: luma pitch = mcux*8*H, chroma pitch = mcux*8
 };
 
-#define CVS_JPG_FIX_0_298631336 2446
-#define CVS_JPG_FIX_0_390180644 3196
-#define CVS_JPG_FIX_0_541196100 4433
-#define CVS_JPG_FIX_0_765366865 6270
-#define CVS_JPG_FIX_0_899976223 7373
-#define CVS_JPG_FIX_1_175875602 9633
-#define CVS_JPG_FIX_1_501321110 12299
-#define CVS_JPG_FIX_1_847759065 15137
-#define CVS_JPG_FIX_1_961570560 16069
-#define CVS_JPG_FIX_2_053119869 16819
-#define CVS_JPG_FIX_2_562915447 20995
-#define CVS_JPG_FIX_3_072711026 25172
+// The arithmetic is libjpeg-turbo's x86-64 SIMD islow IDCT (simd/x86_64/jidctint-avx2.asm), which is what OpenCV runs;
+// it differs from jidctint.c only where values leave 16 bits.  The rules, as in oracle/jpeg_oracle.c idct_islow:
+// dequantisation wraps to int16 (pmullw); in0+in4, in0-in4, in7+in3 and in5+in1 wrap to int16 (paddw / psubw); all
+// other products and sums are 32-bit (pmaddwd / paddd) and cannot overflow; pass 1 saturates to int16 (packssdw); a
+// block whose coefficient rows 1..7 are zero skips pass 1 with row 0 << PASS1_BITS wrapped to int16 (psllw); pass 2
+// saturates to -128..127 and adds 128 (packsswb, paddb).
 
-// the 1-D transform of both passes: eight inputs -> eight outputs descaled by SHIFT (jidctint.c:209-283 / :312-383)
+__device__ __forceinline__ int32_t idct_wrap16(int32_t x) { return (int32_t)(int16_t)x; }
+
+// the 1-D transform of both passes, eight int16 inputs -> eight outputs descaled by SHIFT; the constants are the
+// asm's pmaddwd pairs (sums / differences of jidctint.c's FIX_x values)
 template <int SHIFT>
 __device__ __forceinline__ void idct8(const int32_t (&in)[8], int32_t (&out)[8])
 {
-    int32_t z2 = in[2], z3 = in[6];
-    int32_t z1 = (z2 + z3) * CVS_JPG_FIX_0_541196100;
-    int32_t tmp2 = z1 + z3 * (-CVS_JPG_FIX_1_847759065);
-    int32_t tmp3 = z1 + z2 * CVS_JPG_FIX_0_765366865;
-    int32_t tmp0 = (int32_t)((uint32_t)(in[0] + in[4]) << 13);
-    int32_t tmp1 = (int32_t)((uint32_t)(in[0] - in[4]) << 13);
+    const int32_t tmp3 = in[2] * (4433 + 6270) + in[6] * 4433, tmp2 = in[2] * 4433 + in[6] * (4433 - 15137);
+    const int32_t tmp0 = idct_wrap16(in[0] + in[4]) * (1 << 13), tmp1 = idct_wrap16(in[0] - in[4]) * (1 << 13);
     const int32_t tmp10 = tmp0 + tmp3, tmp13 = tmp0 - tmp3, tmp11 = tmp1 + tmp2, tmp12 = tmp1 - tmp2;
-    tmp0 = in[7];
-    tmp1 = in[5];
-    tmp2 = in[3];
-    tmp3 = in[1];
-    z1 = tmp0 + tmp3;
-    z2 = tmp1 + tmp2;
-    z3 = tmp0 + tmp2;
-    int32_t z4 = tmp1 + tmp3;
-    const int32_t z5 = (z3 + z4) * CVS_JPG_FIX_1_175875602;
-    tmp0 *= CVS_JPG_FIX_0_298631336;
-    tmp1 *= CVS_JPG_FIX_2_053119869;
-    tmp2 *= CVS_JPG_FIX_3_072711026;
-    tmp3 *= CVS_JPG_FIX_1_501321110;
-    z1 *= -CVS_JPG_FIX_0_899976223;
-    z2 *= -CVS_JPG_FIX_2_562915447;
-    z3 *= -CVS_JPG_FIX_1_961570560;
-    z4 *= -CVS_JPG_FIX_0_390180644;
-    z3 += z5;
-    z4 += z5;
-    tmp0 += z1 + z3;
-    tmp1 += z2 + z4;
-    tmp2 += z2 + z3;
-    tmp3 += z1 + z4;
+    const int32_t z3 = idct_wrap16(in[7] + in[3]), z4 = idct_wrap16(in[5] + in[1]);
+    const int32_t Z3 = z3 * (9633 - 16069) + z4 * 9633, Z4 = z3 * 9633 + z4 * (9633 - 3196);
+    const int32_t o0 = in[7] * (2446 - 7373) + in[1] * (-7373) + Z3, o3 = in[7] * (-7373) + in[1] * (12299 - 7373) + Z4;
+    const int32_t o1 = in[5] * (16819 - 20995) + in[3] * (-20995) + Z4, o2 = in[5] * (-20995) + in[3] * (25172 - 20995) + Z3;
     constexpr int32_t rnd = 1 << (SHIFT - 1);
-    out[0] = (tmp10 + tmp3 + rnd) >> SHIFT;
-    out[7] = (tmp10 - tmp3 + rnd) >> SHIFT;
-    out[1] = (tmp11 + tmp2 + rnd) >> SHIFT;
-    out[6] = (tmp11 - tmp2 + rnd) >> SHIFT;
-    out[2] = (tmp12 + tmp1 + rnd) >> SHIFT;
-    out[5] = (tmp12 - tmp1 + rnd) >> SHIFT;
-    out[3] = (tmp13 + tmp0 + rnd) >> SHIFT;
-    out[4] = (tmp13 - tmp0 + rnd) >> SHIFT;
-}
-
-// sample_range_limit + CENTERJSAMPLE indexed with x & 1023 (jdmaster.c prepare_range_limit_table)
-__device__ __forceinline__ uint32_t idct_range_limit(int32_t x)
-{
-    const uint32_t i = (uint32_t)x & 1023u;
-    return i < 128u ? 128u + i : (i < 512u ? 255u : (i < 896u ? 0u : i - 896u));
+    out[0] = (tmp10 + o3 + rnd) >> SHIFT;
+    out[7] = (tmp10 - o3 + rnd) >> SHIFT;
+    out[1] = (tmp11 + o2 + rnd) >> SHIFT;
+    out[6] = (tmp11 - o2 + rnd) >> SHIFT;
+    out[2] = (tmp12 + o1 + rnd) >> SHIFT;
+    out[5] = (tmp12 - o1 + rnd) >> SHIFT;
+    out[3] = (tmp13 + o0 + rnd) >> SHIFT;
+    out[4] = (tmp13 - o0 + rnd) >> SHIFT;
 }
 
 constexpr int kIdctThreads = 128;
@@ -999,30 +967,33 @@ __global__ void __launch_bounds__(kIdctThreads) k_idct(const PlaneParams p)
         pitch = (size_t)g.mcux * 8;
         dst = (c == 1 ? p.cb : p.cr) + (size_t)my * 8 * pitch + (size_t)mx * 8;
     }
-    // coefficients of the block: row r in cf[r][0..7]
+    // dequantised coefficients of the block, wrapped to int16: row r in ws[r][0..7]
     int32_t ws[8][8];
+    uint32_t rows_nz = 0; // OR of the quantised coefficients of rows 1..7
     const uint4 *src = reinterpret_cast<const uint4 *>(p.coef + (size_t)b * 64);
 #pragma unroll
     for (int r = 0; r < 8; r++) {
         const uint4 v = __ldg(src + r);
+        if (r) rows_nz |= v.x | v.y | v.z | v.w;
         const uint32_t wv[4] = {v.x, v.y, v.z, v.w};
 #pragma unroll
         for (int q = 0; q < 8; q++) {
             const int32_t cf = (int32_t)(int16_t)(wv[q >> 1] >> (16 * (q & 1)));
-            ws[r][q] = cf * (int32_t)sq[c][8 * r + q];
+            ws[r][q] = idct_wrap16(cf * (int32_t)sq[c][8 * r + q]);
         }
     }
-    // pass 1: columns
+    // pass 1: columns, saturated to int16; rows 1..7 all zero: row 0 << 2 wrapped to int16 in every row
 #pragma unroll
     for (int col = 0; col < 8; col++) {
         int32_t in[8], out[8];
 #pragma unroll
         for (int r = 0; r < 8; r++) in[r] = ws[r][col];
         idct8<13 - 2>(in, out);
+        const int32_t dc_only = idct_wrap16(in[0] * 4);
 #pragma unroll
-        for (int r = 0; r < 8; r++) ws[r][col] = out[r];
+        for (int r = 0; r < 8; r++) ws[r][col] = rows_nz ? min(max(out[r], -32768), 32767) : dc_only;
     }
-    // pass 2: rows
+    // pass 2: rows, saturated to -128..127, + 128
 #pragma unroll
     for (int r = 0; r < 8; r++) {
         int32_t out[8];
@@ -1030,8 +1001,8 @@ __global__ void __launch_bounds__(kIdctThreads) k_idct(const PlaneParams p)
         uint32_t lo = 0, hi = 0;
 #pragma unroll
         for (int q = 0; q < 4; q++) {
-            lo |= idct_range_limit(out[q]) << (8 * q);
-            hi |= idct_range_limit(out[4 + q]) << (8 * q);
+            lo |= (uint32_t)(min(max(out[q], -128), 127) + 128) << (8 * q);
+            hi |= (uint32_t)(min(max(out[4 + q], -128), 127) + 128) << (8 * q);
         }
         *reinterpret_cast<uint2 *>(dst + (size_t)r * pitch) = make_uint2(lo, hi);
     }

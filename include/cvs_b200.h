@@ -281,7 +281,8 @@ cvs_status cvs_wire_decode_status(const uint32_t *d_scratch, int width, int heig
  * cross PCIe instead of 6.2 MB (1080p), the library's own kernels (csrc/cvs_jpeg.cuh) decode it into the slot's
  * upload buffer and the rest of the path is unchanged.
  *   The decoder reproduces OpenCV's (libjpeg-turbo's default) arithmetic -- sequential-DCT Huffman decoding, the
- *   accurate integer IDCT (jidctint.c), "fancy" chroma upsampling with replicated border rows (jdsample.c /
+ *   accurate integer IDCT in the 16-bit form of its x86-64 SIMD code (jidctint-avx2.asm: wrapping dequantisation,
+ *   saturating passes, whatever the coefficients), "fancy" chroma upsampling with replicated border rows (jdsample.c /
  *   jdmainct.c), fixed-point YCbCr -> RGB (jdcolor.c) -- so the pixels are bit for bit the ones the reference's
  *   capture thread would have produced: on the reference's own f1.jpg / f2.jpg the payload is the reference's, K1 =
  *   369,350 (tests/test_jpeg_ingest.py; oracle: oracle/jpeg_oracle.c, pinned against cv2).

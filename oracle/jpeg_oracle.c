@@ -8,7 +8,11 @@
  * restates the published algorithm of its default decompression path for baseline JPEG:
  *
  *   jdhuff.c   decode_mcu            Huffman decoding of an interleaved scan, DC prediction, restart intervals
- *   jidctint.c jpeg_idct_islow       dequantisation + accurate integer IDCT (JDCT_ISLOW, the default), range limit
+ *   jpeg_idct_islow                  dequantisation + accurate integer IDCT (JDCT_ISLOW, the default) and output range
+ *                                    limit, as x86-64 runs it: the SIMD code simd/x86_64/jidctint-avx2.asm, which is
+ *                                    OpenCV's path (16-bit lanes: wrapping dequantisation, saturating passes), not
+ *                                    jidctint.c, whose int32 arithmetic and x & 1023 range limit differ once
+ *                                    dequantised coefficients leave 16 bits
  *   jdsample.c h2v1/h2v2_fancy_upsample  "fancy" (triangle filter) chroma upsampling (do_fancy_upsampling = TRUE),
  *   jdmainct.c                       with the context rows at the top / bottom of the image replicated
  *   jdcolor.c  ycc_rgb_convert       fixed-point YCbCr -> RGB tables, stored B, G, R (OpenCV's channel order)
@@ -16,7 +20,8 @@
  * PINNED: tests/test_jpeg_oracle.py compares it byte for byte with cv2.imread on the reference's own camera frames
  * (digests in tests/golden/k1_f1_f2.json, made by tests/golden/make_golden.py from the reference's files) and on
  * re-encodings at other qualities / samplings / sizes / restart intervals (tests/golden/jpeg_cases.npz, made by
- * tests/golden/make_jpeg_cases.py with cv2 in the build container).
+ * tests/golden/make_jpeg_cases.py with cv2 in the build container); tests/test_jpeg_coefficient_range.py does the same on
+ * streams designed to reach the edges of the coefficient range.
  *
  * Scope: baseline sequential DCT (SOF0), 8 bit, Huffman, one interleaved scan, 3 components Y Cb Cr with luma sampling
  * 1x1, 2x1 or 2x2 and chroma 1x1 (what UVC cameras and cv2.imwrite produce), or 1 component (gray, replicated to B=G=R).
@@ -322,123 +327,84 @@ static int decode_coefficients(const jpg_t *j, int16_t *coef, size_t nblocks_tot
     return 0;
 }
 
-/* ---- jidctint.c jpeg_idct_islow ------------------------------------------------------------------------------------ */
+/* ---- jpeg_idct_islow as libjpeg-turbo runs it on x86-64: simd/x86_64/jidctint-avx2.asm (jsimd_idct_islow_avx2, the
+ *      path OpenCV's bundled libjpeg-turbo takes on an AVX2 CPU).  jidctint.c's algorithm in 16-bit lanes, which differs
+ *      from the C code only where values leave 16 bits -- large dequantised coefficients:
+ *        - dequantisation is pmullw: coef * q wrapped to int16;
+ *        - the sums in0+in4, in0-in4 (even part) and in7+in3, in5+in1 (odd part's z3, z4) are paddw / psubw: wrapped to
+ *          int16; every other product and sum is a pmaddwd / paddd in 32 bits, where no value of these inputs overflows;
+ *        - pass 1 descales and packs with packssdw: saturated to int16;
+ *        - a block whose coefficient rows 1..7 are all zero skips pass 1: every row of the workspace is the dequantised
+ *          row 0 shifted left by PASS1_BITS with psllw (wrapped to int16, not saturated);
+ *        - pass 2 descales, packs with packssdw and packsswb (saturated to -128..127) and adds CENTERJSAMPLE with paddb.
+ *      tests/test_jpeg_coefficient_range.py states these rules in a Python reference and checks them against cv2. */
 #define CONST_BITS 13
 #define PASS1_BITS 2
-#define FIX_0_298631336 2446
-#define FIX_0_390180644 3196
-#define FIX_0_541196100 4433
-#define FIX_0_765366865 6270
-#define FIX_0_899976223 7373
-#define FIX_1_175875602 9633
-#define FIX_1_501321110 12299
-#define FIX_1_847759065 15137
-#define FIX_1_961570560 16069
-#define FIX_2_053119869 16819
-#define FIX_2_562915447 20995
-#define FIX_3_072711026 25172
 #define DESCALE(x, n) (((x) + ((int32_t)1 << ((n)-1))) >> (n))
+/* the pmaddwd constant pairs of the asm (PW_F130_F054, PW_F054_MF130, PW_MF078_F117, PW_F117_F078, PW_MF060_MF089,
+ * PW_MF089_F060, PW_MF050_MF256, PW_MF256_F050): sums and differences of jidctint.c's FIX_x values */
+#define F_0_541 4433                 /* FIX_0_541196100 */
+#define F_1_306 (4433 + 6270)        /* FIX_0_541196100 + FIX_0_765366865 */
+#define F_M1_306 (4433 - 15137)      /* FIX_0_541196100 - FIX_1_847759065 */
+#define F_1_175 9633                 /* FIX_1_175875602 */
+#define F_M0_785 (9633 - 16069)      /* FIX_1_175875602 - FIX_1_961570560 */
+#define F_0_785 (9633 - 3196)        /* FIX_1_175875602 - FIX_0_390180644 */
+#define F_M0_899 (-7373)             /* -FIX_0_899976223 */
+#define F_M0_601 (2446 - 7373)       /* FIX_0_298631336 - FIX_0_899976223 */
+#define F_0_601 (12299 - 7373)       /* FIX_1_501321110 - FIX_0_899976223 */
+#define F_M2_562 (-20995)            /* -FIX_2_562915447 */
+#define F_M0_509 (16819 - 20995)     /* FIX_2_053119869 - FIX_2_562915447 */
+#define F_0_509 (25172 - 20995)      /* FIX_3_072711026 - FIX_2_562915447 */
 
-static uint8_t range_limit_idct(int32_t x)
+static int32_t wrap16(int32_t x) { return (int32_t)(int16_t)(uint16_t)(uint32_t)x; }
+static int16_t sat16(int32_t x) { return (int16_t)(x < -32768 ? -32768 : (x > 32767 ? 32767 : x)); }
+
+/* one 1-D pass over eight int16 inputs, undescaled: out[0..7] as jidctint.c's tmp10+tmp3 ... tmp10-tmp3 */
+static void idct8_simd(const int16_t *in, int32_t *out)
 {
-    /* sample_range_limit + CENTERJSAMPLE indexed with (x & RANGE_MASK), RANGE_MASK = 1023 (jdmaster.c
-     * prepare_range_limit_table): 0..127 -> 128+i, 128..511 -> 255, 512..895 -> 0, 896..1023 -> i-896 */
-    const int i = (int)(x & 1023);
-    if (i < 128) return (uint8_t)(128 + i);
-    if (i < 512) return 255;
-    if (i < 896) return 0;
-    return (uint8_t)(i - 896);
+    /* even part: tmp3 = z2 * (0.541 + 0.765) + z3 * 0.541, tmp2 = z2 * 0.541 + z3 * (0.541 - 1.848) */
+    const int32_t tmp3 = in[2] * F_1_306 + in[6] * F_0_541, tmp2 = in[2] * F_0_541 + in[6] * F_M1_306;
+    const int32_t tmp0 = wrap16(in[0] + in[4]) * (1 << CONST_BITS), tmp1 = wrap16(in[0] - in[4]) * (1 << CONST_BITS);
+    const int32_t tmp10 = tmp0 + tmp3, tmp13 = tmp0 - tmp3, tmp11 = tmp1 + tmp2, tmp12 = tmp1 - tmp2;
+    /* odd part: z3 = in7 + in3, z4 = in5 + in1 in 16 bits; z5 folded into the pmaddwd constants */
+    const int32_t z3 = wrap16(in[7] + in[3]), z4 = wrap16(in[5] + in[1]);
+    const int32_t Z3 = z3 * F_M0_785 + z4 * F_1_175, Z4 = z3 * F_1_175 + z4 * F_0_785;
+    const int32_t o0 = in[7] * F_M0_601 + in[1] * F_M0_899 + Z3, o3 = in[7] * F_M0_899 + in[1] * F_0_601 + Z4;
+    const int32_t o1 = in[5] * F_M0_509 + in[3] * F_M2_562 + Z4, o2 = in[5] * F_M2_562 + in[3] * F_0_509 + Z3;
+    out[0] = tmp10 + o3;
+    out[7] = tmp10 - o3;
+    out[1] = tmp11 + o2;
+    out[6] = tmp11 - o2;
+    out[2] = tmp12 + o1;
+    out[5] = tmp12 - o1;
+    out[3] = tmp13 + o0;
+    out[4] = tmp13 - o0;
 }
 
 static void idct_islow(const int16_t *in, const uint16_t *qzz, uint8_t *out, size_t pitch)
 {
-    int32_t ws[64];
-    int32_t q[64];
-    for (int k = 0; k < 64; k++) q[zigzag_natural[k]] = qzz[k];
+    int16_t dq[64], ws[64];
+    int rows_zero = 1;
+    for (int k = 0; k < 64; k++) dq[zigzag_natural[k]] = (int16_t)wrap16(in[zigzag_natural[k]] * (int32_t)qzz[k]);
+    for (int k = 8; k < 64; k++) rows_zero &= in[k] == 0; /* tested on the quantised coefficients, before pmullw */
     for (int c = 0; c < 8; c++) {
-        /* (the all-zero-AC shortcut of the original gives the same numbers as the full computation) */
-        int32_t z2 = in[16 + c] * q[16 + c], z3 = in[48 + c] * q[48 + c];
-        int32_t z1 = (z2 + z3) * FIX_0_541196100;
-        int32_t tmp2 = z1 + z3 * (-FIX_1_847759065);
-        int32_t tmp3 = z1 + z2 * FIX_0_765366865;
-        z2 = in[c] * q[c];
-        z3 = in[32 + c] * q[32 + c];
-        int32_t tmp0 = (int32_t)((uint32_t)(z2 + z3) << CONST_BITS);
-        int32_t tmp1 = (int32_t)((uint32_t)(z2 - z3) << CONST_BITS);
-        const int32_t tmp10 = tmp0 + tmp3, tmp13 = tmp0 - tmp3, tmp11 = tmp1 + tmp2, tmp12 = tmp1 - tmp2;
-        tmp0 = in[56 + c] * q[56 + c];
-        tmp1 = in[40 + c] * q[40 + c];
-        tmp2 = in[24 + c] * q[24 + c];
-        tmp3 = in[8 + c] * q[8 + c];
-        z1 = tmp0 + tmp3;
-        z2 = tmp1 + tmp2;
-        z3 = tmp0 + tmp2;
-        int32_t z4 = tmp1 + tmp3;
-        const int32_t z5 = (z3 + z4) * FIX_1_175875602;
-        tmp0 *= FIX_0_298631336;
-        tmp1 *= FIX_2_053119869;
-        tmp2 *= FIX_3_072711026;
-        tmp3 *= FIX_1_501321110;
-        z1 *= -FIX_0_899976223;
-        z2 *= -FIX_2_562915447;
-        z3 *= -FIX_1_961570560;
-        z4 *= -FIX_0_390180644;
-        z3 += z5;
-        z4 += z5;
-        tmp0 += z1 + z3;
-        tmp1 += z2 + z4;
-        tmp2 += z2 + z3;
-        tmp3 += z1 + z4;
-        ws[c] = DESCALE(tmp10 + tmp3, CONST_BITS - PASS1_BITS);
-        ws[56 + c] = DESCALE(tmp10 - tmp3, CONST_BITS - PASS1_BITS);
-        ws[8 + c] = DESCALE(tmp11 + tmp2, CONST_BITS - PASS1_BITS);
-        ws[48 + c] = DESCALE(tmp11 - tmp2, CONST_BITS - PASS1_BITS);
-        ws[16 + c] = DESCALE(tmp12 + tmp1, CONST_BITS - PASS1_BITS);
-        ws[40 + c] = DESCALE(tmp12 - tmp1, CONST_BITS - PASS1_BITS);
-        ws[24 + c] = DESCALE(tmp13 + tmp0, CONST_BITS - PASS1_BITS);
-        ws[32 + c] = DESCALE(tmp13 - tmp0, CONST_BITS - PASS1_BITS);
+        int16_t col[8];
+        int32_t o[8];
+        if (rows_zero) {
+            for (int r = 0; r < 8; r++) ws[8 * r + c] = (int16_t)wrap16(dq[c] * (1 << PASS1_BITS));
+            continue;
+        }
+        for (int r = 0; r < 8; r++) col[r] = dq[8 * r + c];
+        idct8_simd(col, o);
+        for (int r = 0; r < 8; r++) ws[8 * r + c] = sat16(DESCALE(o[r], CONST_BITS - PASS1_BITS));
     }
     for (int r = 0; r < 8; r++) {
-        const int32_t *w = ws + 8 * r;
-        uint8_t *o = out + (size_t)r * pitch;
-        int32_t z2 = w[2], z3 = w[6];
-        int32_t z1 = (z2 + z3) * FIX_0_541196100;
-        int32_t tmp2 = z1 + z3 * (-FIX_1_847759065);
-        int32_t tmp3 = z1 + z2 * FIX_0_765366865;
-        int32_t tmp0 = (int32_t)((uint32_t)(w[0] + w[4]) << CONST_BITS);
-        int32_t tmp1 = (int32_t)((uint32_t)(w[0] - w[4]) << CONST_BITS);
-        const int32_t tmp10 = tmp0 + tmp3, tmp13 = tmp0 - tmp3, tmp11 = tmp1 + tmp2, tmp12 = tmp1 - tmp2;
-        tmp0 = w[7];
-        tmp1 = w[5];
-        tmp2 = w[3];
-        tmp3 = w[1];
-        z1 = tmp0 + tmp3;
-        z2 = tmp1 + tmp2;
-        z3 = tmp0 + tmp2;
-        int32_t z4 = tmp1 + tmp3;
-        const int32_t z5 = (z3 + z4) * FIX_1_175875602;
-        tmp0 *= FIX_0_298631336;
-        tmp1 *= FIX_2_053119869;
-        tmp2 *= FIX_3_072711026;
-        tmp3 *= FIX_1_501321110;
-        z1 *= -FIX_0_899976223;
-        z2 *= -FIX_2_562915447;
-        z3 *= -FIX_1_961570560;
-        z4 *= -FIX_0_390180644;
-        z3 += z5;
-        z4 += z5;
-        tmp0 += z1 + z3;
-        tmp1 += z2 + z4;
-        tmp2 += z2 + z3;
-        tmp3 += z1 + z4;
-        o[0] = range_limit_idct(DESCALE(tmp10 + tmp3, CONST_BITS + PASS1_BITS + 3));
-        o[7] = range_limit_idct(DESCALE(tmp10 - tmp3, CONST_BITS + PASS1_BITS + 3));
-        o[1] = range_limit_idct(DESCALE(tmp11 + tmp2, CONST_BITS + PASS1_BITS + 3));
-        o[6] = range_limit_idct(DESCALE(tmp11 - tmp2, CONST_BITS + PASS1_BITS + 3));
-        o[2] = range_limit_idct(DESCALE(tmp12 + tmp1, CONST_BITS + PASS1_BITS + 3));
-        o[5] = range_limit_idct(DESCALE(tmp12 - tmp1, CONST_BITS + PASS1_BITS + 3));
-        o[3] = range_limit_idct(DESCALE(tmp13 + tmp0, CONST_BITS + PASS1_BITS + 3));
-        o[4] = range_limit_idct(DESCALE(tmp13 - tmp0, CONST_BITS + PASS1_BITS + 3));
+        int32_t o[8];
+        idct8_simd(ws + 8 * r, o);
+        for (int c = 0; c < 8; c++) {
+            const int32_t v = DESCALE(o[c], CONST_BITS + PASS1_BITS + 3);
+            out[(size_t)r * pitch + c] = (uint8_t)((v < -128 ? -128 : (v > 127 ? 127 : v)) + 128);
+        }
     }
 }
 

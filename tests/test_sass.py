@@ -46,6 +46,18 @@ def test_no_kernel_spills_in_the_hot_variants():
         assert not re.search(r"\b(LDL|STL)\b", k), f"{name} spills to local memory"
 
 
+def test_idct_kernel_keeps_its_block_in_registers():
+    # k_idct holds a whole 8x8 block per thread; a spill would put its 64 words in local memory
+    import cudavideostream_b200 as cvs
+    try:
+        res = subprocess.run([CUOBJDUMP, "-res-usage", cvs.library_path()], capture_output=True, text=True, check=True).stdout
+    except (OSError, subprocess.CalledProcessError) as e:
+        pytest.skip(f"cuobjdump unavailable: {e}")
+    m = re.search(r"Function \S*k_idct\S*:\s*\n\s*(.*)", res)
+    assert m, "no k_idct in the library"
+    assert re.search(r"\bSTACK:0\b", m.group(1)) and re.search(r"\bLOCAL:0\b", m.group(1)), m.group(1)
+
+
 def test_noise_filter_is_fma_in_fixed_order():
     # every k_conv_strip<K, NONNEG, WB> launch_conv can pick: WB words (4*WB bytes) per thread
     for K, nonneg, wb in ((3, True, 2), (3, False, 2), (3, True, 1), (3, False, 1), (5, True, 1), (5, False, 1)):

@@ -63,12 +63,15 @@ _ZIGZAG = [0, 1, 8, 16, 9, 2, 3, 10, 17, 24, 32, 25, 18, 11, 4, 5, 12, 19, 26, 3
            35, 42, 49, 56, 57, 50, 43, 36, 29, 22, 15, 23, 30, 37, 44, 51, 58, 59, 52, 45, 38, 31, 39, 46, 53, 60, 61, 54, 47, 55, 62, 63]
 
 
-def transcode_huffman(jpg: bytes, coef: np.ndarray, hs: int, vs: int, ncomp: int, dc_len: int, ac_len: int) -> bytes:
+def transcode_huffman(jpg: bytes, coef: np.ndarray, hs: int, vs: int, ncomp: int, dc_len: int, ac_len: int,
+                      restart_interval: int = 0) -> bytes:
     """Re-encodes the entropy-coded segment of a baseline JPEG (no restart intervals) with Huffman tables in which EVERY
     DC code is dc_len bits and EVERY AC code ac_len bits long (one table pair for all components).  `coef` are the file's
     quantised coefficients [nblocks, 64] in scan order / natural order with absolute DC (oracle.jpeg_coefficients), so the
     result decodes to the same picture.  Long uniform codes give a decoder's look-up tables their worst case: hundreds
-    of distinct long prefixes."""
+    of distinct long prefixes.  With restart_interval > 0 the stream gets a DRI segment and an RSTn marker after every
+    restart_interval MCUs (DC prediction restarts from 0 there).  DC differences must stay within category 11
+    (|difference| <= 2047), AC values within category 10."""
     dc_syms = list(range(12))
     ac_syms = [0x00, 0xF0] + [(r << 4) | s for r in range(16) for s in range(1, 11)]
     assert len(dc_syms) <= (1 << dc_len) - 1 and len(ac_syms) <= (1 << ac_len) - 1
@@ -92,6 +95,8 @@ def transcode_huffman(jpg: bytes, coef: np.ndarray, hs: int, vs: int, ncomp: int
             out += jpg[i:i + 2 + ln]
         i += 2 + ln
     out += dht(0, dc_syms, dc_len) + dht(1, ac_syms, ac_len)
+    if restart_interval:
+        out += b"\xff\xdd\x00\x04" + restart_interval.to_bytes(2, "big")
     sos = bytearray(jpg[i:i + 2 + ln])
     for c in range(ncomp):
         sos[4 + 1 + 2 * c + 1] = 0x00
@@ -119,6 +124,12 @@ def transcode_huffman(jpg: bytes, coef: np.ndarray, hs: int, vs: int, ncomp: int
     pred = [0, 0, 0]
     for b in range(coef.shape[0]):
         j = b % bpm
+        m = b // bpm
+        if restart_interval and j == 0 and m and m % restart_interval == 0:
+            if nacc:
+                put((1 << (8 - nacc)) - 1, 8 - nacc)
+            data += bytes([0xFF, 0xD0 + (m // restart_interval - 1) % 8])
+            pred = [0, 0, 0]
         c = 0 if (ncomp == 1 or j < hs * vs) else j - hs * vs + 1
         blk = coef[b]
         d = int(blk[0]) - pred[c]
