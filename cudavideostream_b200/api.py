@@ -17,6 +17,7 @@ _LIB_PATH = os.environ.get("CVS_B200_LIB") or os.path.join(_HERE, "libcvs_b200.s
 MODE_NONE, MODE_HEAT_MAP, MODE_RED_BLACK, MODE_RED_OVERLAP = 0, 1, 2, 3
 MODE_GRAY_WEIGHTED, MODE_BINARIZE, MODE_GRAY_AVERAGE, MODE_BINARIZE_AVERAGE = 4, 5, 6, 7
 MAX_BATCH = 64  # CVS_MAX_BATCH
+YUV_YUYV, YUV_NV12, YUV_I420 = 1, 2, 3  # cvs_yuv_format
 
 CHARS_STR = "0123456789BFPSWbkps :/"  # server/include/common.h:13
 
@@ -82,6 +83,10 @@ SIGNATURES = {
     "cvs_submit_jpeg": (C.c_int, [_vp, _vp, _sz, _vp, _vp, C.c_char_p, _vp, _vp, C.POINTER(C.c_uint64)]),
     "cvs_submit_jpeg_wire": (C.c_int, [_vp, _vp, _sz, _vp, _vp, C.c_char_p, C.POINTER(C.c_uint64)]),
     "cvs_decode_jpeg_device": (C.c_int, [_vp, _vp, _sz, _vp, _vp]),
+    "cvs_yuv_frame_bytes": (_sz, [C.c_int, C.c_int, C.c_int]),
+    "cvs_submit_yuv": (C.c_int, [_vp, C.c_int, _vp, _vp, _vp, C.c_char_p, _vp, _vp, C.POINTER(C.c_uint64)]),
+    "cvs_submit_yuv_wire": (C.c_int, [_vp, C.c_int, _vp, _vp, _vp, C.c_char_p, C.POINTER(C.c_uint64)]),
+    "cvs_yuv_to_bgr_device": (C.c_int, [C.c_int, C.POINTER(_vp), C.POINTER(_sz), _vp, C.c_int, C.c_int, _vp]),
     "cvs_synth_base_device": (C.c_int, [_vp, C.c_int, C.c_int, C.c_uint64, _vp]),
     "cvs_synth_next_device": (C.c_int, [_vp, _vp, C.c_int, C.c_int, C.c_uint64, C.c_uint32, C.c_uint32, _vp]),
 }
@@ -147,6 +152,11 @@ def alloc_host(nbytes: int) -> HostBuffer:
     return HostBuffer(nbytes)
 
 
+def yuv_frame_bytes(fmt: int, width: int, height: int) -> int:
+    """cvs_yuv_frame_bytes: bytes of one packed YUV frame (0 if the format is unknown or the size odd where it forbids)."""
+    return int(load_library().cvs_yuv_frame_bytes(fmt, width, height))
+
+
 class Stream:
     """One camera stream = one cvs_handle (reference-frame state on one GPU)."""
 
@@ -210,6 +220,20 @@ class Stream:
         """cvs_submit_jpeg_wire: JPEG bitstream in, one compact CVW1 frame out."""
         t = C.c_uint64(0)
         _check(load_library().cvs_submit_jpeg_wire(self._h, jpeg_ptr, jpeg_bytes, wire_ptr, show_ptr, text.encode(), C.byref(t)))
+        return t.value
+
+    def submit_yuv_raw(self, fmt: int, yuv_ptr: int, diff_ptr: int, show_ptr, text: str, pos_ptr: int, xs_ptr: int) -> int:
+        """cvs_submit_yuv: the frame arrives in the camera's packed YUV layout (YUV_YUYV / YUV_NV12 / YUV_I420,
+        yuv_frame_bytes bytes) and is converted to BGR on the GPU (cv2.cvtColor's pixels bit for bit)."""
+        t = C.c_uint64(0)
+        _check(load_library().cvs_submit_yuv(self._h, fmt, yuv_ptr, diff_ptr, show_ptr, text.encode(), pos_ptr, xs_ptr,
+                                             C.byref(t)))
+        return t.value
+
+    def submit_yuv_wire_raw(self, fmt: int, yuv_ptr: int, wire_ptr: int, show_ptr, text: str) -> int:
+        """cvs_submit_yuv_wire: packed YUV frame in, one compact CVW1 frame out."""
+        t = C.c_uint64(0)
+        _check(load_library().cvs_submit_yuv_wire(self._h, fmt, yuv_ptr, wire_ptr, show_ptr, text.encode(), C.byref(t)))
         return t.value
 
     def decode_jpeg_device(self, jpeg: bytes, d_out: int, cuda_stream: int = 0) -> None:

@@ -25,6 +25,7 @@
 #include "cvs_jpeg_host.hpp"
 #include "cvs_stream_kernel.cuh"
 #include "cvs_stream_ws.cuh"
+#include "cvs_yuv.cuh"
 
 namespace {
 
@@ -199,6 +200,7 @@ struct Slot {
     uint32_t *d_starts = nullptr;     // compact wire format: entries before each tile (ntiles + 2 words), on first use
     uint8_t *d_wire = nullptr;        // compact wire format: encoded frame when the caller's buffer is not mapped
     nvjpegJpegState_t jpeg_state = nullptr; // cvs_submit_jpeg: decoder state of this slot (on first use)
+    uint8_t *d_yuv = nullptr;         // cvs_submit_yuv: the camera's packed YUV frame as uploaded (on first use)
     uint8_t *u_wire = nullptr;        // caller's buffer of a cvs_submit_wire ticket (nullptr: reference-format ticket)
     unsigned int *d_status = nullptr; // StatusBits of this ticket's launches (cleared at submit)
     unsigned int *h_status = nullptr; // pinned copy, valid once ev_pos has fired
@@ -979,6 +981,7 @@ cvs_status cvs_destroy(cvs_handle h)
         cudaFreeHost(s.h_status);
         cudaFree(s.d_starts);
         cudaFree(s.d_wire);
+        cudaFree(s.d_yuv);
         if (s.jpeg_state && g_nvjpeg.ok) g_nvjpeg.StateDestroy(s.jpeg_state);
         cudaEvent_t evs[] = {s.ev_h2d0, s.ev_h2d1, s.ev_k0, s.ev_k1, s.ev_pos, s.ev_p0, s.ev_done};
         for (cudaEvent_t e : evs)
@@ -1363,8 +1366,45 @@ static cvs_status egress(cvs_handle h, Slot &s, const uint8_t *frame, uint8_t *d
     return CVS_OK;
 }
 
+// k_yuv_to_bgr<format> on `st`: planes / pitches as cvs_yuv_to_bgr_device takes them, already checked
+static cvs_status yuv_launch(int format, const uint8_t *const *planes, const size_t *pitches, uint8_t *d_out, int width,
+                             int height, cudaStream_t st)
+{
+    cvs::YuvParams p;
+    const int nplanes = format == CVS_YUV_YUYV ? 1 : format == CVS_YUV_NV12 ? 2 : 3;
+    for (int i = 0; i < 3; i++) {
+        p.plane[i] = i < nplanes ? planes[i] : nullptr;
+        p.pitch[i] = i < nplanes ? pitches[i] : 0;
+    }
+    p.bgr = d_out;
+    p.width = width;
+    p.height = height;
+    p.groups = (uint32_t)(width + cvs::kYuvPixels - 1) / cvs::kYuvPixels;
+    const unsigned blocks = (unsigned)(((size_t)p.groups * (size_t)height + cvs::kYuvThreads - 1) / cvs::kYuvThreads);
+    if (format == CVS_YUV_YUYV) cvs::k_yuv_to_bgr<cvs::kYuyv><<<blocks, cvs::kYuvThreads, 0, st>>>(p);
+    else if (format == CVS_YUV_NV12) cvs::k_yuv_to_bgr<cvs::kNv12><<<blocks, cvs::kYuvThreads, 0, st>>>(p);
+    else cvs::k_yuv_to_bgr<cvs::kI420><<<blocks, cvs::kYuvThreads, 0, st>>>(p);
+    CU_TRY(cudaGetLastError());
+    return CVS_OK;
+}
+
+// the planes of a packed frame as cvs_submit_yuv receives it (rows without padding, planes back to back)
+static void yuv_packed_planes(int format, const uint8_t *base, int width, int height, const uint8_t *planes[3], size_t pitches[3])
+{
+    const size_t luma = (size_t)width * (size_t)height;
+    planes[0] = base;
+    pitches[0] = format == CVS_YUV_YUYV ? 2 * (size_t)width : (size_t)width;
+    planes[1] = base + luma;
+    pitches[1] = format == CVS_YUV_NV12 ? (size_t)width : (size_t)width / 2;
+    planes[2] = base + luma + luma / 4;
+    pitches[2] = (size_t)width / 2;
+}
+
+// jpeg_bytes != 0: `frame` is the camera's JPEG bitstream; yuv_format != 0: `frame` is a packed YUV frame of that format
+// (checked by the caller); otherwise the N-byte BGR frame
 static cvs_status submit_common(cvs_handle h, const uint8_t *frame, uint8_t *diff_out, uint8_t *show, const char *text,
-                                unsigned int *pos, int *xs, uint8_t *wire_out, uint64_t *ticket, size_t jpeg_bytes = 0)
+                                unsigned int *pos, int *xs, uint8_t *wire_out, uint64_t *ticket, size_t jpeg_bytes = 0,
+                                int yuv_format = 0)
 {
     cvs_status st = check_handle(h);
     if (st) return st;
@@ -1376,6 +1416,9 @@ static cvs_status submit_common(cvs_handle h, const uint8_t *frame, uint8_t *dif
         CU_TRY(cudaMalloc(&s.d_starts, (size_t)(ntiles + 2) * sizeof(uint32_t)));
         CU_TRY(cudaMalloc(&s.d_wire, cvs_wire_bound(h->width, h->height)));
     }
+    const size_t yuv_bytes = yuv_format ? cvs_yuv_frame_bytes(yuv_format, h->width, h->height) : 0;
+    if (yuv_format && !s.d_yuv) // sized for the largest layout (YUYV, 2WH), so tickets of every format share it
+        CU_TRY(cudaMalloc(&s.d_yuv, round_up(cvs_yuv_frame_bytes(CVS_YUV_YUYV, h->width, h->height), 16)));
 
     const double th0 = h->trace ? host_us() : 0;
     // H2D (kernels.cu:461) -- of the raw frame, or of the camera's JPEG bitstream, decoded on the device.  JPEG tickets
@@ -1393,6 +1436,8 @@ static cvs_status submit_common(cvs_handle h, const uint8_t *frame, uint8_t *dif
         CU_TRY(cudaMemsetAsync(s.d_status, 0, sizeof(unsigned int), s_in));
         st = jpeg_decode(h, jset, &s.jpeg_state, frame, jpeg_bytes, s.d_in, s_in, s.d_status);
         if (st) return st;
+    } else if (yuv_format) { // the camera's packed frame; converted on the compute stream below
+        CU_TRY(cudaMemcpyAsync(s.d_yuv, frame, yuv_bytes, cudaMemcpyHostToDevice, h->s_h2d));
     } else {
         CU_TRY(cudaMemcpyAsync(s.d_in, frame, h->N, cudaMemcpyHostToDevice, h->s_h2d));
     }
@@ -1404,6 +1449,14 @@ static cvs_status submit_common(cvs_handle h, const uint8_t *frame, uint8_t *dif
     uint8_t *dshow = (h->mode && show) ? s.d_show : nullptr;
     const double th1 = h->trace ? host_us() : 0;
     if (!jpeg_bytes) CU_TRY(cudaMemsetAsync(s.d_status, 0, sizeof(unsigned int), h->s_comp));
+    if (yuv_format) { // (inside ev_k0 .. ev_k1: cvs_get_timing counts the conversion as kernel time)
+        const uint8_t *planes[3];
+        size_t pitches[3];
+        yuv_packed_planes(yuv_format, s.d_yuv, h->width, h->height, planes, pitches);
+        st = yuv_launch(yuv_format, planes, pitches, s.d_in, h->width, h->height, h->s_comp);
+        if (st) return st;
+        h->launches++;
+    }
     st = run_frames(h, s.d_in, h->Npad, 1, s.d_pos, s.d_xs, s.d_diff, cap, dshow, h->Npad, text, h->s_comp,
                     /*frames_private=*/true, s.d_status);
     if (st) return st;
@@ -1521,6 +1574,36 @@ cvs_status cvs_decode_jpeg_device(cvs_handle h, const uint8_t *jpeg, size_t jpeg
     if (st) return st;
     CU_TRY(cudaMemcpyAsync(h->h_status, h->d_status, sizeof(unsigned int), cudaMemcpyDeviceToHost, (cudaStream_t)cuda_stream));
     return CVS_OK;
+}
+
+// a YUV submission that cvs_submit_yuv / cvs_submit_yuv_wire refuse before anything is enqueued
+static cvs_status check_yuv_submit(cvs_handle h, int format, const uint8_t *yuv)
+{
+    cvs_status st = check_handle(h);
+    if (st) return st;
+    if (format < CVS_YUV_YUYV || format > CVS_YUV_I420) return fail(CVS_ERR_INVALID, "unknown YUV format %d", format);
+    if (!cvs_yuv_frame_bytes(format, h->width, h->height))
+        return fail(CVS_ERR_INVALID, "a %dx%d stream cannot take YUV format %d (odd %s)", h->width, h->height, format,
+                    format == CVS_YUV_YUYV ? "width" : "width or height");
+    if (!yuv) return fail(CVS_ERR_INVALID, "null argument");
+    return CVS_OK;
+}
+
+cvs_status cvs_submit_yuv(cvs_handle h, int format, const uint8_t *yuv, uint8_t *diff_out, uint8_t *show, const char *text,
+                          unsigned int *pos, int *xs, uint64_t *ticket)
+{
+    cvs_status st = check_yuv_submit(h, format, yuv);
+    if (st) return st;
+    return submit_common(h, yuv, diff_out, show, text, pos, xs, nullptr, ticket, 0, format);
+}
+
+cvs_status cvs_submit_yuv_wire(cvs_handle h, int format, const uint8_t *yuv, uint8_t *wire_out, uint8_t *show,
+                               const char *text, uint64_t *ticket)
+{
+    cvs_status st = check_yuv_submit(h, format, yuv);
+    if (st) return st;
+    if (!wire_out) return fail(CVS_ERR_INVALID, "null argument");
+    return submit_common(h, yuv, nullptr, show, text, nullptr, nullptr, wire_out, ticket, 0, format);
 }
 
 cvs_status cvs_submit_wire(cvs_handle h, const uint8_t *frame, uint8_t *wire_out, uint8_t *show, const char *text,
@@ -1909,6 +1992,40 @@ cvs_status cvs_wire_decode_status(const uint32_t *d_scratch, int width, int heig
     if (flag) return fail(CVS_ERR_INVALID, "encoded frame is inconsistent (magic, tile or geometry, a tile count above its tile's length, counts that do not "
                                        "add up to pos, or offsets out of range or not ascending): nothing was applied");
     return CVS_OK;
+}
+
+size_t cvs_yuv_frame_bytes(int format, int width, int height)
+{
+    if (width <= 0 || height <= 0 || (width & 1)) return 0;
+    const uint64_t luma = (uint64_t)width * (uint64_t)height;
+    if (format == CVS_YUV_YUYV) return (size_t)(2 * luma);
+    if ((format == CVS_YUV_NV12 || format == CVS_YUV_I420) && !(height & 1)) return (size_t)(luma + luma / 2);
+    return 0;
+}
+
+cvs_status cvs_yuv_to_bgr_device(int format, const uint8_t *const *planes, const size_t *pitches, uint8_t *d_out, int width,
+                                 int height, void *cuda_stream)
+{
+    // arguments first: a refusal needs no device
+    if (format < CVS_YUV_YUYV || format > CVS_YUV_I420) return fail(CVS_ERR_INVALID, "unknown YUV format %d", format);
+    if (!cvs_yuv_frame_bytes(format, width, height))
+        return fail(CVS_ERR_INVALID, "%dx%d: not a size YUV format %d takes (positive, width even; 4:2:0 height even)", width,
+                    height, format);
+    if (!planes || !pitches || !d_out) return fail(CVS_ERR_INVALID, "null argument");
+    const int nplanes = format == CVS_YUV_YUYV ? 1 : format == CVS_YUV_NV12 ? 2 : 3;
+    const size_t row_bytes[3] = {format == CVS_YUV_YUYV ? 2 * (size_t)width : (size_t)width,
+                                 format == CVS_YUV_NV12 ? (size_t)width : (size_t)width / 2, (size_t)width / 2};
+    uintptr_t align = (uintptr_t)d_out;
+    for (int i = 0; i < nplanes; i++) {
+        if (!planes[i]) return fail(CVS_ERR_INVALID, "null plane %d", i);
+        if (pitches[i] < row_bytes[i]) return fail(CVS_ERR_INVALID, "pitch of plane %d is %zu, its rows hold %zu bytes", i, pitches[i], row_bytes[i]);
+        align |= (uintptr_t)planes[i] | (uintptr_t)pitches[i];
+    }
+    if (align & 15) return fail(CVS_ERR_ALIGN, "planes, pitches and d_out must be 16-byte aligned");
+    int sms = 0;
+    cvs_status st = filter_common(sms);
+    if (st) return st;
+    return yuv_launch(format, planes, pitches, d_out, width, height, (cudaStream_t)cuda_stream);
 }
 
 cvs_status cvs_synth_base_device(uint8_t *d_out, int width, int height, uint64_t seed, void *cuda_stream)

@@ -3,7 +3,7 @@ from __future__ import annotations
 
 import numpy as np
 
-from .api import _check, _f32p, load_library
+from .api import _check, _f32p, _sz, _vp, load_library
 
 
 def heat_map(d_prev: int, d_cur: int, d_out: int, width: int, height: int, stream: int = 0) -> None:
@@ -35,3 +35,11 @@ def noise_filter(d_frame: int, d_out: int, width: int, height: int, ksize: int, 
 
 def client_apply(d_frame: int, d_xs: int, d_diff: int, d_pos: int, capacity: int, stream: int = 0) -> None:
     _check(load_library().cvs_client_apply_device(d_frame, d_xs, d_diff, d_pos, capacity, stream or None))
+
+
+def yuv_to_bgr(fmt: int, planes, pitches, d_out: int, width: int, height: int, stream: int = 0) -> None:
+    """cvs_yuv_to_bgr_device: a raw YUV frame in device memory -> packed BGR24 (cv2.cvtColor's pixels).  planes: the
+    device addresses of the format's planes (YUYV: 1; NV12: Y, UV; I420: Y, U, V), pitches: their row pitches in bytes."""
+    # three entries whatever the format: missing planes arrive as NULL and are refused, never read past the array
+    _check(load_library().cvs_yuv_to_bgr_device(fmt, (_vp * 3)(*planes), (_sz * 3)(*pitches), d_out, width, height,
+                                                stream or None))

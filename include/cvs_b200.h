@@ -309,6 +309,48 @@ cvs_status cvs_submit_jpeg_wire(cvs_handle h, const uint8_t *jpeg, size_t jpeg_b
 cvs_status cvs_decode_jpeg_device(cvs_handle h, const uint8_t *jpeg, size_t jpeg_bytes, uint8_t *d_out,
                                   void *cuda_stream);
 
+/* ---------------------------------------------------------------------------------------------------------------
+ * Raw YUV cameras: the capture side's colour conversion on the GPU (SURVEY.md section 8f row 4).  UVC webcams in
+ * uncompressed mode deliver YUYV, CSI/ISP cameras and NVDEC deliver NV12, software decoders I420.  cvs_submit_yuv takes
+ * the camera's packed frame instead of the BGR frame a host-side cv2.cvtColor would make of it: 2WH (YUYV) or 3WH/2
+ * (NV12, I420) bytes cross PCIe instead of 3WH (1080p: 4.1 / 3.1 MB instead of 6.2 MB), and no host CPU converts.
+ *   The pixels are cv2.cvtColor's (COLOR_YUV2BGR_YUYV / _NV12 / _I420, BT.601 limited range) bit for bit, integer only:
+ *       y = max(0, Y - 16) * 1220542,  u = U - 128,  v = V - 128
+ *       B = clamp((y + 2^19 + 2116026 u) >> 20),  G = clamp((y + 2^19 - 409993 u - 852492 v) >> 20),
+ *       R = clamp((y + 2^19 + 1673527 v) >> 20)                                               (clamp to 0..255)
+ *   with nearest-neighbour chroma: one (U, V) serves 2x1 pixels (YUYV) or 2x2 pixels (NV12, I420).
+ *   Packed layouts (rows without padding):
+ *     CVS_YUV_YUYV  Y0 U Y1 V per pixel pair, 2W bytes per row;                        width even
+ *     CVS_YUV_NV12  Y plane (W x H), then U V interleaved (W bytes x H/2 rows);          width and height even
+ *     CVS_YUV_I420  Y plane (W x H), then the U plane and the V plane (W/2 x H/2 each);  width and height even
+ *   The frame is uploaded on the handle's copy stream into a buffer of the ticket's slot, converted on the compute
+ *   stream in front of the stream kernel into the slot's frame buffer, and from there everything is what cvs_submit_io /
+ *   cvs_submit_wire do (noise filter, overlay, display modes, egress, tickets, cvs_wait).  cvs_get_timing reports the
+ *   upload of the YUV bytes as h2d and counts the conversion into the kernel time.
+ *   Refused with CVS_ERR_INVALID before anything is enqueued, without consuming a ticket (the reference and the next
+ *   ticket stay as they were): an unknown format, a stream whose width (YUYV) or width or height (NV12, I420) is odd, a
+ *   NULL argument.  The base frame stays BGR (cvs_create, cvs_reset): INTEGRATION.md says how to get it.
+ *   Not covered: UYVY, NV21, YV12, full-range or BT.709 matrices.
+ * --------------------------------------------------------------------------------------------------------------- */
+typedef enum cvs_yuv_format { CVS_YUV_YUYV = 1, CVS_YUV_NV12 = 2, CVS_YUV_I420 = 3 } cvs_yuv_format;
+/* bytes of one packed frame (2WH or 3WH/2); 0 if the format is unknown or the size is not positive, or odd where the
+ * format forbids it */
+size_t cvs_yuv_frame_bytes(int format, int width, int height);
+/* cvs_submit_io with the frame in the camera's packed YUV layout (cvs_yuv_frame_bytes bytes, host; pinned memory from
+ * cvs_alloc_host lets the upload overlap) */
+cvs_status cvs_submit_yuv(cvs_handle h, int format, const uint8_t *yuv, uint8_t *diff_out, uint8_t *show,
+                          const char *text, unsigned int *pos, int *xs, uint64_t *ticket);
+/* cvs_submit_wire with the frame in the camera's packed YUV layout */
+cvs_status cvs_submit_yuv_wire(cvs_handle h, int format, const uint8_t *yuv, uint8_t *wire_out, uint8_t *show,
+                               const char *text, uint64_t *ticket);
+/* the conversion alone, device to device, asynchronous on cuda_stream: planes[0..nplanes) (YUYV: 1 plane, NV12: Y and UV,
+ * I420: Y, U and V; separate allocations allowed) with their row pitches in bytes (NVDEC surfaces, torch tensors) ->
+ * 3 * width * height bytes of packed BGR24 at d_out, nothing written outside them.  Pitches at least the row's bytes
+ * (YUYV 2W; Y and NV12's UV plane W; I420's U and V W/2), else CVS_ERR_INVALID; planes, pitches and d_out 16-byte
+ * aligned, else CVS_ERR_ALIGN. */
+cvs_status cvs_yuv_to_bgr_device(int format, const uint8_t *const *planes, const size_t *pitches, uint8_t *d_out,
+                                 int width, int height, void *cuda_stream);
+
 /* Synthetic camera used by bench.py and the parity tests (SURVEY.md section 8d): counter-based
  * splitmix64 so that the numpy twin in cudavideostream_b200/synth.py produces identical bytes.
  *   cvs_synth_base_device   : base frame (diagonal gradient + noise)
