@@ -11,7 +11,9 @@
 #include <vector>
 #include <cooperative_groups.h>
 
+#include <algorithm>
 #include <atomic>
+#include <cassert>
 #include <cmath>
 #include <cstdarg>
 #include <cstdio>
@@ -20,6 +22,7 @@
 #include <ctime>
 #include <mutex>
 #include <string>
+#include <type_traits>
 
 #include "cvs_filter_kernels.cuh"
 #include "cvs_jpeg_host.hpp"
@@ -47,7 +50,85 @@ cvs_status fail(cvs_status st, const char *fmt, ...)
             return fail(CVS_ERR_CUDA, "%s failed: %s (%s:%d)", #expr, cudaGetErrorString(e_), __FILE__, __LINE__);     \
     } while (0)
 
+#define CVS_TRY(expr)                                                                                                  \
+    do {                                                                                                               \
+        const cvs_status s_ = (expr);                                                                                  \
+        if (s_ != CVS_OK) return s_;                                                                                   \
+    } while (0)
+
 inline size_t round_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
+
+inline uintptr_t addr_bits(const void *p) { return (uintptr_t)p; }
+inline uintptr_t addr_bits(size_t v) { return v; }
+// true when every pointer and stride is a multiple of 16 bytes (the kernels' vector loads and stores)
+template <class... T>
+bool aligned16(T... v)
+{
+    return ((addr_bits(v) & 15) | ...) == 0;
+}
+
+// Device memory owned by the handle (or one of its slots): freed with it.  Grow-only: a buffer that is too small is
+// freed and allocated anew, after a synchronise, because earlier launches may still use it.
+template <class T>
+struct DevBuf {
+    T *p = nullptr;
+    size_t bytes = 0;
+    DevBuf() = default;
+    DevBuf(const DevBuf &) = delete;
+    DevBuf &operator=(const DevBuf &) = delete;
+    ~DevBuf() { cudaFree(p); }
+    operator T *() const { return p; }
+
+    // any stream of the device may use the buffer: the whole device is synchronised; zero: the new buffer is cleared
+    cvs_status grow(size_t need, const char *what, bool zero = false)
+    {
+        if (need <= bytes) return CVS_OK;
+        if (p) CU_TRY(cudaDeviceSynchronize());
+        CVS_TRY(replace(need, what));
+        if (zero) CU_TRY(cudaMemset(p, 0, need));
+        return CVS_OK;
+    }
+    // only stream `user` uses the buffer: it alone is synchronised
+    cvs_status grow_on(cudaStream_t user, size_t need, const char *what)
+    {
+        if (need <= bytes) return CVS_OK;
+        if (p) CU_TRY(cudaStreamSynchronize(user));
+        return replace(need, what);
+    }
+
+  private:
+    cvs_status replace(size_t need, const char *what)
+    {
+        // forget the old buffer before anything can fail: a later call (or the destructor) must not free it again
+        cudaFree(p);
+        p = nullptr;
+        bytes = 0;
+        const cudaError_t e = cudaMalloc(&p, need);
+        if (e != cudaSuccess) {
+            cudaGetLastError();
+            p = nullptr;
+            return fail(CVS_ERR_NOMEM, "%s: %zu bytes of device memory do not fit (%s)", what, need, cudaGetErrorString(e));
+        }
+        bytes = need;
+        return CVS_OK;
+    }
+};
+
+// one word of pinned host memory that a count or status word is copied back into
+struct PinnedWord {
+    unsigned int *p = nullptr;
+    PinnedWord() = default;
+    PinnedWord(const PinnedWord &) = delete;
+    PinnedWord &operator=(const PinnedWord &) = delete;
+    ~PinnedWord() { cudaFreeHost(p); }
+    operator unsigned int *() const { return p; }
+    cvs_status alloc()
+    {
+        CU_TRY(cudaHostAlloc(&p, sizeof *p, cudaHostAllocDefault));
+        *p = 0;
+        return CVS_OK;
+    }
+};
 
 bool device_is_sm100(int dev)
 {
@@ -164,10 +245,10 @@ constexpr int kSlots = 4; // tickets that may be outstanding per stream
 
 // scratch of the GPU JPEG decoder (cvs_jpeg.cuh), one set per handle: decodes of a handle are ordered on one stream
 struct JpegDecoder {
-    uint8_t *d_arena = nullptr;   // everything below points into this one allocation
+    DevBuf<uint8_t> arena;        // every d_* below points into this one allocation (carve)
+    size_t raw_cap = 0, block_cap = 0; // entropy-coded bytes and blocks the arena is carved for
     size_t zero_bytes_fixed = 0;  // bytes in front of the coefficients that every decode clears
     uint8_t *d_raw = nullptr, *d_unst = nullptr; // entropy-coded segment as received / unstuffed (zero-padded)
-    size_t raw_cap = 0;
     uint32_t *d_block_kept = nullptr, *d_block_marks = nullptr, *d_total_bits = nullptr, *d_total_marks = nullptr, *d_seg_start = nullptr;
     uint32_t seg_cap = 0;
     cvs::jpg::Tables *d_tables = nullptr;
@@ -180,30 +261,83 @@ struct JpegDecoder {
     uint32_t *d_mid_state = nullptr, *d_mid_nblk = nullptr;
     int32_t *d_mid_dc = nullptr;
     int32_t *d_dcs = nullptr, *d_tile_dc = nullptr;
-    size_t sub_cap = 0;
     unsigned int *d_changed = nullptr;
     int16_t *d_coef = nullptr;
     uint8_t *d_planes = nullptr;
-    size_t block_cap = 0;
     int coop_blocks_per_sm = 0;
     uint32_t sub_bits = 1024;
-    void release() { cudaFree(d_arena); }
+
+    // Lays the scratch for raw_cap entropy-coded bytes and block_cap blocks out from `base` and returns its size;
+    // base == nullptr only sizes it (the pointers are then null).
+    size_t carve(uint8_t *base, size_t raw_cap, size_t block_cap)
+    {
+        namespace J = cvs::jpg;
+        const size_t nsub = (raw_cap * 8 + sub_bits - 1) / sub_bits + 1;
+        const size_t nhalf = 2 * nsub, ntile = nhalf / J::kEntropyThreads + 2; // the rounds may work on half subsequences
+        const size_t nunstuff = raw_cap / (J::kUnstuffThreads * J::kUnstuffBytes) + 1;
+        size_t off = 0;
+        auto take = [&](auto *&ptr, size_t count) {
+            using T = std::remove_reference_t<decltype(*ptr)>;
+            ptr = base ? reinterpret_cast<T *>(base + off) : nullptr;
+            off += round_up(count * sizeof(T), 256);
+        };
+        take(d_changed, J::kRoundCounters);
+        take(d_entry, nhalf + 2);
+        take(d_unst, raw_cap);
+        take(d_coef, block_cap * 64);
+        take(d_raw, raw_cap);
+        take(d_block_kept, nunstuff);
+        take(d_block_marks, nunstuff);
+        take(d_seg_start, block_cap + 2);
+        take(d_total_bits, 2);
+        take(d_tables, 1);
+        take(d_used, nhalf);
+        take(d_nblk, nhalf);
+        take(d_dcs, 3 * nhalf);
+        take(d_tile_blk, ntile);
+        take(d_tile_dc, 3 * ntile);
+        take(d_hx, 6 * nsub);
+        take(d_hy, 6 * nsub);
+        take(d_hw, 6 * nsub);
+        take(d_hym, 6 * nsub);
+        take(d_hwm, 6 * nsub);
+        take(d_hmap, 16 * nsub);
+        take(d_mid_state, J::kMaxSplit * nsub);
+        take(d_mid_nblk, J::kMaxSplit * nsub);
+        take(d_mid_dc, 3 * J::kMaxSplit * nsub);
+        take(d_planes, block_cap * 64 + 256);
+        d_total_marks = d_total_bits ? d_total_bits + 1 : nullptr;
+        seg_cap = (uint32_t)block_cap + 2;
+        if (base) {
+            // a decode with restart intervals clears [base, base + zero_bytes_fixed + nblocks * 128) with one memset, so
+            // what it must clear besides the coefficients (round counters, entry states, unstuffed string) lies in front
+            const uint8_t *coef = reinterpret_cast<uint8_t *>(d_coef);
+            zero_bytes_fixed = (size_t)(coef - base);
+            assert(reinterpret_cast<uint8_t *>(d_changed + J::kRoundCounters) <= coef &&
+                   reinterpret_cast<uint8_t *>(d_entry + nhalf + 2) <= coef && d_unst + raw_cap <= coef);
+        }
+        return off;
+    }
 };
 
+// decoder sets of a handle: tickets of cvs_submit_jpeg alternate between two, each decoding on a stream of its own
+// (consecutive frames decode side by side); cvs_decode_jpeg_device decodes with the third on the caller's stream
+enum JpegSet { kJpegTicketEven, kJpegTicketOdd, kJpegCallerStream, kJpegSets };
+
 struct Slot {
-    uint8_t *d_in = nullptr;   // raw frame as uploaded
-    int *d_xs = nullptr;
-    uint8_t *d_diff = nullptr;
-    unsigned int *d_pos = nullptr;
-    uint8_t *d_show = nullptr;
-    unsigned int *h_pos = nullptr; // pinned
-    uint32_t *d_starts = nullptr;     // compact wire format: entries before each tile (ntiles + 2 words), on first use
-    uint8_t *d_wire = nullptr;        // compact wire format: encoded frame when the caller's buffer is not mapped
+    DevBuf<uint8_t> d_in;      // raw frame as uploaded
+    DevBuf<int> d_xs;
+    DevBuf<uint8_t> d_diff;
+    DevBuf<unsigned int> d_pos;
+    DevBuf<uint8_t> d_show;
+    PinnedWord h_pos;
+    DevBuf<uint32_t> d_starts;        // compact wire format: entries before each tile (ntiles + 2 words), on first use
+    DevBuf<uint8_t> d_wire;           // compact wire format: encoded frame when the caller's buffer is not mapped
     nvjpegJpegState_t jpeg_state = nullptr; // cvs_submit_jpeg: decoder state of this slot (on first use)
-    uint8_t *d_yuv = nullptr;         // cvs_submit_yuv: the camera's packed YUV frame as uploaded (on first use)
+    DevBuf<uint8_t> d_yuv;            // cvs_submit_yuv: the camera's packed YUV frame as uploaded (on first use)
     uint8_t *u_wire = nullptr;        // caller's buffer of a cvs_submit_wire ticket (nullptr: reference-format ticket)
-    unsigned int *d_status = nullptr; // StatusBits of this ticket's launches (cleared at submit)
-    unsigned int *h_status = nullptr; // pinned copy, valid once ev_pos has fired
+    DevBuf<unsigned int> d_status;    // StatusBits of this ticket's launches (cleared at submit)
+    PinnedWord h_status;              // copy of d_status, valid once ev_pos has fired
     cudaEvent_t ev_h2d0 = nullptr, ev_h2d1 = nullptr, ev_k0 = nullptr, ev_k1 = nullptr, ev_pos = nullptr,
                 ev_p0 = nullptr, ev_done = nullptr;
     bool busy = false;
@@ -236,66 +370,21 @@ bool mapped_device_pointer(const void *host, void **dev)
     return true;
 }
 
+// the stream kernels: k_stream (one warp group; walks a frame in segments with the reference through L2), k_stream_ws
+// (front / back warp groups; a frame or band in one pass with the reference in registers), k_stream_ws_batch (k_stream_ws
+// over one frame of each of several handles)
+enum Family { kFamStream, kFamWs, kFamBatch, kFamilies };
 typedef void (*StreamKernel)(const cvs::StreamParams);
-
-template <int MODE>
-StreamKernel pick_h(bool hi)
-{
-    return hi ? cvs::k_stream<MODE, true> : cvs::k_stream<MODE, false>;
-}
-StreamKernel pick_kernel(int mode, bool hi)
-{
-    switch (mode) {
-    case 1: return pick_h<1>(hi);
-    case 2: return pick_h<2>(hi);
-    case 3: return pick_h<3>(hi);
-    case 4: return pick_h<4>(hi);
-    case 5: return pick_h<5>(hi);
-    case 6: return pick_h<6>(hi);
-    case 7: return pick_h<7>(hi);
-    default: return pick_h<0>(hi);
-    }
-}
-
-template <int MODE>
-StreamKernel pick_ws_h(bool hi)
-{
-    return hi ? cvs::k_stream_ws<MODE, true> : cvs::k_stream_ws<MODE, false>;
-}
-StreamKernel pick_ws_kernel(int mode, bool hi)
-{
-    switch (mode) {
-    case 1: return pick_ws_h<1>(hi);
-    case 2: return pick_ws_h<2>(hi);
-    case 3: return pick_ws_h<3>(hi);
-    case 4: return pick_ws_h<4>(hi);
-    case 5: return pick_ws_h<5>(hi);
-    case 6: return pick_ws_h<6>(hi);
-    case 7: return pick_ws_h<7>(hi);
-    default: return pick_ws_h<0>(hi);
-    }
-}
-
 typedef void (*BatchKernel)(const cvs::StreamParams, const cvs::BatchTable);
 
-template <int MODE>
-BatchKernel pick_batch_h(bool hi)
-{
-    return hi ? cvs::k_stream_ws_batch<MODE, true> : cvs::k_stream_ws_batch<MODE, false>;
-}
-BatchKernel pick_batch_kernel(int mode, bool hi)
-{
-    switch (mode) {
-    case 1: return pick_batch_h<1>(hi);
-    case 2: return pick_batch_h<2>(hi);
-    case 3: return pick_batch_h<3>(hi);
-    case 4: return pick_batch_h<4>(hi);
-    case 5: return pick_batch_h<5>(hi);
-    case 6: return pick_batch_h<6>(hi);
-    case 7: return pick_batch_h<7>(hi);
-    default: return pick_batch_h<0>(hi);
-    }
-}
+// every variant of a stream kernel, by display mode and threshold form: [mode][hi]
+#define CVS_BY_MODE(K)                                                                                                 \
+    {{K<0, false>, K<0, true>}, {K<1, false>, K<1, true>}, {K<2, false>, K<2, true>}, {K<3, false>, K<3, true>},     \
+     {K<4, false>, K<4, true>}, {K<5, false>, K<5, true>}, {K<6, false>, K<6, true>}, {K<7, false>, K<7, true>}}
+const StreamKernel kStreamKernels[8][2] = CVS_BY_MODE(cvs::k_stream);
+const StreamKernel kWsKernels[8][2] = CVS_BY_MODE(cvs::k_stream_ws);
+const BatchKernel kBatchKernels[8][2] = CVS_BY_MODE(cvs::k_stream_ws_batch);
+#undef CVS_BY_MODE
 static_assert(cvs::kMaxBatch == CVS_MAX_BATCH, "batch table and public limit");
 
 } // namespace
@@ -313,113 +402,38 @@ struct cvs_stream_s {
     cvs::ConvWeights weights;
     int sms = 0;
     // glyph atlas
-    uint8_t *d_glyphs = nullptr;
+    DevBuf<uint8_t> d_glyphs;
     int glyph_w = 0, glyph_h = 0;
     std::string glyph_chars;
     // device state
-    uint8_t *d_ref = nullptr;
-    uint32_t *d_lut = nullptr;
-    unsigned int *d_status = nullptr;
-    unsigned int *h_status = nullptr; // pinned
-    unsigned long long *d_desc = nullptr;
-    size_t desc_words = 0;
-    JpegDecoder jd[3];                  // the library's own decoder (cvs_jpeg.cuh), scratch allocated on first use: sets 0 / 1
-                                        // for cvs_submit_jpeg on two streams (consecutive frames decode side by side),
-                                        // set 2 for cvs_decode_jpeg_device on the caller's stream
-    cudaStream_t s_jpg[2] = {nullptr, nullptr};
+    DevBuf<uint8_t> d_ref;
+    DevBuf<uint32_t> d_lut;
+    DevBuf<unsigned int> d_status;
+    PinnedWord h_status;
+    DevBuf<unsigned long long> d_desc;  // look-back descriptors of the stream kernels
+    JpegDecoder jd[kJpegSets];          // the library's own decoder (cvs_jpeg.cuh), scratch allocated on first use
+    cudaStream_t s_jpg[kJpegCallerStream] = {}; // decode streams of the cvs_submit_jpeg sets (on first use)
     bool jpeg_own_only = false;         // own decoder only: refuse the forms it does not cover instead of using nvJPEG
     nvjpegHandle_t jpeg = nullptr;      // cvs_submit_jpeg / cvs_decode_jpeg_device: nvJPEG handle (on first use)
     bool jpeg_batched = false;          // the handle's backend wants the batched entry points (hardware engine / GPU Huffman)
     nvjpegJpegState_t jpeg_state = nullptr; // decoder state of cvs_decode_jpeg_device
-    unsigned int *d_band_pos = nullptr; // banded launches: two arrays of per-frame counts so far (ping-pong)
-    size_t band_frames = 0;
     uint32_t epoch = 0;
-    // scratch that grows with the longest sequence seen
-    uint8_t *d_work = nullptr;   // filtered / overlaid frames
-    size_t work_frames = 0;
-    uint8_t *d_gray1 = nullptr;  // binarise: 1 B per pixel per frame
-    unsigned int *d_hist = nullptr;
-    int *d_thr = nullptr;
-    size_t bin_frames = 0;
-    // geometry of the persistent launch (per kernel variant)
+    // scratch that grows with the longest piece seen
+    DevBuf<unsigned int> d_band_pos; // banded launches: two arrays of per-frame counts so far (ping-pong)
+    DevBuf<uint8_t> d_work;      // filtered / overlaid frames
+    DevBuf<uint8_t> d_gray1;     // binarise: 1 B per pixel per frame
+    DevBuf<unsigned int> d_hist;
+    DevBuf<int> d_thr;
     cudaStream_t s_comp = nullptr, s_h2d = nullptr, s_d2h = nullptr, s_pay = nullptr;
     Slot slot[kSlots];
     int last_slot = -1; // slot of the most recently completed ticket (for cvs_get_timing)
-    int occ_cache[8][2] = {}; // co-resident blocks per SM of each k_stream variant (0 = not queried yet)
-    int occ_ws[8][2] = {};    // same for k_stream_ws
-    int occ_batch[8][2] = {}; // same for k_stream_ws_batch
+    int occ[kFamilies][8][2] = {}; // co-resident blocks per SM of each stream-kernel variant (0 = not queried yet)
     uint64_t next_ticket = 1;
     uint64_t launches = 0;
     float t_h2d = 0, t_kernel = 0, t_d2h = 0;
-    cvs_status seq_status = CVS_OK;
 };
 
 namespace {
-
-cvs_status ensure_desc(cvs_handle h, size_t words)
-{
-    if (h->desc_words >= words) return CVS_OK;
-    if (h->d_desc) {
-        CU_TRY(cudaDeviceSynchronize());
-        CU_TRY(cudaFree(h->d_desc));
-        h->d_desc = nullptr;
-        h->desc_words = 0;
-    }
-    CU_TRY(cudaMalloc(&h->d_desc, words * sizeof(unsigned long long)));
-    CU_TRY(cudaMemset(h->d_desc, 0, words * sizeof(unsigned long long)));
-    h->desc_words = words;
-    return CVS_OK;
-}
-
-cvs_status ensure_work(cvs_handle h, size_t frames)
-{
-    if (h->work_frames >= frames) return CVS_OK;
-    if (h->d_work) {
-        CU_TRY(cudaDeviceSynchronize());
-        CU_TRY(cudaFree(h->d_work));
-        h->d_work = nullptr;
-        h->work_frames = 0;
-    }
-    CU_TRY(cudaMalloc(&h->d_work, frames * h->Npad + 64));
-    CU_TRY(cudaMemset(h->d_work, 0, frames * h->Npad + 64));
-    h->work_frames = frames;
-    return CVS_OK;
-}
-
-cvs_status ensure_bin(cvs_handle h, size_t frames)
-{
-    if (h->bin_frames >= frames) return CVS_OK;
-    if (h->d_gray1 || h->d_hist || h->d_thr) {
-        CU_TRY(cudaDeviceSynchronize());
-        // forget the pointers before anything below can fail: a later call (or cvs_destroy) must not free them again
-        uint8_t *g = h->d_gray1;
-        unsigned int *hi = h->d_hist;
-        int *th = h->d_thr;
-        h->d_gray1 = nullptr;
-        h->d_hist = nullptr;
-        h->d_thr = nullptr;
-        h->bin_frames = 0;
-        cudaFree(g);
-        cudaFree(hi);
-        cudaFree(th);
-    }
-    uint8_t *g = nullptr;
-    unsigned int *hi = nullptr;
-    int *th = nullptr;
-    if (cudaMalloc(&g, frames * h->P16 + 64) != cudaSuccess || cudaMalloc(&hi, frames * 256 * sizeof(unsigned int)) != cudaSuccess ||
-        cudaMalloc(&th, frames * sizeof(int)) != cudaSuccess) {
-        cudaGetLastError();
-        cudaFree(g);
-        cudaFree(hi);
-        cudaFree(th);
-        return fail(CVS_ERR_NOMEM, "binarisation scratch for %zu frames does not fit", frames);
-    }
-    h->d_gray1 = g;
-    h->d_hist = hi;
-    h->d_thr = th;
-    h->bin_frames = frames;
-    return CVS_OK;
-}
 
 cvs_status launch_conv(const uint8_t *in, uint8_t *out, int width, int height, size_t in_stride, size_t out_stride,
                        int nframes, int K, const cvs::ConvWeights &w, cudaStream_t st)
@@ -519,6 +533,137 @@ cvs_status binarize_pass(cvs_handle h, int piece, uint8_t *d_show, size_t show_s
     return CVS_OK;
 }
 
+// scratch for pieces of `frames` frames: the pre-pass's private copy (noise filter, or an overlay that may not be
+// blitted into the frames themselves) and binarisation's gray bytes, histograms and thresholds
+cvs_status ensure_scratch(cvs_handle h, size_t frames, const cvs::OverlayText &txt, bool frames_private, bool binarize)
+{
+    if (h->noise_filter || (txt.n && !frames_private)) CVS_TRY(h->d_work.grow(frames * h->Npad + 64, "pre-pass frames", true));
+    if (binarize) {
+        CVS_TRY(h->d_gray1.grow(frames * h->P16 + 64, "binarisation gray bytes"));
+        CVS_TRY(h->d_hist.grow(frames * 256 * sizeof(unsigned int), "binarisation histograms"));
+        CVS_TRY(h->d_thr.grow(frames * sizeof(int), "binarisation thresholds"));
+    }
+    return CVS_OK;
+}
+
+// What a stream-kernel launch needs: the kernel, G co-resident blocks, each owning the same cps consecutive chunks of
+// every frame (or band) in each of nseg segments, the ring stages and the shared memory they take.
+struct LaunchPlan {
+    bool per_handle = false; // batch only: run the handles one by one through run_frames instead
+    Family fam = kFamWs;
+    const void *kern = nullptr;
+    int G = 0, block = 0, nbands = 1, nstages = 0, smem = 0;
+    uint32_t cps = 0, nseg = 0;
+
+    // The blocks only ever wait for blocks of LOWER index of the same step (look-back), never at a grid barrier, and
+    // G <= the blocks the device can hold, so a plain launch cannot deadlock (blocks are dispatched in index order); a
+    // cooperative launch additionally waits until the WHOLE grid fits at once.  Sequences keep that (every block starts
+    // together: the timings of DESIGN 4.1); a single frame of the submit / exec path is launched plain, so that its
+    // blocks start as SMs become free instead of draining the device first -- with several camera streams on a GPU,
+    // whose decode kernels (cvs_jpeg.cuh) and payload pushes would otherwise run strictly one after the other: 3 JPEG
+    // streams 3.8 k -> 7.1 k frames/s, raw streams unchanged.  (Frames walked in several segments wait for the totals of
+    // ALL blocks of the previous segment: cooperative.)  A batch is launched plain, as the single frames it replaces.
+    bool cooperative(int piece) const { return fam != kFamBatch && (piece > 1 || nseg > 1); }
+};
+
+// The launch plan of the stream kernel over pieces of `piece` frames of h (batch: one frame of each of `piece` handles
+// shaped like h) in display mode kmode.
+// k_stream_ws (front / back warp groups) wherever the reference can stay in registers.  Frames that do not fit one pass
+// of the grid (3840x2160): a SEQUENCE is walked band by band -- every band is a byte range of the frame that does fit,
+// and one k_stream_ws launch takes that band through all frames of the piece with its reference bytes in registers;
+// frame t's entries of band j are appended behind those of the bands before it (counts handed from launch to launch).
+// Same payload, 1.3-1.8x faster than walking the frame in segments with the reference going through L2, which is what
+// single frames (the drop-in call) still do, with the one-group kernel k_stream (k_stream_ws measured 25 against 17 us
+// per 4K frame there).  A batch of such frames, or a batch of one, runs handle by handle (see run_batch).
+cvs_status plan_launch(cvs_handle h, bool batch, int kmode, int piece, LaunchPlan &lp)
+{
+    lp = LaunchPlan();
+    const int g0 = std::min(h->sms, 32 * cvs::kWsLook);
+    const bool one_pass = h->nchunks <= (size_t)g0 * cvs::kThreads;
+    if (batch && (piece == 1 || !one_pass)) {
+        lp.per_handle = true;
+        return CVS_OK;
+    }
+    lp.fam = batch ? kFamBatch : (one_pass || piece >= 4) ? kFamWs : kFamStream;
+    const bool ws = lp.fam != kFamStream;
+    if (!one_pass && ws) lp.nbands = (int)((h->nchunks + (size_t)g0 * cvs::kThreads - 1) / ((size_t)g0 * cvs::kThreads));
+    const uint32_t chunks = (h->nchunks + lp.nbands - 1) / lp.nbands; // of a frame or band
+    const int look_max = ws ? 32 * cvs::kWsLook : cvs::kLook * cvs::kThreads; // predecessors the look-back can read
+    lp.G = std::min({ws ? h->sms : cvs::kBlocksPerSM * h->sms, look_max, (int)chunks});
+    auto split = [&] {
+        lp.nseg = (uint32_t)((chunks + (size_t)lp.G * cvs::kThreads - 1) / ((size_t)lp.G * cvs::kThreads));
+        lp.cps = (uint32_t)((chunks + (size_t)lp.G * lp.nseg - 1) / ((size_t)lp.G * lp.nseg));
+    };
+    split();
+    // k_stream_ws keeps the reference in registers, so it takes a frame (or a band) in one pass; k_stream walks the
+    // frame in segments
+    if ((lp.nseg == 1) != ws)
+        return fail(CVS_ERR_INTERNAL, "%s launch geometry has %u passes per frame", ws ? "k_stream_ws" : "k_stream", lp.nseg);
+    const bool hi = h->hi;
+    lp.kern = lp.fam == kFamBatch ? (const void *)kBatchKernels[kmode][hi]
+              : ws                ? (const void *)kWsKernels[kmode][hi]
+                                  : (const void *)kStreamKernels[kmode][hi];
+    lp.block = ws ? cvs::kWsThreads : cvs::kThreads;
+    // ring depth: all four stages for k_stream_ws (measured +5 % at 1080p), three for k_stream (a deeper prefetch
+    // measured 17 % slower at 3840x2160); fewer if shared memory is short
+    int smem_max = 0;
+    CU_TRY(cudaDeviceGetAttribute(&smem_max, cudaDevAttrMaxSharedMemoryPerBlockOptin, h->device));
+    auto smem_need = [&](int ns) { return ws ? (int)cvs::WsLayout::total(lp.cps, (uint32_t)ns) : cvs::SmemLayout::total(ns); };
+    lp.nstages = ws ? cvs::kStages : cvs::kStages - 1;
+    while (lp.nstages > 2 && smem_need(lp.nstages) > smem_max) lp.nstages--;
+    lp.smem = smem_need(lp.nstages);
+    if (lp.smem > smem_max) return fail(CVS_ERR_INTERNAL, "stream kernel needs %d bytes of shared memory, device has %d", lp.smem, smem_max);
+    int &occ = h->occ[lp.fam][kmode][hi];
+    if (occ == 0) { // first launch of this variant on this handle
+        CU_TRY(cudaFuncSetAttribute(lp.kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max));
+        CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, lp.kern, lp.block, lp.smem));
+    }
+    if (occ < 1) return fail(CVS_ERR_INTERNAL, "stream kernel does not fit on an SM");
+    if (lp.G > occ * h->sms) { // fewer co-resident blocks than planned: recompute
+        const uint32_t nseg = lp.nseg;
+        lp.G = occ * h->sms;
+        split();
+        if (lp.nseg != nseg) return fail(CVS_ERR_INTERNAL, "occupancy changed the segment count");
+    }
+    return CVS_OK;
+}
+
+// The parameters of a launch of h that come from the handle and the plan, under a fresh epoch tag of h's descriptors;
+// the caller adds the frames, the outputs and, for a band, its byte range.
+cvs_status stream_params(cvs_handle h, const LaunchPlan &lp, size_t cap, unsigned int *status, cudaStream_t st,
+                         cvs::StreamParams &p)
+{
+    h->epoch++;
+    if (h->epoch == 0) { // tag wrapped: stale descriptors could alias
+        CU_TRY(cudaMemsetAsync(h->d_desc, 0, h->d_desc.bytes, st));
+        h->epoch = 1;
+    }
+    memset(&p, 0, sizeof p);
+    p.nbytes = h->N;
+    p.nbytes16 = h->N16;
+    p.nchunks = h->nchunks;
+    p.nseg = lp.nseg;
+    p.cps = lp.cps;
+    p.nstages = (uint32_t)lp.nstages;
+    p.cap = cap;
+    p.heat_lut = h->d_lut;
+    p.desc = h->d_desc;
+    p.epoch = h->epoch;
+    p.addc = h->addc;
+    p.status = status;
+    return CVS_OK;
+}
+
+cvs_status launch(cvs_handle h, const LaunchPlan &lp, void **args, int piece, cudaStream_t st)
+{
+    if (lp.cooperative(piece))
+        CU_TRY(cudaLaunchCooperativeKernel(lp.kern, dim3(lp.G), dim3(lp.block), args, (size_t)lp.smem, st));
+    else
+        CU_TRY(cudaLaunchKernel(lp.kern, dim3(lp.G), dim3(lp.block), args, (size_t)lp.smem, st));
+    h->launches++;
+    return CVS_OK;
+}
+
 // One pass of the whole hot path over nframes device-resident frames (A11, kernels.cu:455-520).
 // Long sequences are walked in pieces of at most max_sequence frames; every piece runs the complete chain (noise
 // filter / overlay pre-pass, fused stream kernel, binarisation pass 2), so the scratch buffers are sized by the piece
@@ -540,80 +685,10 @@ cvs_status run_frames(cvs_handle h, const uint8_t *d_frames, size_t stride, int 
     const bool split_gray = binarize && nframes >= 2;
     const int kmode = d_show && !split_gray ? mode : 0; // without a display buffer only the payload is produced
     const int piece_max = h->max_sequence < nframes ? h->max_sequence : nframes;
-    const bool need_work = h->noise_filter || (txt.n && !frames_private);
-    if (need_work) {
-        cvs_status s = ensure_work(h, (size_t)piece_max);
-        if (s) return s;
-    }
-    if (binarize) {
-        cvs_status s = ensure_bin(h, (size_t)piece_max);
-        if (s) return s;
-    }
-
-    // ---- geometry of the persistent launch: G co-resident blocks, each owning the same cps consecutive chunks of
-    //      every frame.  k_stream_ws (front / back warp groups) wherever the reference can stay in registers.
-    // Frames that do not fit one pass of the grid (3840x2160): a SEQUENCE is walked band by band -- every band is a
-    // byte range of the frame that does fit, and one k_stream_ws launch takes that band through all frames of the
-    // piece with its reference bytes in registers; frame t's entries of band j are appended behind those of the bands
-    // before it (counts handed from launch to launch).  Same payload, 1.3-1.8x faster than walking the frame in
-    // segments with the reference going through L2, which is what single frames (the drop-in call) still do, with
-    // the one-group kernel k_stream (k_stream_ws measured 25 against 17 us per 4K frame there).
-    bool ws = true;
-    int nbands = 1;
-    {
-        const int g0 = h->sms < 32 * cvs::kWsLook ? h->sms : 32 * cvs::kWsLook;
-        if (h->nchunks > (size_t)g0 * cvs::kThreads) {
-            if (piece_max >= 4)
-                nbands = (int)((h->nchunks + (size_t)g0 * cvs::kThreads - 1) / ((size_t)g0 * cvs::kThreads));
-            else
-                ws = false; // k_stream (segments, reference through L2)
-        }
-    }
-    const size_t band_chunks_total = (h->nchunks + nbands - 1) / nbands; // chunks per band before rounding to the grid
-    const uint32_t geo_chunks = nbands > 1 ? (uint32_t)band_chunks_total : h->nchunks;
-    int G = ws ? h->sms : cvs::kBlocksPerSM * h->sms;
-    const int look_max = ws ? 32 * cvs::kWsLook : cvs::kLook * cvs::kThreads; // predecessors the look-back can read
-    if (G > look_max) G = look_max;
-    if ((uint32_t)G > geo_chunks) G = (int)geo_chunks;
-    uint32_t nseg = (uint32_t)((geo_chunks + (size_t)G * cvs::kThreads - 1) / ((size_t)G * cvs::kThreads));
-    uint32_t cps = (uint32_t)((geo_chunks + (size_t)G * nseg - 1) / ((size_t)G * nseg));
-    // k_stream_ws keeps the reference in registers, so it takes a frame (or a band) in one pass; k_stream walks the
-    // frame in segments
-    if ((nseg == 1) != ws)
-        return fail(CVS_ERR_INTERNAL, "%s launch geometry has %u passes per frame", ws ? "k_stream_ws" : "k_stream", nseg);
-    StreamKernel kern = ws ? pick_ws_kernel(kmode, h->hi) : pick_kernel(kmode, h->hi);
-    const int block_threads = ws ? cvs::kWsThreads : cvs::kThreads;
-    // ring depth: all four stages for k_stream_ws (measured +5 % at 1080p), three for k_stream (a deeper prefetch
-    // measured 17 % slower at 3840x2160); fewer if shared memory is short
-    int nstages = ws ? cvs::kStages : cvs::kStages - 1;
-    int smem_max = 0;
-    CU_TRY(cudaDeviceGetAttribute(&smem_max, cudaDevAttrMaxSharedMemoryPerBlockOptin, h->device));
-    auto smem_need = [&](int ns) { return ws ? (int)cvs::WsLayout::total(cps, (uint32_t)ns) : cvs::SmemLayout::total(ns); };
-    while (nstages > 2 && smem_need(nstages) > smem_max) nstages--;
-    const int smem_bytes = smem_need(nstages);
-    if (smem_bytes > smem_max) return fail(CVS_ERR_INTERNAL, "stream kernel needs %d bytes of shared memory, device has %d", smem_bytes, smem_max);
-    int &occ = ws ? h->occ_ws[kmode][h->hi ? 1 : 0] : h->occ_cache[kmode][h->hi ? 1 : 0];
-    if (occ == 0) { // first launch of this variant on this handle
-        CU_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max));
-        CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, block_threads, smem_bytes));
-    }
-    if (occ < 1) return fail(CVS_ERR_INTERNAL, "stream kernel does not fit on an SM");
-    if (G > occ * h->sms) { // fewer co-resident blocks than planned: recompute
-        G = occ * h->sms;
-        nseg = (uint32_t)((geo_chunks + (size_t)G * cvs::kThreads - 1) / ((size_t)G * cvs::kThreads));
-        cps = (uint32_t)((geo_chunks + (size_t)G * nseg - 1) / ((size_t)G * nseg));
-        if ((nseg == 1) != ws) return fail(CVS_ERR_INTERNAL, "occupancy changed the segment count");
-    }
-    if (nbands > 1 && h->band_frames < (size_t)piece_max) {
-        if (h->d_band_pos) {
-            CU_TRY(cudaDeviceSynchronize());
-            cudaFree(h->d_band_pos);
-            h->d_band_pos = nullptr;
-            h->band_frames = 0;
-        }
-        CU_TRY(cudaMalloc(&h->d_band_pos, 2 * (size_t)piece_max * sizeof(unsigned int)));
-        h->band_frames = (size_t)piece_max;
-    }
+    CVS_TRY(ensure_scratch(h, (size_t)piece_max, txt, frames_private, binarize));
+    LaunchPlan lp;
+    CVS_TRY(plan_launch(h, false, kmode, piece_max, lp));
+    if (lp.nbands > 1) CVS_TRY(h->d_band_pos.grow(2 * (size_t)piece_max * sizeof(unsigned int), "band counts"));
 
     int done = 0;
     while (done < nframes) {
@@ -622,10 +697,7 @@ cvs_status run_frames(cvs_handle h, const uint8_t *d_frames, size_t stride, int 
         const uint8_t *frames = d_frames + (size_t)done * stride;
         size_t fstride = stride;
 
-        {
-            cvs_status s = pre_pass(h, frames, fstride, piece, txt, frames_private, binarize, st);
-            if (s) return s;
-        }
+        CVS_TRY(pre_pass(h, frames, fstride, piece, txt, frames_private, binarize, st));
         if (split_gray) { // gray byte + histogram of the frames as the diff will see them (filtered, overlay blitted)
             const size_t groups = ((size_t)h->N + cvs::kGroupBytes - 1) / cvs::kGroupBytes;
             dim3 grid(grid_for((groups + cvs::kGrayHistGroupsPerThread - 1) / cvs::kGrayHistGroupsPerThread, 256, h->sms), piece);
@@ -635,66 +707,38 @@ cvs_status run_frames(cvs_handle h, const uint8_t *d_frames, size_t stride, int 
             h->launches++;
         }
 
-        cvs_status s = ensure_desc(h, (size_t)piece * nseg * (G + 1));
-        if (s) return s;
-        const size_t band_bytes = (size_t)G * cps * cvs::kChunkBytes; // bytes of a band (the last one may be shorter)
-        for (int band = 0; band < nbands; band++) {
-            const size_t boff = nbands > 1 ? (size_t)band * band_bytes : 0;
+        CVS_TRY(h->d_desc.grow((size_t)piece * lp.nseg * (lp.G + 1) * sizeof(unsigned long long), "stream-kernel descriptors", true));
+        const size_t band_bytes = (size_t)lp.G * lp.cps * cvs::kChunkBytes; // bytes of a band (the last one may be shorter)
+        for (int band = 0; band < lp.nbands; band++) {
+            const bool banded = lp.nbands > 1;
+            const size_t boff = banded ? (size_t)band * band_bytes : 0;
             if (boff >= h->N) break;
-            const uint32_t bbytes = nbands > 1 ? (uint32_t)((h->N - boff) < band_bytes ? (h->N - boff) : band_bytes) : h->N;
-            h->epoch++;
-            if (h->epoch == 0) { // tag wrapped: stale descriptors could alias
-                CU_TRY(cudaMemsetAsync(h->d_desc, 0, h->desc_words * sizeof(unsigned long long), st));
-                h->epoch = 1;
-            }
-            const bool last_band = nbands == 1 || boff + band_bytes >= h->N;
+            const uint32_t bbytes = banded ? (uint32_t)((h->N - boff) < band_bytes ? (h->N - boff) : band_bytes) : h->N;
+            const bool last_band = !banded || boff + band_bytes >= h->N;
             cvs::StreamParams p;
+            CVS_TRY(stream_params(h, lp, cap, d_status, st, p));
             p.frames = frames + boff;
             p.frame_stride = fstride;
             p.nframes = piece;
             p.ref = h->d_ref + boff;
             p.nbytes = bbytes;
-            p.nbytes16 = nbands > 1 ? (uint32_t)round_up(bbytes, 16) : h->N16;
+            p.nbytes16 = banded ? (uint32_t)round_up(bbytes, 16) : h->N16;
             p.nchunks = (bbytes + cvs::kChunkBytes - 1) / cvs::kChunkBytes;
-            p.nseg = nseg;
-            p.cps = cps;
-            p.nstages = (uint32_t)nstages;
-            p.pos = last_band ? d_pos + done : h->d_band_pos + (size_t)(band & 1) * h->band_frames;
-            p.pos_prior = band ? h->d_band_pos + (size_t)((band - 1) & 1) * h->band_frames : nullptr;
+            p.pos = last_band ? d_pos + done : h->d_band_pos + (size_t)(band & 1) * piece_max;
+            p.pos_prior = band ? h->d_band_pos + (size_t)((band - 1) & 1) * piece_max : nullptr;
             p.index_base = (uint32_t)boff;
             p.xs = d_xs + (size_t)done * cap;
             p.diff = d_diff + (size_t)done * cap;
-            p.cap = cap;
             p.show = d_show ? d_show + (size_t)done * show_stride : nullptr;
             p.show_stride = show_stride;
-            p.gray1 = binarize && !split_gray ? h->d_gray1 : nullptr;
+            p.gray1 = binarize && !split_gray ? h->d_gray1.p : nullptr;
             p.gray_stride = h->P16;
-            p.hist = binarize && !split_gray ? h->d_hist : nullptr;
-            p.heat_lut = h->d_lut;
-            p.desc = h->d_desc;
-            p.epoch = h->epoch;
-            p.addc = h->addc;
-            p.status = d_status;
+            p.hist = binarize && !split_gray ? h->d_hist.p : nullptr;
             void *args[] = {&p};
-            // The blocks only ever wait for blocks of LOWER index of the same step (look-back), never at a grid barrier, and
-            // G <= the blocks the device can hold, so a plain launch cannot deadlock (blocks are dispatched in index
-            // order); a cooperative launch additionally waits until the WHOLE grid fits at once.  Sequences keep that
-            // (every block starts together: the timings of DESIGN 4.1); a single frame of the submit / exec path is
-            // launched plain, so that its blocks start as SMs become free instead of draining the device first -- with
-            // several camera streams on a GPU, whose decode kernels (cvs_jpeg.cuh) and payload pushes would otherwise
-            // run strictly one after the other: 3 JPEG streams 3.8 k -> 7.1 k frames/s, raw streams unchanged.
-            // (frames walked in several segments wait for the totals of ALL blocks of the previous segment: cooperative)
-            if (piece > 1 || nseg > 1)
-                CU_TRY(cudaLaunchCooperativeKernel((const void *)kern, dim3(G), dim3(block_threads), args, (size_t)smem_bytes, st));
-            else
-                CU_TRY(cudaLaunchKernel((const void *)kern, dim3(G), dim3(block_threads), args, (size_t)smem_bytes, st));
-            h->launches++;
+            CVS_TRY(launch(h, lp, args, piece, st));
         }
 
-        if (binarize) {
-            cvs_status s = binarize_pass(h, piece, d_show + (size_t)done * show_stride, show_stride, st);
-            if (s) return s;
-        }
+        if (binarize) CVS_TRY(binarize_pass(h, piece, d_show + (size_t)done * show_stride, show_stride, st));
         done += piece;
     }
     return CVS_OK;
@@ -712,83 +756,35 @@ cvs_status run_batch(const cvs_handle *hs, int n, const uint8_t *const *frames, 
                      bool frames_private, unsigned int *const *status)
 {
     cvs_handle h0 = hs[0];
-    const int G = std::min(std::min(h0->sms, 32 * cvs::kWsLook), (int)h0->nchunks);
-    if (n == 1 || h0->nchunks > (size_t)G * cvs::kThreads) {
-        for (int i = 0; i < n; i++) {
-            cvs_status s = run_frames(hs[i], frames[i], hs[i]->Npad, 1, pos[i], xs[i], diff[i], cap, show ? show[i] : nullptr,
-                                      hs[i]->Npad, texts ? texts[i] : nullptr, st, frames_private, status[i]);
-            if (s) return s;
-        }
+    const bool binarize = (h0->mode == 5 || h0->mode == 7) && show;
+    LaunchPlan lp;
+    CVS_TRY(plan_launch(h0, true, show ? h0->mode : 0, n, lp));
+    if (lp.per_handle) {
+        for (int i = 0; i < n; i++)
+            CVS_TRY(run_frames(hs[i], frames[i], hs[i]->Npad, 1, pos[i], xs[i], diff[i], cap, show ? show[i] : nullptr,
+                               hs[i]->Npad, texts ? texts[i] : nullptr, st, frames_private, status[i]));
         return CVS_OK;
     }
-    const int mode = h0->mode;
-    const bool binarize = (mode == 5 || mode == 7) && show;
-    const int kmode = show ? mode : 0;
-    const uint32_t cps = (h0->nchunks + G - 1) / G;
-    const BatchKernel kern = pick_batch_kernel(kmode, h0->hi);
-    int smem_max = 0;
-    CU_TRY(cudaDeviceGetAttribute(&smem_max, cudaDevAttrMaxSharedMemoryPerBlockOptin, h0->device));
-    int nstages = cvs::kStages;
-    while (nstages > 2 && (int)cvs::WsLayout::total(cps, (uint32_t)nstages) > smem_max) nstages--;
-    const int smem_bytes = (int)cvs::WsLayout::total(cps, (uint32_t)nstages);
-    if (smem_bytes > smem_max) return fail(CVS_ERR_INTERNAL, "stream kernel needs %d bytes of shared memory, device has %d", smem_bytes, smem_max);
-    int &occ = h0->occ_batch[kmode][h0->hi ? 1 : 0];
-    if (occ == 0) {
-        CU_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max));
-        CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, cvs::kWsThreads, smem_bytes));
-    }
-    if (occ < 1) return fail(CVS_ERR_INTERNAL, "stream kernel does not fit on an SM");
 
     cvs::BatchTable tbl; // (copied into the launch's parameters by cudaLaunchKernel)
     for (int i = 0; i < n; i++) {
         cvs_handle h = hs[i];
         const cvs::OverlayText txt = overlay_text(h, texts ? texts[i] : nullptr);
-        if (h->noise_filter || (txt.n && !frames_private)) {
-            cvs_status s = ensure_work(h, 1);
-            if (s) return s;
-        }
-        if (binarize) {
-            cvs_status s = ensure_bin(h, 1);
-            if (s) return s;
-        }
+        CVS_TRY(ensure_scratch(h, 1, txt, frames_private, binarize));
         const uint8_t *f = frames[i];
         size_t fstride = h->Npad;
-        cvs_status s = pre_pass(h, f, fstride, 1, txt, frames_private, binarize, st);
-        if (s) return s;
-        tbl.cam[i] = {f, h->d_ref, pos[i], xs[i], diff[i], show ? show[i] : nullptr, binarize ? h->d_gray1 : nullptr,
-                      binarize ? h->d_hist : nullptr, status[i]};
+        CVS_TRY(pre_pass(h, f, fstride, 1, txt, frames_private, binarize, st));
+        tbl.cam[i] = {f, h->d_ref, pos[i], xs[i], diff[i], show ? show[i] : nullptr, binarize ? h->d_gray1.p : nullptr,
+                      binarize ? h->d_hist.p : nullptr, status[i]};
     }
-    cvs_status s = ensure_desc(h0, (size_t)n * (G + 1));
-    if (s) return s;
-    h0->epoch++;
-    if (h0->epoch == 0) { // tag wrapped: stale descriptors could alias
-        CU_TRY(cudaMemsetAsync(h0->d_desc, 0, h0->desc_words * sizeof(unsigned long long), st));
-        h0->epoch = 1;
-    }
+    CVS_TRY(h0->d_desc.grow((size_t)n * (lp.G + 1) * sizeof(unsigned long long), "stream-kernel descriptors", true));
     cvs::StreamParams p;
-    memset(&p, 0, sizeof p);
+    CVS_TRY(stream_params(h0, lp, cap, status[0], st, p));
     p.nframes = n;
-    p.nbytes = h0->N;
-    p.nbytes16 = h0->N16;
-    p.nchunks = h0->nchunks;
-    p.nseg = 1;
-    p.cps = cps;
-    p.nstages = (uint32_t)nstages;
-    p.cap = cap;
-    p.heat_lut = h0->d_lut;
-    p.desc = h0->d_desc;
-    p.epoch = h0->epoch;
-    p.addc = h0->addc;
-    p.status = status[0];
     void *args[] = {&p, &tbl};
-    // plain launch, as for the single frames it replaces: blocks only wait for blocks of lower index (look-back)
-    CU_TRY(cudaLaunchKernel((const void *)kern, dim3(G), dim3(cvs::kWsThreads), args, (size_t)smem_bytes, st));
-    h0->launches++;
+    CVS_TRY(launch(h0, lp, args, n, st));
     if (binarize)
-        for (int i = 0; i < n; i++) {
-            s = binarize_pass(hs[i], 1, show[i], hs[i]->Npad, st);
-            if (s) return s;
-        }
+        for (int i = 0; i < n; i++) CVS_TRY(binarize_pass(hs[i], 1, show[i], hs[i]->Npad, st));
     return CVS_OK;
 }
 
@@ -914,40 +910,34 @@ cvs_status init_device_state(cvs_handle h, const cvs_config *cfg)
     CU_TRY(cudaStreamCreateWithFlags(&h->s_h2d, cudaStreamNonBlocking));
     CU_TRY(cudaStreamCreateWithFlags(&h->s_d2h, cudaStreamNonBlocking));
     CU_TRY(cudaStreamCreateWithFlags(&h->s_pay, cudaStreamNonBlocking));
-    CU_TRY(cudaMalloc(&h->d_ref, h->Npad + 64));
-    CU_TRY(cudaMemset(h->d_ref, 0, h->Npad + 64));
+    CVS_TRY(h->d_ref.grow(h->Npad + 64, "reference frame", true));
     CU_TRY(cudaMemcpy(h->d_ref, cfg->base_frame, h->N, cudaMemcpyHostToDevice)); // kernels.cu:406
     {
         uint32_t lut[768];
         build_heat_lut(lut);
-        CU_TRY(cudaMalloc(&h->d_lut, sizeof lut));
+        CVS_TRY(h->d_lut.grow(sizeof lut, "heat-map table"));
         CU_TRY(cudaMemcpy(h->d_lut, lut, sizeof lut, cudaMemcpyHostToDevice));
     }
-    CU_TRY(cudaMalloc(&h->d_status, sizeof(unsigned int)));
-    CU_TRY(cudaMemset(h->d_status, 0, sizeof(unsigned int)));
-    CU_TRY(cudaHostAlloc(&h->h_status, sizeof(unsigned int), cudaHostAllocDefault));
-    *h->h_status = 0;
+    CVS_TRY(h->d_status.grow(sizeof(unsigned int), "status word", true));
+    CVS_TRY(h->h_status.alloc());
     if (cfg->glyphs && cfg->glyph_w > 0 && cfg->glyph_h > 0 && cfg->glyph_chars) {
         h->glyph_chars = cfg->glyph_chars;
         h->glyph_w = cfg->glyph_w;
         h->glyph_h = cfg->glyph_h;
         size_t bytes = h->glyph_chars.size() * 3 * (size_t)cfg->glyph_w * cfg->glyph_h;
-        CU_TRY(cudaMalloc(&h->d_glyphs, bytes + 16));
+        CVS_TRY(h->d_glyphs.grow(bytes + 16, "glyph atlas"));
         CU_TRY(cudaMemcpy(h->d_glyphs, cfg->glyphs, bytes, cudaMemcpyHostToDevice));
     }
     const size_t cap = round_up(h->N, 4);
     for (Slot &s : h->slot) {
-        CU_TRY(cudaMalloc(&s.d_in, h->Npad + 64));
-        CU_TRY(cudaMemset(s.d_in, 0, h->Npad + 64));
-        CU_TRY(cudaMalloc(&s.d_xs, cap * sizeof(int)));
-        CU_TRY(cudaMalloc(&s.d_diff, cap));
-        CU_TRY(cudaMalloc(&s.d_pos, sizeof(unsigned int)));
-        if (h->mode) CU_TRY(cudaMalloc(&s.d_show, h->Npad + 64));
-        CU_TRY(cudaHostAlloc(&s.h_pos, sizeof(unsigned int), cudaHostAllocDefault));
-        CU_TRY(cudaMalloc(&s.d_status, sizeof(unsigned int)));
-        CU_TRY(cudaMemset(s.d_status, 0, sizeof(unsigned int)));
-        CU_TRY(cudaHostAlloc(&s.h_status, sizeof(unsigned int), cudaHostAllocDefault));
-        *s.h_status = 0;
+        CVS_TRY(s.d_in.grow(h->Npad + 64, "upload frame", true));
+        CVS_TRY(s.d_xs.grow(cap * sizeof(int), "payload indices"));
+        CVS_TRY(s.d_diff.grow(cap, "payload bytes"));
+        CVS_TRY(s.d_pos.grow(sizeof(unsigned int), "payload count"));
+        if (h->mode) CVS_TRY(s.d_show.grow(h->Npad + 64, "display frame"));
+        CVS_TRY(s.h_pos.alloc());
+        CVS_TRY(s.d_status.grow(sizeof(unsigned int), "status word", true));
+        CVS_TRY(s.h_status.alloc());
         cudaEvent_t *evs[] = {&s.ev_h2d0, &s.ev_h2d1, &s.ev_k0, &s.ev_k1, &s.ev_pos, &s.ev_p0, &s.ev_done};
         for (cudaEvent_t *e : evs) CU_TRY(cudaEventCreate(e));
     }
@@ -975,32 +965,20 @@ cvs_status cvs_destroy(cvs_handle h)
     cudaSetDevice(h->device);
     cudaDeviceSynchronize();
     for (Slot &s : h->slot) {
-        cudaFree(s.d_in); cudaFree(s.d_xs); cudaFree(s.d_diff); cudaFree(s.d_pos); cudaFree(s.d_show);
-        cudaFreeHost(s.h_pos);
-        cudaFree(s.d_status);
-        cudaFreeHost(s.h_status);
-        cudaFree(s.d_starts);
-        cudaFree(s.d_wire);
-        cudaFree(s.d_yuv);
         if (s.jpeg_state && g_nvjpeg.ok) g_nvjpeg.StateDestroy(s.jpeg_state);
         cudaEvent_t evs[] = {s.ev_h2d0, s.ev_h2d1, s.ev_k0, s.ev_k1, s.ev_pos, s.ev_p0, s.ev_done};
         for (cudaEvent_t e : evs)
             if (e) cudaEventDestroy(e);
     }
-    cudaFree(h->d_ref); cudaFree(h->d_lut); cudaFree(h->d_status); cudaFreeHost(h->h_status);
-    cudaFree(h->d_band_pos);
-    for (JpegDecoder &jd : h->jd) jd.release();
     for (cudaStream_t js : h->s_jpg)
         if (js) cudaStreamDestroy(js);
     if (h->jpeg_state && g_nvjpeg.ok) g_nvjpeg.StateDestroy(h->jpeg_state);
     if (h->jpeg && g_nvjpeg.ok) g_nvjpeg.Destroy(h->jpeg);
-    cudaFree(h->d_desc); cudaFree(h->d_work); cudaFree(h->d_gray1); cudaFree(h->d_hist); cudaFree(h->d_thr);
-    cudaFree(h->d_glyphs);
     if (h->s_comp) cudaStreamDestroy(h->s_comp);
     if (h->s_h2d) cudaStreamDestroy(h->s_h2d);
     if (h->s_d2h) cudaStreamDestroy(h->s_d2h);
     if (h->s_pay) cudaStreamDestroy(h->s_pay);
-    delete h;
+    delete h; // device and pinned memory: freed by the buffers of the handle and its slots
     return CVS_OK;
 }
 
@@ -1111,70 +1089,16 @@ static cvs_status jpeg_decode_own(cvs_handle h, JpegDecoder &jd, const uint8_t *
     if (g.width != h->width || g.height != h->height)
         return fail(CVS_ERR_INVALID, "JPEG is %dx%d, the stream is %dx%d", g.width, g.height, h->width, h->height);
 
-    // ---- scratch: one arena, carved; the part every decode needs zeroed (round counters, entry states, the unstuffed
-    //      string's padding, the coefficients) sits in front so that one memset clears it
+    // ---- scratch: one arena, carved (JpegDecoder::carve), grown by half again when a frame needs more
     const size_t raw_pad = round_up(P.scan_bytes, 4096) + 4096;
     const size_t luma_bytes = (size_t)g.mcux * 8 * g.H * g.mcuy * 8 * g.V, chroma_bytes = (size_t)g.mcux * 8 * g.mcuy * 8;
     if (raw_pad > jd.raw_cap || g.nblocks > jd.block_cap) {
         const size_t raw_cap = std::max(jd.raw_cap, raw_pad + raw_pad / 2), block_cap = std::max<size_t>(jd.block_cap, g.nblocks);
-        CU_TRY(cudaStreamSynchronize(st));
-        cudaFree(jd.d_arena);
-        jd.d_arena = nullptr;
-        jd.raw_cap = jd.block_cap = jd.sub_cap = 0;
-        const size_t nsub_cap = (raw_cap * 8 + jd.sub_bits - 1) / jd.sub_bits + 1;
-        const size_t nhalf_cap = 2 * nsub_cap, ntile_cap = nhalf_cap / J::kEntropyThreads + 2; // the rounds may work on half subsequences
-        size_t off = 0;
-        auto carve = [&](size_t bytes) {
-            const size_t o = off;
-            off += round_up(bytes, 256);
-            return o;
-        };
-        const size_t o_changed = carve(J::kRoundCounters * sizeof(unsigned int)), o_entry = carve((nhalf_cap + 2) * sizeof(uint32_t)),
-                     o_unst = carve(raw_cap), o_coef = carve(block_cap * 64 * sizeof(int16_t));
-        jd.zero_bytes_fixed = o_coef; // + nblocks * 128 of the coefficients
-        const size_t o_raw = carve(raw_cap), o_kept = carve((raw_cap / (J::kUnstuffThreads * J::kUnstuffBytes) + 1) * sizeof(uint32_t)),
-                     o_marks = carve((raw_cap / (J::kUnstuffThreads * J::kUnstuffBytes) + 1) * sizeof(uint32_t)),
-                     o_seg = carve((block_cap + 2) * sizeof(uint32_t)), o_total = carve(2 * sizeof(uint32_t)), o_tables = carve(sizeof(J::Tables)), o_used = carve(nhalf_cap * sizeof(uint32_t)),
-                     o_nblk = carve(nhalf_cap * sizeof(uint32_t)), o_dcs = carve(3 * nhalf_cap * sizeof(int32_t)),
-                     o_tile_blk = carve(ntile_cap * sizeof(uint32_t)), o_tile_dc = carve(3 * ntile_cap * sizeof(int32_t)),
-                     o_hx = carve(6 * nsub_cap * sizeof(uint32_t)), o_hy = carve(6 * nsub_cap * sizeof(uint32_t)),
-                     o_hw = carve(6 * nsub_cap * sizeof(uint32_t)), o_hym = carve(6 * nsub_cap * sizeof(uint32_t)),
-                     o_hwm = carve(6 * nsub_cap * sizeof(uint32_t)),
-                     o_hmap = carve(16 * nsub_cap), o_mid_state = carve(J::kMaxSplit * nsub_cap * sizeof(uint32_t)),
-                     o_mid_nblk = carve(J::kMaxSplit * nsub_cap * sizeof(uint32_t)),
-                     o_mid_dc = carve(3 * J::kMaxSplit * nsub_cap * sizeof(int32_t)), o_planes = carve(block_cap * 64 + 256);
-        CU_TRY(cudaMalloc(&jd.d_arena, off));
-        uint8_t *a = jd.d_arena;
-        jd.d_changed = reinterpret_cast<unsigned int *>(a + o_changed);
-        jd.d_entry = reinterpret_cast<uint32_t *>(a + o_entry);
-        jd.d_unst = a + o_unst;
-        jd.d_coef = reinterpret_cast<int16_t *>(a + o_coef);
-        jd.d_raw = a + o_raw;
-        jd.d_block_kept = reinterpret_cast<uint32_t *>(a + o_kept);
-        jd.d_block_marks = reinterpret_cast<uint32_t *>(a + o_marks);
-        jd.d_seg_start = reinterpret_cast<uint32_t *>(a + o_seg);
-        jd.seg_cap = (uint32_t)block_cap + 2;
-        jd.d_total_bits = reinterpret_cast<uint32_t *>(a + o_total);
-        jd.d_total_marks = jd.d_total_bits + 1;
-        jd.d_tables = reinterpret_cast<J::Tables *>(a + o_tables);
-        jd.d_used = reinterpret_cast<uint32_t *>(a + o_used);
-        jd.d_nblk = reinterpret_cast<uint32_t *>(a + o_nblk);
-        jd.d_dcs = reinterpret_cast<int32_t *>(a + o_dcs);
-        jd.d_tile_blk = reinterpret_cast<uint32_t *>(a + o_tile_blk);
-        jd.d_tile_dc = reinterpret_cast<int32_t *>(a + o_tile_dc);
-        jd.d_hx = reinterpret_cast<uint32_t *>(a + o_hx);
-        jd.d_hy = reinterpret_cast<uint32_t *>(a + o_hy);
-        jd.d_hw = reinterpret_cast<uint32_t *>(a + o_hw);
-        jd.d_hym = reinterpret_cast<uint32_t *>(a + o_hym);
-        jd.d_hwm = reinterpret_cast<uint32_t *>(a + o_hwm);
-        jd.d_hmap = a + o_hmap;
-        jd.d_mid_state = reinterpret_cast<uint32_t *>(a + o_mid_state);
-        jd.d_mid_nblk = reinterpret_cast<uint32_t *>(a + o_mid_nblk);
-        jd.d_mid_dc = reinterpret_cast<int32_t *>(a + o_mid_dc);
-        jd.d_planes = a + o_planes;
+        jd.raw_cap = jd.block_cap = 0; // until the arena holds the new layout
+        CVS_TRY(jd.arena.grow_on(st, jd.carve(nullptr, raw_cap, block_cap), "JPEG decoder scratch"));
+        jd.carve(jd.arena, raw_cap, block_cap);
         jd.raw_cap = raw_cap;
         jd.block_cap = block_cap;
-        jd.sub_cap = nsub_cap;
         jd.tables_valid = false;
     }
     if (!jd.tables_valid || memcmp(&jd.tables_host, &P.t, sizeof(J::Tables)) != 0) {
@@ -1191,7 +1115,7 @@ static cvs_status jpeg_decode_own(cvs_handle h, JpegDecoder &jd, const uint8_t *
 
     if (P.restart_interval) {
         // ---- scratch cleared, FF 00 -> FF and FF Dn dropped (launches of their own on this path)
-        CU_TRY(cudaMemsetAsync(jd.d_arena, 0, jd.zero_bytes_fixed + (size_t)g.nblocks * 64 * sizeof(int16_t), st));
+        CU_TRY(cudaMemsetAsync(jd.arena, 0, jd.zero_bytes_fixed + (size_t)g.nblocks * 64 * sizeof(int16_t), st));
         J::k_unstuff_count<<<ublocks, J::kUnstuffThreads, 0, st>>>(jd.d_raw, raw_len, jd.d_block_kept, jd.d_block_marks);
         J::k_unstuff_write<<<ublocks, J::kUnstuffThreads, 0, st>>>(jd.d_raw, raw_len, jd.d_block_kept, jd.d_block_marks, jd.d_unst,
                                                                      jd.d_total_bits, jd.d_seg_start, jd.seg_cap, jd.d_total_marks);
@@ -1282,7 +1206,7 @@ static cvs_status jpeg_decode_own(cvs_handle h, JpegDecoder &jd, const uint8_t *
 }
 
 // decode one baseline JPEG of the stream's frame size into d_out (BGR interleaved, pitch 3*width), asynchronously on `st`
-static cvs_status jpeg_decode(cvs_handle h, int set, nvjpegJpegState_t *state, const uint8_t *jpeg, size_t jpeg_bytes,
+static cvs_status jpeg_decode(cvs_handle h, JpegSet set, nvjpegJpegState_t *state, const uint8_t *jpeg, size_t jpeg_bytes,
                               uint8_t *d_out, cudaStream_t st, unsigned int *d_status)
 {
     bool unsupported = false;
@@ -1326,7 +1250,7 @@ static cvs_status egress(cvs_handle h, Slot &s, const uint8_t *frame, uint8_t *d
         // encoded frame -- its size depends on the count, which only the device knows yet -- straight into the
         // caller's pinned buffer; a pageable buffer gets the bytes from s.d_wire in cvs_wait
         void *dev_wire = nullptr;
-        s.pushed = mapped_device_pointer(wire_out, &dev_wire) && ((uintptr_t)dev_wire % 16 == 0);
+        s.pushed = mapped_device_pointer(wire_out, &dev_wire) && aligned16(dev_wire);
         cvs::k_wire_bounds<<<(ntiles + 256) / 256, 256, 0, h->s_d2h>>>(s.d_xs, s.d_pos, cap, ntiles, s.d_starts);
         CU_TRY(cudaGetLastError());
         cvs::k_wire_pack<<<2 * h->sms, 256, 0, h->s_d2h>>>(s.d_xs, s.d_diff, s.d_pos, cap, ntiles, s.d_starts,
@@ -1342,8 +1266,7 @@ static cvs_status egress(cvs_handle h, Slot &s, const uint8_t *frame, uint8_t *d
         const size_t guess = round_up(h->pred, 4);
         s.spec = (uint32_t)(guess > h->N ? h->N : guess);
     } else {
-        s.pushed = mapped_device_pointer(diff_out, &dev_diff) && mapped_device_pointer(xs, &dev_xs) &&
-                   ((uintptr_t)dev_diff % 16 == 0) && ((uintptr_t)dev_xs % 16 == 0);
+        s.pushed = mapped_device_pointer(diff_out, &dev_diff) && mapped_device_pointer(xs, &dev_xs) && aligned16(dev_diff, dev_xs);
     }
     if (s.pushed && !wire_out) {
         cvs::k_payload_push<<<h->sms, 256, 0, h->s_d2h>>>(s.d_xs, s.d_diff, s.d_pos, (int *)dev_xs, (uint8_t *)dev_diff, cap);
@@ -1400,6 +1323,36 @@ static void yuv_packed_planes(int format, const uint8_t *base, int width, int he
     pitches[2] = (size_t)width / 2;
 }
 
+// H2D of a ticket's frame into s.d_in (kernels.cu:461) between the slot's timing events: the N-byte BGR frame, or
+// (yuv_format != 0) a packed YUV frame into s.d_yuv, converted on the compute stream later, or (jpeg_bytes != 0) the
+// camera's JPEG bitstream, decoded on the device.  JPEG tickets alternate between two decode streams with their own
+// scratch: frame t+1 is decoded beside frame t (a decode is a latency chain that leaves most of the GPU idle); the
+// stream kernel still takes the frames in ticket order.  The compute stream waits for the frame and marks ev_k0.
+static cvs_status ingest(cvs_handle h, Slot &s, const uint8_t *frame, size_t jpeg_bytes = 0, int yuv_format = 0)
+{
+    cudaStream_t s_in = h->s_h2d;
+    const JpegSet jset = (h->next_ticket & 1) ? kJpegTicketOdd : kJpegTicketEven;
+    if (jpeg_bytes) {
+        if (!h->s_jpg[jset]) CU_TRY(cudaStreamCreateWithFlags(&h->s_jpg[jset], cudaStreamNonBlocking));
+        s_in = h->s_jpg[jset];
+    }
+    CU_TRY(cudaEventRecord(s.ev_h2d0, s_in));
+    if (jpeg_bytes) {
+        // (the ticket's status word is cleared here, in front of the decoder that may raise bits in it)
+        CU_TRY(cudaMemsetAsync(s.d_status, 0, sizeof(unsigned int), s_in));
+        CVS_TRY(jpeg_decode(h, jset, &s.jpeg_state, frame, jpeg_bytes, s.d_in, s_in, s.d_status));
+    } else if (yuv_format) {
+        CU_TRY(cudaMemcpyAsync(s.d_yuv, frame, cvs_yuv_frame_bytes(yuv_format, h->width, h->height), cudaMemcpyHostToDevice,
+                               h->s_h2d));
+    } else {
+        CU_TRY(cudaMemcpyAsync(s.d_in, frame, h->N, cudaMemcpyHostToDevice, h->s_h2d));
+    }
+    CU_TRY(cudaEventRecord(s.ev_h2d1, s_in));
+    CU_TRY(cudaStreamWaitEvent(h->s_comp, s.ev_h2d1, 0));
+    CU_TRY(cudaEventRecord(s.ev_k0, h->s_comp));
+    return CVS_OK;
+}
+
 // jpeg_bytes != 0: `frame` is the camera's JPEG bitstream; yuv_format != 0: `frame` is a packed YUV frame of that format
 // (checked by the caller); otherwise the N-byte BGR frame
 static cvs_status submit_common(cvs_handle h, const uint8_t *frame, uint8_t *diff_out, uint8_t *show, const char *text,
@@ -1411,42 +1364,18 @@ static cvs_status submit_common(cvs_handle h, const uint8_t *frame, uint8_t *dif
     if (!frame || !ticket || (!wire_out && (!diff_out || !pos || !xs))) return fail(CVS_ERR_INVALID, "null argument");
     Slot &s = h->slot[h->next_ticket % kSlots];
     if (s.busy) return fail(CVS_ERR_INVALID, "%d tickets are already outstanding; cvs_wait the oldest first", kSlots);
-    const uint32_t ntiles = (h->N + cvs::kWireTile - 1) / cvs::kWireTile;
-    if (wire_out && !s.d_starts) {
-        CU_TRY(cudaMalloc(&s.d_starts, (size_t)(ntiles + 2) * sizeof(uint32_t)));
-        CU_TRY(cudaMalloc(&s.d_wire, cvs_wire_bound(h->width, h->height)));
+    if (wire_out) {
+        const uint32_t ntiles = (h->N + cvs::kWireTile - 1) / cvs::kWireTile;
+        CVS_TRY(s.d_starts.grow((size_t)(ntiles + 2) * sizeof(uint32_t), "wire tile starts"));
+        CVS_TRY(s.d_wire.grow(cvs_wire_bound(h->width, h->height), "wire frame"));
     }
-    const size_t yuv_bytes = yuv_format ? cvs_yuv_frame_bytes(yuv_format, h->width, h->height) : 0;
-    if (yuv_format && !s.d_yuv) // sized for the largest layout (YUYV, 2WH), so tickets of every format share it
-        CU_TRY(cudaMalloc(&s.d_yuv, round_up(cvs_yuv_frame_bytes(CVS_YUV_YUYV, h->width, h->height), 16)));
+    // sized for the largest layout (YUYV, 2WH), so tickets of every format share it
+    if (yuv_format) CVS_TRY(s.d_yuv.grow(round_up(cvs_yuv_frame_bytes(CVS_YUV_YUYV, h->width, h->height), 16), "YUV frame"));
 
     const double th0 = h->trace ? host_us() : 0;
-    // H2D (kernels.cu:461) -- of the raw frame, or of the camera's JPEG bitstream, decoded on the device.  JPEG tickets
-    // alternate between two decode streams with their own scratch: frame t+1 is decoded beside frame t (a decode is a
-    // latency chain that leaves most of the GPU idle); the stream kernel below still takes the frames in ticket order.
-    cudaStream_t s_in = h->s_h2d;
-    const int jset = (int)(h->next_ticket & 1);
-    if (jpeg_bytes) {
-        if (!h->s_jpg[jset]) CU_TRY(cudaStreamCreateWithFlags(&h->s_jpg[jset], cudaStreamNonBlocking));
-        s_in = h->s_jpg[jset];
-    }
-    CU_TRY(cudaEventRecord(s.ev_h2d0, s_in));
-    if (jpeg_bytes) {
-        // (the ticket's status word is cleared here, in front of the decoder that may raise bits in it)
-        CU_TRY(cudaMemsetAsync(s.d_status, 0, sizeof(unsigned int), s_in));
-        st = jpeg_decode(h, jset, &s.jpeg_state, frame, jpeg_bytes, s.d_in, s_in, s.d_status);
-        if (st) return st;
-    } else if (yuv_format) { // the camera's packed frame; converted on the compute stream below
-        CU_TRY(cudaMemcpyAsync(s.d_yuv, frame, yuv_bytes, cudaMemcpyHostToDevice, h->s_h2d));
-    } else {
-        CU_TRY(cudaMemcpyAsync(s.d_in, frame, h->N, cudaMemcpyHostToDevice, h->s_h2d));
-    }
-    CU_TRY(cudaEventRecord(s.ev_h2d1, s_in));
-    // kernels
-    CU_TRY(cudaStreamWaitEvent(h->s_comp, s.ev_h2d1, 0));
-    CU_TRY(cudaEventRecord(s.ev_k0, h->s_comp));
+    CVS_TRY(ingest(h, s, frame, jpeg_bytes, yuv_format));
     const size_t cap = round_up(h->N, 4);
-    uint8_t *dshow = (h->mode && show) ? s.d_show : nullptr;
+    uint8_t *dshow = (h->mode && show) ? s.d_show.p : nullptr;
     const double th1 = h->trace ? host_us() : 0;
     if (!jpeg_bytes) CU_TRY(cudaMemsetAsync(s.d_status, 0, sizeof(unsigned int), h->s_comp));
     if (yuv_format) { // (inside ev_k0 .. ev_k1: cvs_get_timing counts the conversion as kernel time)
@@ -1519,17 +1448,13 @@ cvs_status cvs_submit_io_batch(const cvs_handle *hs, int n, const uint8_t *const
         Slot &s = h->slot[h->next_ticket % kSlots];
         // upload on the stream's own copy stream; its compute stream then marks the point behind the upload and behind
         // the stream's earlier tickets (which updated the reference this batch starts from)
-        CU_TRY(cudaEventRecord(s.ev_h2d0, h->s_h2d));
-        CU_TRY(cudaMemcpyAsync(s.d_in, frames[i], h->N, cudaMemcpyHostToDevice, h->s_h2d));
-        CU_TRY(cudaEventRecord(s.ev_h2d1, h->s_h2d));
-        CU_TRY(cudaStreamWaitEvent(h->s_comp, s.ev_h2d1, 0));
-        CU_TRY(cudaEventRecord(s.ev_k0, h->s_comp));
+        CVS_TRY(ingest(h, s, frames[i]));
         CU_TRY(cudaStreamWaitEvent(L->s_comp, s.ev_k0, 0));
         d_frames[i] = s.d_in;
         d_pos[i] = s.d_pos;
         d_xs[i] = s.d_xs;
         d_diff[i] = s.d_diff;
-        d_show[i] = any_show ? s.d_show : nullptr; // (a camera without a show buffer still gets its frame: not copied out)
+        d_show[i] = any_show ? s.d_show.p : nullptr; // (a camera without a show buffer still gets its frame: not copied out)
         d_status[i] = s.d_status;
         CU_TRY(cudaMemsetAsync(s.d_status, 0, sizeof(unsigned int), L->s_comp));
     }
@@ -1543,7 +1468,7 @@ cvs_status cvs_submit_io_batch(const cvs_handle *hs, int n, const uint8_t *const
         CU_TRY(cudaEventRecord(s.ev_k1, L->s_comp));
         CU_TRY(cudaStreamWaitEvent(h->s_comp, s.ev_k1, 0));
         uint8_t *sh = show ? show[i] : nullptr;
-        st = egress(h, s, frames[i], diff_out[i], sh, sh && any_show ? s.d_show : nullptr, pos[i], xs[i], nullptr);
+        st = egress(h, s, frames[i], diff_out[i], sh, sh && any_show ? s.d_show.p : nullptr, pos[i], xs[i], nullptr);
         if (st) return st;
         tickets[i] = s.ticket;
     }
@@ -1570,7 +1495,7 @@ cvs_status cvs_decode_jpeg_device(cvs_handle h, const uint8_t *jpeg, size_t jpeg
     if (st) return st;
     if (!jpeg || jpeg_bytes == 0 || !d_out) return fail(CVS_ERR_INVALID, "null argument");
     // (status bits of the decoder go to the handle's own status word: cvs_decode_status reads it)
-    st = jpeg_decode(h, 2, &h->jpeg_state, jpeg, jpeg_bytes, d_out, (cudaStream_t)cuda_stream, h->d_status);
+    st = jpeg_decode(h, kJpegCallerStream, &h->jpeg_state, jpeg, jpeg_bytes, d_out, (cudaStream_t)cuda_stream, h->d_status);
     if (st) return st;
     CU_TRY(cudaMemcpyAsync(h->h_status, h->d_status, sizeof(unsigned int), cudaMemcpyDeviceToHost, (cudaStream_t)cuda_stream));
     return CVS_OK;
@@ -1729,14 +1654,12 @@ cvs_status cvs_run_sequence_device(cvs_handle h, const uint8_t *d_frames, size_t
     cvs_status st = check_handle(h);
     if (st) return st;
     if (nframes < 0 || !d_frames || !d_pos || !d_xs || !d_diff) return fail(CVS_ERR_INVALID, "null argument");
-    if (((uintptr_t)d_frames & 15) || (frame_stride & 15) || ((uintptr_t)d_xs & 15) || ((uintptr_t)d_diff & 15) ||
-        (d_show && (((uintptr_t)d_show & 15) || (show_stride & 15))))
+    if (!aligned16(d_frames, frame_stride, d_xs, d_diff) || (d_show && !aligned16(d_show, show_stride)))
         return fail(CVS_ERR_ALIGN, "device pointers and strides must be 16-byte aligned");
     if (frame_stride < h->N16) return fail(CVS_ERR_INVALID, "frame_stride %zu < %u", frame_stride, h->N16);
     if (d_show && show_stride < h->N) return fail(CVS_ERR_INVALID, "show_stride too small");
     if (payload_capacity == 0 || (payload_capacity & 3))
         return fail(CVS_ERR_INVALID, "payload_capacity must be a positive multiple of 4");
-    h->seq_status = CVS_OK;
     cudaStream_t s = (cudaStream_t)cuda_stream;
     st = run_frames(h, d_frames, frame_stride, nframes, d_pos, d_xs, d_diff, payload_capacity, d_show, show_stride, text, s,
                     /*frames_private=*/false, h->d_status);
@@ -1754,9 +1677,9 @@ cvs_status cvs_run_batch_device(const cvs_handle *hs, int n, const uint8_t *cons
     if (!d_frames || !d_pos || !d_xs || !d_diff) return fail(CVS_ERR_INVALID, "null argument");
     for (int i = 0; i < n; i++)
         if (!d_frames[i]) return fail(CVS_ERR_INVALID, "null frame at %d", i);
-    for (int i = 0; i < n; i++)
-        if ((uintptr_t)d_frames[i] & 15) return fail(CVS_ERR_ALIGN, "device pointers and strides must be 16-byte aligned");
-    if (((uintptr_t)d_xs & 15) || ((uintptr_t)d_diff & 15) || (d_show && (((uintptr_t)d_show & 15) || (show_stride & 15))))
+    bool aligned = aligned16(d_xs, d_diff) && (!d_show || aligned16(d_show, show_stride));
+    for (int i = 0; i < n; i++) aligned = aligned && aligned16(d_frames[i]);
+    if (!aligned)
         return fail(CVS_ERR_ALIGN, "device pointers and strides must be 16-byte aligned");
     if (d_show && show_stride < hs[0]->N) return fail(CVS_ERR_INVALID, "show_stride too small");
     if (payload_capacity == 0 || (payload_capacity & 3))
@@ -1765,7 +1688,6 @@ cvs_status cvs_run_batch_device(const cvs_handle *hs, int n, const uint8_t *cons
     int *xs[CVS_MAX_BATCH];
     uint8_t *diff[CVS_MAX_BATCH], *show[CVS_MAX_BATCH];
     for (int i = 0; i < n; i++) {
-        hs[i]->seq_status = CVS_OK;
         pos[i] = d_pos + i;
         xs[i] = d_xs + (size_t)i * payload_capacity;
         diff[i] = d_diff + (size_t)i * payload_capacity;
@@ -1816,7 +1738,7 @@ cvs_status cvs_heat_map_device(const uint8_t *d_prev, const uint8_t *d_cur, uint
     cvs_status st = filter_common(sms);
     if (st) return st;
     if (!d_prev || !d_cur || !d_out || width <= 0 || height <= 0) return fail(CVS_ERR_INVALID, "bad argument");
-    if (((uintptr_t)d_prev | (uintptr_t)d_cur | (uintptr_t)d_out) & 15) return fail(CVS_ERR_ALIGN, "16-byte alignment required");
+    if (!aligned16(d_prev, d_cur, d_out)) return fail(CVS_ERR_ALIGN, "16-byte alignment required");
     uint32_t *lut = nullptr;
     st = device_heat_lut(&lut);
     if (st) return st;
@@ -1833,7 +1755,7 @@ cvs_status cvs_red_map_device(const uint8_t *d_prev, const uint8_t *d_cur, uint8
     cvs_status st = filter_common(sms);
     if (st) return st;
     if (!d_prev || !d_cur || !d_out || width <= 0 || height <= 0) return fail(CVS_ERR_INVALID, "bad argument");
-    if (((uintptr_t)d_prev | (uintptr_t)d_cur | (uintptr_t)d_out) & 15) return fail(CVS_ERR_ALIGN, "16-byte alignment required");
+    if (!aligned16(d_prev, d_cur, d_out)) return fail(CVS_ERR_ALIGN, "16-byte alignment required");
     bool hi;
     uint32_t addc;
     threshold_consts(threshold, hi, addc);
@@ -1868,7 +1790,7 @@ cvs_status cvs_grayscale_device(const uint8_t *d_frame, uint8_t *d_out, int widt
     if (st) return st;
     if (!d_frame || !d_out || width <= 0 || height <= 0 || (channels != 1 && channels != 3))
         return fail(CVS_ERR_INVALID, "bad argument");
-    if (((uintptr_t)d_frame | (uintptr_t)d_out) & 15) return fail(CVS_ERR_ALIGN, "16-byte alignment required");
+    if (!aligned16(d_frame, d_out)) return fail(CVS_ERR_ALIGN, "16-byte alignment required");
     return gray_launch(d_frame, d_out, 3u * (uint32_t)width * (uint32_t)height, weighted, channels, nullptr, sms,
                        (cudaStream_t)cuda_stream);
 }
@@ -1881,7 +1803,7 @@ cvs_status cvs_binarize_device(const uint8_t *d_frame, uint8_t *d_out, uint8_t *
     if (st) return st;
     if (!d_frame || !d_out || !d_gray || !d_hist_thr || width <= 0 || height <= 0)
         return fail(CVS_ERR_INVALID, "bad argument");
-    if (((uintptr_t)d_frame | (uintptr_t)d_out | (uintptr_t)d_gray) & 15)
+    if (!aligned16(d_frame, d_out, d_gray))
         return fail(CVS_ERR_ALIGN, "16-byte alignment required");
     cudaStream_t s = (cudaStream_t)cuda_stream;
     const uint32_t npix = (uint32_t)width * (uint32_t)height;
@@ -1951,7 +1873,7 @@ cvs_status cvs_wire_encode_device(const int *d_xs, const uint8_t *d_diff, const 
     if (st) return st;
     if (!d_xs || !d_diff || !d_pos || !d_scratch || !d_wire || width <= 0 || height <= 0)
         return fail(CVS_ERR_INVALID, "bad argument");
-    if (((uintptr_t)d_xs | (uintptr_t)d_diff | (uintptr_t)d_wire) & 15) return fail(CVS_ERR_ALIGN, "16-byte alignment required");
+    if (!aligned16(d_xs, d_diff, d_wire)) return fail(CVS_ERR_ALIGN, "16-byte alignment required");
     const uint32_t n = 3u * (uint32_t)width * (uint32_t)height, ntiles = (n + cvs::kWireTile - 1) / cvs::kWireTile;
     cudaStream_t s = (cudaStream_t)cuda_stream;
     cvs::k_wire_bounds<<<(ntiles + 256) / 256, 256, 0, s>>>(d_xs, d_pos, capacity, ntiles, d_scratch);
@@ -1968,7 +1890,7 @@ cvs_status cvs_wire_decode_device(const uint8_t *d_wire, uint32_t *d_scratch, ui
     cvs_status st = filter_common(sms);
     if (st) return st;
     if (!d_wire || !d_scratch || width <= 0 || height <= 0) return fail(CVS_ERR_INVALID, "bad argument");
-    if ((uintptr_t)d_wire & 15) return fail(CVS_ERR_ALIGN, "16-byte alignment required");
+    if (!aligned16(d_wire)) return fail(CVS_ERR_ALIGN, "16-byte alignment required");
     const uint32_t n = 3u * (uint32_t)width * (uint32_t)height, ntiles = (n + cvs::kWireTile - 1) / cvs::kWireTile;
     const uint32_t last_len = n - (ntiles - 1) * cvs::kWireTile;
     cudaStream_t s = (cudaStream_t)cuda_stream;
@@ -2015,13 +1937,13 @@ cvs_status cvs_yuv_to_bgr_device(int format, const uint8_t *const *planes, const
     const int nplanes = format == CVS_YUV_YUYV ? 1 : format == CVS_YUV_NV12 ? 2 : 3;
     const size_t row_bytes[3] = {format == CVS_YUV_YUYV ? 2 * (size_t)width : (size_t)width,
                                  format == CVS_YUV_NV12 ? (size_t)width : (size_t)width / 2, (size_t)width / 2};
-    uintptr_t align = (uintptr_t)d_out;
+    bool aligned = aligned16(d_out);
     for (int i = 0; i < nplanes; i++) {
         if (!planes[i]) return fail(CVS_ERR_INVALID, "null plane %d", i);
         if (pitches[i] < row_bytes[i]) return fail(CVS_ERR_INVALID, "pitch of plane %d is %zu, its rows hold %zu bytes", i, pitches[i], row_bytes[i]);
-        align |= (uintptr_t)planes[i] | (uintptr_t)pitches[i];
+        aligned = aligned && aligned16(planes[i], pitches[i]);
     }
-    if (align & 15) return fail(CVS_ERR_ALIGN, "planes, pitches and d_out must be 16-byte aligned");
+    if (!aligned) return fail(CVS_ERR_ALIGN, "planes, pitches and d_out must be 16-byte aligned");
     int sms = 0;
     cvs_status st = filter_common(sms);
     if (st) return st;

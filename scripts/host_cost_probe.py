@@ -1,8 +1,8 @@
 import ctypes as C, os, sys, time
-sys.path.insert(0, "/root/repo")
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT)
 import numpy as np
 import cudavideostream_b200 as cvs
-ROOT="/root/repo"
 w,h=1920,1080; n=3*w*h
 jpgs=[open(os.path.join(ROOT,"tests","golden",f),"rb").read() for f in ("k1_f1.jpg","k1_f2.jpg")]
 hb=[]
