@@ -18,6 +18,7 @@ MODE_NONE, MODE_HEAT_MAP, MODE_RED_BLACK, MODE_RED_OVERLAP = 0, 1, 2, 3
 MODE_GRAY_WEIGHTED, MODE_BINARIZE, MODE_GRAY_AVERAGE, MODE_BINARIZE_AVERAGE = 4, 5, 6, 7
 MAX_BATCH = 64  # CVS_MAX_BATCH
 YUV_YUYV, YUV_NV12, YUV_I420 = 1, 2, 3  # cvs_yuv_format
+BAYER_BGGR, BAYER_GBRG, BAYER_GRBG, BAYER_RGGB = 1, 2, 3, 4  # cvs_bayer_pattern (V4L2 sensor order)
 
 CHARS_STR = "0123456789BFPSWbkps :/"  # server/include/common.h:13
 
@@ -87,6 +88,9 @@ SIGNATURES = {
     "cvs_submit_yuv": (C.c_int, [_vp, C.c_int, _vp, _vp, _vp, C.c_char_p, _vp, _vp, C.POINTER(C.c_uint64)]),
     "cvs_submit_yuv_wire": (C.c_int, [_vp, C.c_int, _vp, _vp, _vp, C.c_char_p, C.POINTER(C.c_uint64)]),
     "cvs_yuv_to_bgr_device": (C.c_int, [C.c_int, C.POINTER(_vp), C.POINTER(_sz), _vp, C.c_int, C.c_int, _vp]),
+    "cvs_submit_bayer": (C.c_int, [_vp, C.c_int, _vp, _vp, _vp, C.c_char_p, _vp, _vp, C.POINTER(C.c_uint64)]),
+    "cvs_submit_bayer_wire": (C.c_int, [_vp, C.c_int, _vp, _vp, _vp, C.c_char_p, C.POINTER(C.c_uint64)]),
+    "cvs_bayer_to_bgr_device": (C.c_int, [C.c_int, _vp, _sz, _vp, C.c_int, C.c_int, _vp]),
     "cvs_synth_base_device": (C.c_int, [_vp, C.c_int, C.c_int, C.c_uint64, _vp]),
     "cvs_synth_next_device": (C.c_int, [_vp, _vp, C.c_int, C.c_int, C.c_uint64, C.c_uint32, C.c_uint32, _vp]),
 }
@@ -234,6 +238,22 @@ class Stream:
         """cvs_submit_yuv_wire: packed YUV frame in, one compact CVW1 frame out."""
         t = C.c_uint64(0)
         _check(load_library().cvs_submit_yuv_wire(self._h, fmt, yuv_ptr, wire_ptr, show_ptr, text.encode(), C.byref(t)))
+        return t.value
+
+    def submit_bayer_raw(self, pattern: int, raw_ptr: int, diff_ptr: int, show_ptr, text: str, pos_ptr: int,
+                         xs_ptr: int) -> int:
+        """cvs_submit_bayer: the frame arrives as the camera's 8-bit Bayer mosaic (BAYER_BGGR / _GBRG / _GRBG / _RGGB,
+        width * height bytes) and is demosaiced to BGR on the GPU (cv2.cvtColor's pixels bit for bit)."""
+        t = C.c_uint64(0)
+        _check(load_library().cvs_submit_bayer(self._h, pattern, raw_ptr, diff_ptr, show_ptr, text.encode(), pos_ptr,
+                                               xs_ptr, C.byref(t)))
+        return t.value
+
+    def submit_bayer_wire_raw(self, pattern: int, raw_ptr: int, wire_ptr: int, show_ptr, text: str) -> int:
+        """cvs_submit_bayer_wire: Bayer mosaic in, one compact CVW1 frame out."""
+        t = C.c_uint64(0)
+        _check(load_library().cvs_submit_bayer_wire(self._h, pattern, raw_ptr, wire_ptr, show_ptr, text.encode(),
+                                                    C.byref(t)))
         return t.value
 
     def decode_jpeg_device(self, jpeg: bytes, d_out: int, cuda_stream: int = 0) -> None:

@@ -13,7 +13,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(_HERE, "csrc")
 LIB = os.path.join(_HERE, "libcvs_b200.so")
 SOURCES = ["cvs_api.cu", "cvs_shim.cu"]
-HEADERS = ["cvs_device.cuh", "cvs_pixel.cuh", "cvs_stream_kernel.cuh", "cvs_stream_ws.cuh", "cvs_filter_kernels.cuh", "cvs_jpeg.cuh", "cvs_jpeg_host.hpp", "cvs_yuv.cuh",
+HEADERS = ["cvs_device.cuh", "cvs_pixel.cuh", "cvs_stream_kernel.cuh", "cvs_stream_ws.cuh", "cvs_filter_kernels.cuh", "cvs_jpeg.cuh", "cvs_jpeg_host.hpp", "cvs_yuv.cuh", "cvs_bayer.cuh",
            os.path.join("..", "..", "include", "cvs_b200.h"), os.path.join("..", "..", "include", "cvs_cuda_core.hpp")]
 
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",

@@ -24,6 +24,7 @@
 #include <string>
 #include <type_traits>
 
+#include "cvs_bayer.cuh"
 #include "cvs_filter_kernels.cuh"
 #include "cvs_jpeg_host.hpp"
 #include "cvs_stream_kernel.cuh"
@@ -334,7 +335,7 @@ struct Slot {
     DevBuf<uint32_t> d_starts;        // compact wire format: entries before each tile (ntiles + 2 words), on first use
     DevBuf<uint8_t> d_wire;           // compact wire format: encoded frame when the caller's buffer is not mapped
     nvjpegJpegState_t jpeg_state = nullptr; // cvs_submit_jpeg: decoder state of this slot (on first use)
-    DevBuf<uint8_t> d_yuv;            // cvs_submit_yuv: the camera's packed YUV frame as uploaded (on first use)
+    DevBuf<uint8_t> d_cam;            // cvs_submit_yuv / _bayer: the camera's raw frame as uploaded (on first use)
     uint8_t *u_wire = nullptr;        // caller's buffer of a cvs_submit_wire ticket (nullptr: reference-format ticket)
     DevBuf<unsigned int> d_status;    // StatusBits of this ticket's launches (cleared at submit)
     PinnedWord h_status;              // copy of d_status, valid once ev_pos has fired
@@ -1323,12 +1324,52 @@ static void yuv_packed_planes(int format, const uint8_t *base, int width, int he
     pitches[2] = (size_t)width / 2;
 }
 
+// k_bayer_to_bgr on `st`: arguments as cvs_bayer_to_bgr_device takes them, already checked
+static cvs_status bayer_launch(int pattern, const uint8_t *raw, size_t pitch, uint8_t *d_out, int width, int height,
+                               cudaStream_t st)
+{
+    cvs::BayerParams p;
+    p.raw = raw;
+    p.pitch = pitch;
+    p.bgr = d_out;
+    p.width = width;
+    p.height = height;
+    p.groups = (uint32_t)(width + cvs::kBayerPixels - 1) / cvs::kBayerPixels;
+    p.py = (pattern - CVS_BAYER_BGGR) >> 1; // BGGR, GBRG, GRBG, RGGB: (py, px) = (0, 0), (0, 1), (1, 0), (1, 1)
+    p.px = (pattern - CVS_BAYER_BGGR) & 1;
+    const unsigned blocks = (unsigned)(((size_t)p.groups * (size_t)height + cvs::kBayerThreads - 1) / cvs::kBayerThreads);
+    cvs::k_bayer_to_bgr<<<blocks, cvs::kBayerThreads, 0, st>>>(p);
+    CU_TRY(cudaGetLastError());
+    return CVS_OK;
+}
+
+// The camera format of a submitted frame: 0 for a BGR frame (or a JPEG bitstream), a cvs_yuv_format, or kCamBayer plus a
+// cvs_bayer_pattern.  A raw camera frame is uploaded as packed rows into the slot's staging buffer s.d_cam and converted
+// to BGR on the compute stream in front of the stream kernel.
+constexpr int kCamBayer = 16;
+
+// bytes of a packed raw camera frame (cam != 0, checked by the caller)
+static size_t cam_frame_bytes(int cam, int width, int height)
+{
+    return cam > kCamBayer ? (size_t)width * (size_t)height : cvs_yuv_frame_bytes(cam, width, height);
+}
+
+// the packed raw camera frame at `src` (device) -> BGR at d_out, on `st`
+static cvs_status cam_to_bgr(int cam, const uint8_t *src, uint8_t *d_out, int width, int height, cudaStream_t st)
+{
+    if (cam > kCamBayer) return bayer_launch(cam - kCamBayer, src, (size_t)width, d_out, width, height, st);
+    const uint8_t *planes[3];
+    size_t pitches[3];
+    yuv_packed_planes(cam, src, width, height, planes, pitches);
+    return yuv_launch(cam, planes, pitches, d_out, width, height, st);
+}
+
 // H2D of a ticket's frame into s.d_in (kernels.cu:461) between the slot's timing events: the N-byte BGR frame, or
-// (yuv_format != 0) a packed YUV frame into s.d_yuv, converted on the compute stream later, or (jpeg_bytes != 0) the
+// (cam != 0) a raw camera frame into s.d_cam, converted on the compute stream later, or (jpeg_bytes != 0) the
 // camera's JPEG bitstream, decoded on the device.  JPEG tickets alternate between two decode streams with their own
 // scratch: frame t+1 is decoded beside frame t (a decode is a latency chain that leaves most of the GPU idle); the
 // stream kernel still takes the frames in ticket order.  The compute stream waits for the frame and marks ev_k0.
-static cvs_status ingest(cvs_handle h, Slot &s, const uint8_t *frame, size_t jpeg_bytes = 0, int yuv_format = 0)
+static cvs_status ingest(cvs_handle h, Slot &s, const uint8_t *frame, size_t jpeg_bytes = 0, int cam = 0)
 {
     cudaStream_t s_in = h->s_h2d;
     const JpegSet jset = (h->next_ticket & 1) ? kJpegTicketOdd : kJpegTicketEven;
@@ -1341,9 +1382,8 @@ static cvs_status ingest(cvs_handle h, Slot &s, const uint8_t *frame, size_t jpe
         // (the ticket's status word is cleared here, in front of the decoder that may raise bits in it)
         CU_TRY(cudaMemsetAsync(s.d_status, 0, sizeof(unsigned int), s_in));
         CVS_TRY(jpeg_decode(h, jset, &s.jpeg_state, frame, jpeg_bytes, s.d_in, s_in, s.d_status));
-    } else if (yuv_format) {
-        CU_TRY(cudaMemcpyAsync(s.d_yuv, frame, cvs_yuv_frame_bytes(yuv_format, h->width, h->height), cudaMemcpyHostToDevice,
-                               h->s_h2d));
+    } else if (cam) {
+        CU_TRY(cudaMemcpyAsync(s.d_cam, frame, cam_frame_bytes(cam, h->width, h->height), cudaMemcpyHostToDevice, h->s_h2d));
     } else {
         CU_TRY(cudaMemcpyAsync(s.d_in, frame, h->N, cudaMemcpyHostToDevice, h->s_h2d));
     }
@@ -1353,11 +1393,11 @@ static cvs_status ingest(cvs_handle h, Slot &s, const uint8_t *frame, size_t jpe
     return CVS_OK;
 }
 
-// jpeg_bytes != 0: `frame` is the camera's JPEG bitstream; yuv_format != 0: `frame` is a packed YUV frame of that format
+// jpeg_bytes != 0: `frame` is the camera's JPEG bitstream; cam != 0: `frame` is a raw camera frame of that format
 // (checked by the caller); otherwise the N-byte BGR frame
 static cvs_status submit_common(cvs_handle h, const uint8_t *frame, uint8_t *diff_out, uint8_t *show, const char *text,
                                 unsigned int *pos, int *xs, uint8_t *wire_out, uint64_t *ticket, size_t jpeg_bytes = 0,
-                                int yuv_format = 0)
+                                int cam = 0)
 {
     cvs_status st = check_handle(h);
     if (st) return st;
@@ -1370,19 +1410,16 @@ static cvs_status submit_common(cvs_handle h, const uint8_t *frame, uint8_t *dif
         CVS_TRY(s.d_wire.grow(cvs_wire_bound(h->width, h->height), "wire frame"));
     }
     // sized for the largest layout (YUYV, 2WH), so tickets of every format share it
-    if (yuv_format) CVS_TRY(s.d_yuv.grow(round_up(cvs_yuv_frame_bytes(CVS_YUV_YUYV, h->width, h->height), 16), "YUV frame"));
+    if (cam) CVS_TRY(s.d_cam.grow(round_up(2 * (size_t)h->width * (size_t)h->height, 16), "camera frame"));
 
     const double th0 = h->trace ? host_us() : 0;
-    CVS_TRY(ingest(h, s, frame, jpeg_bytes, yuv_format));
+    CVS_TRY(ingest(h, s, frame, jpeg_bytes, cam));
     const size_t cap = round_up(h->N, 4);
     uint8_t *dshow = (h->mode && show) ? s.d_show.p : nullptr;
     const double th1 = h->trace ? host_us() : 0;
     if (!jpeg_bytes) CU_TRY(cudaMemsetAsync(s.d_status, 0, sizeof(unsigned int), h->s_comp));
-    if (yuv_format) { // (inside ev_k0 .. ev_k1: cvs_get_timing counts the conversion as kernel time)
-        const uint8_t *planes[3];
-        size_t pitches[3];
-        yuv_packed_planes(yuv_format, s.d_yuv, h->width, h->height, planes, pitches);
-        st = yuv_launch(yuv_format, planes, pitches, s.d_in, h->width, h->height, h->s_comp);
+    if (cam) { // (inside ev_k0 .. ev_k1: cvs_get_timing counts the conversion as kernel time)
+        st = cam_to_bgr(cam, s.d_cam, s.d_in, h->width, h->height, h->s_comp);
         if (st) return st;
         h->launches++;
     }
@@ -1529,6 +1566,34 @@ cvs_status cvs_submit_yuv_wire(cvs_handle h, int format, const uint8_t *yuv, uin
     if (st) return st;
     if (!wire_out) return fail(CVS_ERR_INVALID, "null argument");
     return submit_common(h, yuv, nullptr, show, text, nullptr, nullptr, wire_out, ticket, 0, format);
+}
+
+// a Bayer submission that cvs_submit_bayer / cvs_submit_bayer_wire refuse before anything is enqueued (every frame size
+// is accepted, as cv2.cvtColor does)
+static cvs_status check_bayer_submit(cvs_handle h, int pattern, const uint8_t *raw)
+{
+    cvs_status st = check_handle(h);
+    if (st) return st;
+    if (pattern < CVS_BAYER_BGGR || pattern > CVS_BAYER_RGGB) return fail(CVS_ERR_INVALID, "unknown Bayer pattern %d", pattern);
+    if (!raw) return fail(CVS_ERR_INVALID, "null argument");
+    return CVS_OK;
+}
+
+cvs_status cvs_submit_bayer(cvs_handle h, int pattern, const uint8_t *raw, uint8_t *diff_out, uint8_t *show,
+                            const char *text, unsigned int *pos, int *xs, uint64_t *ticket)
+{
+    cvs_status st = check_bayer_submit(h, pattern, raw);
+    if (st) return st;
+    return submit_common(h, raw, diff_out, show, text, pos, xs, nullptr, ticket, 0, kCamBayer + pattern);
+}
+
+cvs_status cvs_submit_bayer_wire(cvs_handle h, int pattern, const uint8_t *raw, uint8_t *wire_out, uint8_t *show,
+                                 const char *text, uint64_t *ticket)
+{
+    cvs_status st = check_bayer_submit(h, pattern, raw);
+    if (st) return st;
+    if (!wire_out) return fail(CVS_ERR_INVALID, "null argument");
+    return submit_common(h, raw, nullptr, show, text, nullptr, nullptr, wire_out, ticket, 0, kCamBayer + pattern);
 }
 
 cvs_status cvs_submit_wire(cvs_handle h, const uint8_t *frame, uint8_t *wire_out, uint8_t *show, const char *text,
@@ -1948,6 +2013,21 @@ cvs_status cvs_yuv_to_bgr_device(int format, const uint8_t *const *planes, const
     cvs_status st = filter_common(sms);
     if (st) return st;
     return yuv_launch(format, planes, pitches, d_out, width, height, (cudaStream_t)cuda_stream);
+}
+
+cvs_status cvs_bayer_to_bgr_device(int pattern, const uint8_t *d_raw, size_t pitch, uint8_t *d_out, int width, int height,
+                                   void *cuda_stream)
+{
+    // arguments first: a refusal needs no device
+    if (pattern < CVS_BAYER_BGGR || pattern > CVS_BAYER_RGGB) return fail(CVS_ERR_INVALID, "unknown Bayer pattern %d", pattern);
+    if (width <= 0 || height <= 0) return fail(CVS_ERR_INVALID, "%dx%d: not a frame size", width, height);
+    if (!d_raw || !d_out) return fail(CVS_ERR_INVALID, "null argument");
+    if (pitch < (size_t)width) return fail(CVS_ERR_INVALID, "pitch %zu is less than the width %d", pitch, width);
+    if (!aligned16(d_raw, pitch, d_out)) return fail(CVS_ERR_ALIGN, "d_raw, pitch and d_out must be 16-byte aligned");
+    int sms = 0;
+    cvs_status st = filter_common(sms);
+    if (st) return st;
+    return bayer_launch(pattern, d_raw, pitch, d_out, width, height, (cudaStream_t)cuda_stream);
 }
 
 cvs_status cvs_synth_base_device(uint8_t *d_out, int width, int height, uint64_t seed, void *cuda_stream)

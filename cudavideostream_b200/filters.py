@@ -43,3 +43,9 @@ def yuv_to_bgr(fmt: int, planes, pitches, d_out: int, width: int, height: int, s
     # three entries whatever the format: missing planes arrive as NULL and are refused, never read past the array
     _check(load_library().cvs_yuv_to_bgr_device(fmt, (_vp * 3)(*planes), (_sz * 3)(*pitches), d_out, width, height,
                                                 stream or None))
+
+
+def bayer_to_bgr(pattern: int, d_raw: int, pitch: int, d_out: int, width: int, height: int, stream: int = 0) -> None:
+    """cvs_bayer_to_bgr_device: an 8-bit Bayer mosaic in device memory (rows `pitch` bytes apart) -> packed BGR24
+    (cv2.cvtColor's pixels)."""
+    _check(load_library().cvs_bayer_to_bgr_device(pattern, d_raw, pitch, d_out, width, height, stream or None))

@@ -351,6 +351,52 @@ cvs_status cvs_submit_yuv_wire(cvs_handle h, int format, const uint8_t *yuv, uin
 cvs_status cvs_yuv_to_bgr_device(int format, const uint8_t *const *planes, const size_t *pitches, uint8_t *d_out,
                                  int width, int height, void *cuda_stream);
 
+/* ---------------------------------------------------------------------------------------------------------------
+ * Raw Bayer cameras: the capture side's demosaic on the GPU.  Raw-sensor and machine-vision cameras (CSI sensors exposed
+ * as raw V4L2 devices, USB3 / GigE industrial cameras) deliver an 8-bit Bayer mosaic, one byte per pixel.
+ * cvs_submit_bayer takes that mosaic instead of the BGR frame a host-side cv2.cvtColor would make of it: WH bytes cross
+ * PCIe instead of 3WH (1080p: 2.07 MB instead of 6.2 MB), and no host CPU demosaics.
+ *   The pattern names the sensor's top-left 2x2 in V4L2 order: CVS_BAYER_BGGR is row 0 B G B G ..., row 1 G R G R ...
+ *   (V4L2_PIX_FMT_SBGGR8, cv2.COLOR_BayerBGGR2BGR; likewise GBRG, GRBG, RGGB).  OpenCV's older two-letter names are
+ *   shifted against this order (COLOR_BayerBG2BGR is COLOR_BayerRGGB2BGR): use the four-letter ones.
+ *   The pixels are cv2.cvtColor's default (bilinear) demosaic bit for bit, integer only:
+ *     W < 3 or H < 3: all zero.  Otherwise out(y, x) = I(clamp(y, 1, H-2), clamp(x, 1, W-2)), where at an interior
+ *     pixel of mosaic colour c:  channel c = raw[y][x];
+ *       c = G:      the horizontal neighbours' colour = (left + right + 1) >> 1, the vertical ones' = (up + down + 1) >> 1;
+ *       c = R or B: G = (left + right + up + down + 2) >> 2, the opposite colour = (four diagonals + 2) >> 2.
+ *   Layout: W x H bytes, rows without padding.  Every positive frame size is accepted, odd ones included.
+ *   The frame is uploaded on the handle's copy stream into a buffer of the ticket's slot, demosaiced on the compute
+ *   stream in front of the stream kernel into the slot's frame buffer, and from there everything is what cvs_submit_io
+ *   / cvs_submit_wire do (noise filter, overlay, display modes, egress, tickets, cvs_wait).  cvs_get_timing reports the
+ *   upload of the mosaic as h2d and counts the demosaic into the kernel time.
+ *   Refused with CVS_ERR_INVALID before anything is enqueued, without consuming a ticket (the reference and the next
+ *   ticket stay as they were): a pattern outside CVS_BAYER_BGGR..CVS_BAYER_RGGB, a NULL argument.  The base frame
+ *   stays BGR (cvs_create, cvs_reset): INTEGRATION.md says how to get it.
+ *   Measured on a B200 at its 1000 W power limit (DESIGN.md section 5.4): the demosaic takes 5.0 us per 1080p frame;
+ *   three 1080p streams run at 7.2 k frames/s end to end against 5.4 k with the same mosaics demosaiced on the host and
+ *   uploaded as BGR.
+ *   Not covered: 10/12/16-bit mosaics, VNG and edge-aware demosaics.
+ * --------------------------------------------------------------------------------------------------------------- */
+typedef enum cvs_bayer_pattern {
+    CVS_BAYER_BGGR = 1,
+    CVS_BAYER_GBRG = 2,
+    CVS_BAYER_GRBG = 3,
+    CVS_BAYER_RGGB = 4
+} cvs_bayer_pattern;
+/* cvs_submit_io with the frame as the camera's W*H mosaic bytes (host; pinned memory from cvs_alloc_host lets the upload
+ * overlap) */
+cvs_status cvs_submit_bayer(cvs_handle h, int pattern, const uint8_t *raw, uint8_t *diff_out, uint8_t *show,
+                            const char *text, unsigned int *pos, int *xs, uint64_t *ticket);
+/* cvs_submit_wire with the frame as the camera's W*H mosaic bytes */
+cvs_status cvs_submit_bayer_wire(cvs_handle h, int pattern, const uint8_t *raw, uint8_t *wire_out, uint8_t *show,
+                                 const char *text, uint64_t *ticket);
+/* the demosaic alone, device to device, asynchronous on cuda_stream: a mosaic at d_raw with rows `pitch` bytes apart ->
+ * 3 * width * height bytes of packed BGR24 at d_out, nothing written outside them.  pitch < width, a size that is not
+ * positive, a NULL pointer or an unknown pattern: CVS_ERR_INVALID; d_raw, pitch or d_out not 16-byte aligned:
+ * CVS_ERR_ALIGN. */
+cvs_status cvs_bayer_to_bgr_device(int pattern, const uint8_t *d_raw, size_t pitch, uint8_t *d_out, int width,
+                                   int height, void *cuda_stream);
+
 /* Synthetic camera used by bench.py and the parity tests (SURVEY.md section 8d): counter-based
  * splitmix64 so that the numpy twin in cudavideostream_b200/synth.py produces identical bytes.
  *   cvs_synth_base_device   : base frame (diagonal gradient + noise)

@@ -1,19 +1,23 @@
-"""Raw YUV ingest on the GPU: what k_yuv_to_bgr costs and what cvs_submit_yuv buys end to end.
+"""Raw camera ingest on the GPU (YUV and Bayer): what k_yuv_to_bgr and k_bayer_to_bgr cost and what cvs_submit_yuv and
+cvs_submit_bayer buy end to end.
 
-1. Kernel time per frame of cvs_yuv_to_bgr_device for NV12, I420 and YUYV at 1920x1080 and 3840x2160: CUDA events around
-   a CUDA graph of launches that walks a ring of frames larger than the 126 MB L2 (every frame is read from and written
-   to HBM), against the bytes model (read 1.5 or 2 bytes per pixel, write 3) and the HBM copy peak: the one bench.py
-   uses (MEASURED_PEAKS.json, else its fallback) and a device-to-device copy measured here.  Beside them the same graph
-   of launches on a 16x2 frame (one block): the fixed cost of a launch in a graph, which no frame size goes below.
+1. Kernel time per frame of cvs_yuv_to_bgr_device for NV12, I420 and YUYV and of cvs_bayer_to_bgr_device (RGGB) at
+   1920x1080 and 3840x2160: CUDA events around a CUDA graph of launches that walks a ring of frames larger than the
+   126 MB L2 (every frame is read from and written to HBM), against the bytes model (read 1.5 or 2 bytes per pixel for
+   YUV, 1 for Bayer; write 3) and the HBM copy peak: the one bench.py uses (MEASURED_PEAKS.json, else its fallback) and
+   a device-to-device copy measured here.  Beside them the same graph of launches on a 16x2 (16x3 for Bayer) frame, one
+   block: the fixed cost of a launch in a graph, which no frame size goes below.
 2. End to end, frames/s of three camera streams per GPU submitted round-robin with four tickets in flight each, as in
    bench.py's e2e leg (1080p, 1 / 10 / 50 % change density, pinned host rings): cvs_submit_yuv with NV12 and with YUYV
-   frames, each against cvs_submit_io with the very BGR frames they convert to ("raw:nv12", "raw:yuyv": the pictures,
-   change densities and payloads of a pair are identical; YUYV keeps more chroma than NV12, so the two pairs differ in
-   payload), the four forms alternated in the same process.
+   frames and cvs_submit_bayer with RGGB mosaics, each against cvs_submit_io with the very BGR frames they convert to
+   ("raw:nv12", "raw:yuyv", "raw:bayer": the pictures, change densities and payloads of a pair are identical; the
+   formats keep different colour detail, so the pairs differ from each other in payload), the six forms alternated in
+   the same process.
 3. The same three streams under CVS_TRACE=1 (a run of its own, 8 warm-up and 40 timed frames per stream and form, the
    warm-up tickets dropped): device time of each ticket's upload and kernels.
 
-Run on the GPU box: python scripts/yuv_probe.py > profiles/yuv_probe.txt"""
+Run on the GPU box: python scripts/yuv_probe.py > profiles/bayer_probe.txt (profiles/yuv_probe.txt is the earlier run,
+before the Bayer rows)"""
 import ctypes as C
 import json
 import os
@@ -30,6 +34,7 @@ import numpy as np  # noqa: E402
 import torch  # noqa: E402
 
 import cudavideostream_b200 as cvs  # noqa: E402
+import bayer_ref as B  # noqa: E402
 import yuv_ref as Y  # noqa: E402
 from oracle import oracle  # noqa: E402
 
@@ -37,7 +42,8 @@ W, H = 1920, 1080
 N = 3 * W * H
 DENSITIES_PPM = (10000, 100000, 500000)
 L2_BYTES = 126 << 20
-FORMS = ("raw:nv12", "nv12", "raw:yuyv", "yuyv")
+FORMS = ("raw:nv12", "nv12", "raw:yuyv", "yuyv", "raw:bayer", "bayer")
+BAYER = B.RGGB
 
 
 def packed(fmt, base, w, h):
@@ -76,9 +82,26 @@ def copy_peak():
     return gbs
 
 
+def convert(fmt, src, dst, w, h, stream):
+    """one packed frame at device address src -> BGR at dst; fmt: a YUV format, or "bayer" """
+    if fmt == "bayer":
+        cvs.filters.bayer_to_bgr(BAYER, src, w, dst, w, h, stream)
+    else:
+        pl, pi = packed(fmt, src, w, h)
+        cvs.filters.yuv_to_bgr(fmt, pl, pi, dst, w, h, stream)
+
+
+def in_bytes(fmt, w, h):
+    return w * h if fmt == "bayer" else Y.frame_bytes(fmt, w, h)
+
+
+def name(fmt):
+    return "bayer" if fmt == "bayer" else Y.NAMES[fmt]
+
+
 def graph_us(fmt, w, h, K):
-    """device time per launch of cvs_yuv_to_bgr_device in a CUDA graph that converts a ring of K packed frames"""
-    fin, fout = Y.frame_bytes(fmt, w, h), 3 * w * h
+    """device time per launch of the conversion in a CUDA graph that converts a ring of K packed frames"""
+    fin, fout = in_bytes(fmt, w, h), 3 * w * h
     sin, sout = (fin + 15) // 16 * 16, (fout + 15) // 16 * 16
     src = torch.randint(0, 256, (K * sin,), dtype=torch.uint8, device="cuda")
     dst = torch.empty(K * sout, dtype=torch.uint8, device="cuda")
@@ -86,8 +109,7 @@ def graph_us(fmt, w, h, K):
 
     def launch_ring(stream):
         for i in range(K):
-            pl, pi = packed(fmt, src.data_ptr() + i * sin, w, h)
-            cvs.filters.yuv_to_bgr(fmt, pl, pi, dst.data_ptr() + i * sout, w, h, stream)
+            convert(fmt, src.data_ptr() + i * sin, dst.data_ptr() + i * sout, w, h, stream)
 
     with torch.cuda.stream(st):
         launch_ring(st.cuda_stream)  # warm-up, outside the graph
@@ -111,22 +133,26 @@ def graph_us(fmt, w, h, K):
 
 
 def kernel_times(peak):
-    print("\n== k_yuv_to_bgr: device time per frame (CUDA graph of launches over an L2-cold ring, CUDA events) ==")
+    print("\n== k_yuv_to_bgr / k_bayer_to_bgr: device time per frame (CUDA graph of launches over an L2-cold ring, CUDA "
+          "events) ==")
     print(f"{'size':>10} {'format':>6} {'ring':>5} {'us/frame':>9} {'model MB':>9} {'GB/s':>7} {'of peak':>8}")
     for w, h in ((1920, 1080), (3840, 2160)):
-        for fmt in (Y.NV12, Y.I420, Y.YUYV):
-            fin, fout = Y.frame_bytes(fmt, w, h), 3 * w * h
+        for fmt in (Y.NV12, Y.I420, Y.YUYV, "bayer"):
+            fin, fout = in_bytes(fmt, w, h), 3 * w * h
             K = max(8, -(-3 * L2_BYTES // (fin + fout + 32)))  # ring of three L2 sizes
             us = graph_us(fmt, w, h, K)
             gbs = (fin + fout) / (us * 1e-6) / 1e9
-            print(f"{w}x{h:<5} {Y.NAMES[fmt]:>6} {K:5d} {us:9.2f} {(fin + fout) / 1e6:9.2f} {gbs:7.0f} {gbs / peak:8.1%}")
-    for fmt in (Y.NV12, Y.YUYV):  # 16 x 2: one block, and plane pitches that are multiples of 16 as the entry requires
-        print(f"{'16x2':>10} {Y.NAMES[fmt]:>6} {64:5d} {graph_us(fmt, 16, 2, 64):9.2f}   (one block: the fixed cost of a launch)")
+            print(f"{w}x{h:<5} {name(fmt):>6} {K:5d} {us:9.2f} {(fin + fout) / 1e6:9.2f} {gbs:7.0f} {gbs / peak:8.1%}")
+    # one block, and plane pitches that are multiples of 16 as the entries require (16x3: the smallest frame the
+    # demosaic computes rather than zeroes)
+    for fmt, (w, h) in ((Y.NV12, (16, 2)), (Y.YUYV, (16, 2)), ("bayer", (16, 3))):
+        print(f"{f'{w}x{h}':>10} {name(fmt):>6} {64:5d} {graph_us(fmt, w, h, 64):9.2f}   (one block: the fixed cost of a launch)")
 
 
 def make_rings(R=16):
-    """per density: R frames as NV12 and as YUYV, and as the BGR frames cv2.cvtColor makes of each (raw:nv12, raw:yuyv:
-    what a server uploads today after converting on the host), with the base frame of each"""
+    """per density: R frames as NV12, as YUYV and as an RGGB mosaic, and as the BGR frames cv2.cvtColor makes of each
+    (raw:nv12, raw:yuyv, raw:bayer: what a server uploads today after converting on the host), with the base frame of
+    each"""
     rings = []
     for k, d in enumerate(DENSITIES_PPM):
         base, frames = oracle.synth_sequence(W, H, R, d, 0xC0FFEE + k)
@@ -135,6 +161,9 @@ def make_rings(R=16):
             bases[name] = bases["raw:" + name] = Y.yuv_to_bgr(fmt, Y.from_bgr(fmt, base, W, H), W, H).reshape(-1)
             forms[name] = [Y.from_bgr(fmt, f, W, H) for f in frames]
             forms["raw:" + name] = [Y.yuv_to_bgr(fmt, b, W, H).reshape(-1) for b in forms[name]]
+        bases["bayer"] = bases["raw:bayer"] = B.bayer_to_bgr(BAYER, B.mosaic(base.reshape(H, W, 3), BAYER)).reshape(-1)
+        forms["bayer"] = [B.mosaic(f.reshape(H, W, 3), BAYER).reshape(-1) for f in frames]
+        forms["raw:bayer"] = [B.bayer_to_bgr(BAYER, m.reshape(H, W)).reshape(-1) for m in forms["bayer"]]
         host = {}
         for name, lst in forms.items():
             sz = lst[0].size
@@ -168,6 +197,8 @@ def e2e(rings, form, nframes, R=16):
                 src = hb.ptr + order[i % len(order)] * sz
                 if form.startswith("raw"):
                     tk = s.submit_io_raw(src, fb.ptr, None, "", C.addressof(pb), xb.ptr)
+                elif form == "bayer":
+                    tk = s.submit_bayer_raw(BAYER, src, fb.ptr, None, "", C.addressof(pb), xb.ptr)
                 else:
                     tk = s.submit_yuv_raw(Y.NV12 if form == "nv12" else Y.YUYV, src, fb.ptr, None, "", C.addressof(pb), xb.ptr)
                 pending.append((tk, pb))
@@ -198,9 +229,9 @@ def e2e_table(nframes=300, rounds=5):
             fps, mean_pos, h2d = e2e(rings, form, nframes)
             res[form].append(fps)
             meta[form] = (mean_pos, h2d)
-    print(f"{'form':>8} {'H2D B/frame':>12} {'mean pos':>10} {'frames/s median':>16} {'min':>8} {'max':>8}  per round")
+    print(f"{'form':>9} {'H2D B/frame':>12} {'mean pos':>10} {'frames/s median':>16} {'min':>8} {'max':>8}  per round")
     for form, v in res.items():
-        print(f"{form:>8} {meta[form][1]:12d} {meta[form][0]:10.0f} {statistics.median(v):16.0f} {min(v):8.0f} {max(v):8.0f}  "
+        print(f"{form:>9} {meta[form][1]:12d} {meta[form][0]:10.0f} {statistics.median(v):16.0f} {min(v):8.0f} {max(v):8.0f}  "
               + " ".join(f"{x:.0f}" for x in v))
     for q in rings:
         q["stream"].close()
@@ -232,7 +263,7 @@ def trace_summary():
     for form, v in rows.items():
         v = v[24:]  # past the warm-up frames
         if v:
-            print(f"{form:>8}: upload {np.mean([x[0] for x in v]):7.1f} us  kernels {np.mean([x[1] for x in v]):6.1f} us  "
+            print(f"{form:>9}: upload {np.mean([x[0] for x in v]):7.1f} us  kernels {np.mean([x[1] for x in v]):6.1f} us  "
                   f"kernels end -> payload on host {np.mean([x[2] for x in v]):7.1f} us  ({len(v)} tickets)")
     if r.returncode:
         print("trace run failed:", r.stderr[-600:])
